@@ -16,7 +16,7 @@ One STEP = the WHOLE filter job (/root/reference/filter.py:92-166) of the graph,
 strong scaling: the same job on N GPUs.  Nothing is cached between steps.  `e2e` = the same call with HOST
 inputs: graph, features and weights uploaded from pinned memory and both [k,3] lists copied back, every step.
 
-  python bench.py [--gpus N --steps K --warmup W] [--workload ppa|collab|ddi|small|tiny]
+  python bench.py [--gpus N --steps K --warmup W] [--workload ppa|collab|ddi|small|tiny] [--dump-outputs DIR]
   python bench.py --impl reference ...     # the reference's CPU path (oracle port) on host cores
 """
 from __future__ import annotations
@@ -64,7 +64,16 @@ def parse():
                    help="skip the ddi / collab shape lines, the library baseline and the multi-GPU self-check")
     p.add_argument("--no-pushdown", action="store_true", help="K4 select over every slab instead of K4b push-down (A/B)")
     p.add_argument("--cpu-seconds", type=float, default=12.0)
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the proposal lists of the last timed step to DIR/<filter model>.npy (float32 rows u, v, "
+                        "score; lists over their share of 60 MiB cut to rows at fixed seeded positions), so that two "
+                        "builds can be compared output for output")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs is not None and a.impl != "b200":
+        p.error("--dump-outputs writes the b200 arm's outputs")
+    return a
 
 
 # ------------------------------------------------------------------------------------------
@@ -500,6 +509,19 @@ def measure(wl: Workload, steps: int, warmup: int, rank: int, world: int, e2e_st
                 spmm_ms=spmm_ms, e2e=e2e, outs=outs, adj=adj, x=x)
 
 
+def dump_outputs(outs, out_dir, budget=60 << 20):
+    """``outs`` (Workload.step's [k,3] lists: u, v, score) -> out_dir/<filter model>.npy, float32.  A list larger than
+    its share of ``budget`` bytes keeps the rows at a seeded sample of positions, ascending: the same positions in
+    every run of the same arguments, so that the files of two builds compare row for row."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in zip(("adamic_ogb", "gcn"), outs):
+        a = t.float().cpu().numpy()
+        rows = budget // len(outs) // (a.shape[1] * a.itemsize)
+        if a.shape[0] > rows:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], rows, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def library_baseline(wl: Workload, adj, x, k):
     """SURVEY §2.1's bar, same box: the library kernels the reference reaches — ATen index_select + mul,
     cuBLAS Linear, relu, sigmoid (models.py:478-485,506) in fp32 (TF32 off, the reference default) and in bf16
@@ -590,6 +612,8 @@ def run_b200(args):
     sampler = ClockSampler(local) if rank == 0 else None
     res = measure(wl, args.steps, args.warmup, rank, world, e2e_steps=min(args.steps, 5), sampler=sampler)
     clocks = sampler.stop() if sampler is not None else None
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(res["outs"], args.dump_outputs)
     adj, x = res["adj"], res["x"]
     st = res["stats"]
     phase_ms = res["phase_ms"]

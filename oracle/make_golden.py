@@ -1,4 +1,5 @@
-"""Generate tests/golden/*.npz by EXECUTING the reference in the build container.
+"""Generate tests/golden/{twitch,fb}.npz (graph split, whole-set checksums) and {twitch,fb}_sample.npz
+(the reference's scores on a seeded sample of candidates) by EXECUTING the reference.
 
 TEST INFRASTRUCTURE — see ``oracle/__init__.py``.  Run from the repo root:
 
@@ -111,11 +112,6 @@ def main():
             test_edges=test.astype(np.uint16),
             num_candidates=np.int64(N),
             cand_sha256=np.array(sha(cand.astype(np.int32))),
-            sample_index=samp.astype(np.int64),
-            sample_edges=s_edges.astype(np.int32),
-            sample_cn=cn_vals[samp].astype(np.int32),
-            sample_aa=aa_all[samp].astype(np.float32),
-            sample_ra=ra_s.astype(np.float32),
             sum_cn=np.int64(cn_vals.astype(np.int64).sum()),
             sum_aa=np.float64(aa_all.astype(np.float64).sum()),
             max_cn=np.int64(cn_vals.max()),
@@ -125,7 +121,15 @@ def main():
             topk_cn_tail=topk_cn[-64:],
             ref_aa_pairs_per_s_1core=np.float64(N / t_aa),
         )
-        print(f"   wrote {name}.npz  sum_cn={int(cn_vals.sum())} max_cn={int(cn_vals.max())}")
+        np.savez_compressed(
+            os.path.join(OUT, f"{name}_sample.npz"),
+            sample_index=samp.astype(np.int64),
+            sample_edges=s_edges.astype(np.int32),
+            sample_cn=cn_vals[samp].astype(np.int32),
+            sample_aa=aa_all[samp].astype(np.float32),
+            sample_ra=ra_s.astype(np.float32),
+        )
+        print(f"   wrote {name}.npz, {name}_sample.npz  sum_cn={int(cn_vals.sum())} max_cn={int(cn_vals.max())}")
 
 
 if __name__ == "__main__":

@@ -1,5 +1,5 @@
 """LinkPredictor and default_model_configs against vectors produced by EXECUTING the reference's
-own models.py (oracle/make_golden_models.py -> tests/golden/linkpred.npz, model_configs.json)."""
+own models.py (oracle/make_golden_models.py -> tests/golden/linkpred_H*_L*.npz, model_configs.json)."""
 import argparse
 import json
 import os
@@ -17,8 +17,8 @@ FIELDS = ["num_layers", "hidden_channels", "dropout", "batch_size", "lr", "epoch
 
 
 def _case(H, L):
-    z = np.load(os.path.join(GOLDEN, "linkpred.npz"))
     tag = f"H{H}_L{L}"
+    z = np.load(os.path.join(GOLDEN, f"linkpred_{tag}.npz"))
     sd = {f"linkpred.lins.{i}.{p}": torch.from_numpy(z[f"{tag}/lins.{i}.{p}"]) for i in range(L) for p in ("weight", "bias")}
     return torch.from_numpy(z[f"{tag}/x_i"]), torch.from_numpy(z[f"{tag}/x_j"]), z[f"{tag}/y"], sd
 

@@ -3,6 +3,7 @@ construction (train_and_eval.py:43-56), transposed CSR values for the SpMM backw
 checkpoint layout, and the run log against the reference's own logger.py."""
 import contextlib
 import io
+import json
 import os
 import sys
 
@@ -14,6 +15,7 @@ from oracle import refshim
 from edge_proposal_sets_b200 import autograd, train_step
 from edge_proposal_sets_b200.graph import SparseAdj, add_edges
 from edge_proposal_sets_b200.rank_step import RunLog
+from util import GOLDEN
 
 
 def _graph(n=60, m=200, seed=0, dataset="x"):
@@ -81,6 +83,28 @@ def test_link_loss_formula():
     assert float(train_step.link_loss(p, q)) == pytest.approx(want, rel=1e-6)
 
 
+def test_runlog_prints_the_stored_logger_output():
+    """RunLog on the results stored in tests/golden/runlog.json prints what the file says and takes the same curve
+    point.  The file records its source: written from RunLog itself, because the reference's logger.py was not
+    available then, it pins RunLog's output on every checkout; the test below ties it to the reference."""
+    gold = json.load(open(os.path.join(GOLDEN, "runlog.json")))
+    ours = RunLog(len(gold["results"]))
+    for run, rows in enumerate(gold["results"]):
+        for r in rows:
+            ours.add_result(run, r)
+
+    def cap(*a):
+        buf = io.StringIO()
+        with contextlib.redirect_stdout(buf):
+            ours.print_statistics(*a)
+        return buf.getvalue()
+    for run in range(len(gold["results"])):
+        assert cap(run) == gold["printed"][str(run)]
+    assert cap() == gold["printed"]["all"]
+    cp = ours.curve_point(1, 77)
+    assert [cp[0], float(cp[1]), float(cp[2])] == gold["curve_point_run1"]
+
+
 @pytest.mark.skipif(not refshim.available(), reason="/root/reference not present")
 def test_runlog_prints_what_the_reference_logger_prints():
     sys.path.insert(0, refshim.REFERENCE_ROOT)
@@ -107,3 +131,8 @@ def test_runlog_prints_what_the_reference_logger_prints():
     am = res[:, 1].argmax().item()
     cp = ours.curve_point(1, 77)
     assert cp[0] == 77 and float(cp[1]) == float(res[am, 1]) and float(cp[2]) == float(res[am, 2])
+    from oracle.make_golden_models import runlog_vectors
+    want = runlog_vectors(ref_logger.Logger, "")
+    gold = json.load(open(os.path.join(GOLDEN, "runlog.json")))
+    for key in ("results", "printed", "curve_point_run1"):
+        assert gold[key] == want[key], f"tests/golden/runlog.json differs from the reference ({key}): python -m oracle.make_golden_models"

@@ -10,7 +10,11 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def load_golden(name):
-    return np.load(os.path.join(GOLDEN, f"{name}.npz"))
+    """The arrays of tests/golden/{name}.npz (graph split, whole-set checksums) and {name}_sample.npz (the
+    reference's scores on a seeded sample of candidates), in one mapping."""
+    z = dict(np.load(os.path.join(GOLDEN, f"{name}.npz")))
+    z.update(np.load(os.path.join(GOLDEN, f"{name}_sample.npz")))
+    return z
 
 
 def undirected(train, n):
