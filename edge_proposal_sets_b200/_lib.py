@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libeps_b200.so")
 
 EPS_OK = 0
-EPS_VERSION = 201          # must equal EPS_VERSION in include/eps.h (checked by load())
+EPS_VERSION = 202          # must equal EPS_VERSION in include/eps.h (checked by load())
 EPS_REDUCE_SUM, EPS_REDUCE_MEAN = 0, 1
 EPS_CN_SIGMOID, EPS_CN_GROUPED_BY_V = 1, 2
 EPS_MLP_FP32, EPS_MLP_TC_F16 = 0, 1
@@ -46,6 +46,9 @@ SIGNATURES = {
     "eps_threshold_workspace_bytes": (_sz, [_i64]),
     "eps_threshold_count": (_int, [_vp, _i64, _vp, C.c_float, _int, _vp, _vp, _sz, _vp]),
     "eps_threshold_write": (_int, [_vp, _vp, _vp, _i64, _vp, C.c_float, _int, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "eps_segment_topk_workspace_bytes": (_sz, [_i64]),
+    "eps_segment_topk_select": (_int, [_vp, _i64, _vp, _i64, _i64, C.c_float, _int, _vp, _vp, _sz, _vp]),
+    "eps_segment_topk_write": (_int, [_vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "eps_gather_pairs2": (_int, [_vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _vp]),
     "eps_twohop_candidates": (_int, [_vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "eps_twohop_workspace_bytes": (_sz, []),

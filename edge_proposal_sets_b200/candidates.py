@@ -123,17 +123,20 @@ def _onepass(adj: SparseAdj, wtable, v_lo: int, v_hi: int, bounds, sigmoid: bool
 
 
 def two_hop(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, counts: torch.Tensor | None = None,
-            cap: int | None = None):
+            cap: int | None = None, want_offsets: bool = False):
     """(u, v) candidate list of owners [v_lo, v_hi): int32 [2, N], column-major reference order.
     ``counts`` (from ``owner_counts``) selects the two-pass kernels; without it the one-pass kernel
     runs (no count pass) and the result is a [2, N] view of a buffer sized by the owner_bounds sum
-    (``cap`` = that sum, when the caller already has it on the host)."""
+    (``cap`` = that sum, when the caller already has it on the host).  ``want_offsets`` returns
+    ``(edges, offsets)``: offsets int64 [v_hi - v_lo + 1], owner v's candidates are
+    ``edges[:, offsets[v - v_lo]:offsets[v - v_lo + 1]]`` (the segments of ``ops.segment_topk``)."""
     _need_cuda(adj.col)
     lib = _lib.load()
     v_hi = adj.n if v_hi is None else v_hi
     if counts is None:
         # one pass: padded per-owner slots sized by owner_bounds, compacted by the finalize pass
-        return _onepass(adj, None, v_lo, v_hi, None, False, False, False, cap)[0]
+        r = _onepass(adj, None, v_lo, v_hi, None, False, False, False, cap)
+        return (r[0], r[3]) if want_offsets else r[0]
     offsets = torch.zeros(counts.numel() + 1, dtype=torch.int64, device=adj.device)
     torch.cumsum(counts, 0, out=offsets[1:])
     N = int(offsets[-1].item())
@@ -141,19 +144,19 @@ def two_hop(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, counts: torc
         raise EpsError(f"{N} candidates in one slab; split the owner range (see filter_step.iter_slabs)")
     edges = torch.empty((2, N), dtype=torch.int32, device=adj.device)
     if N == 0:
-        return edges
+        return (edges, offsets) if want_offsets else edges
     ws = _ws(lib.eps_twohop_workspace_bytes(), adj.device)
     check(lib.eps_twohop_candidates(_ptr(adj.rowptr), _ptr(adj.col), adj.n, v_lo, v_hi, _ptr(offsets), None,
                                     _ptr(edges[0]), _ptr(edges[1]), _ptr(ws), ws.numel(), _stream()),
           "eps_twohop_candidates")
     from . import ops as _ops
     _ops.LAUNCHES["n"] += 1
-    return edges
+    return (edges, offsets) if want_offsets else edges
 
 
 def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int = 0, v_hi: int | None = None,
                    counts: torch.Tensor | None = None, sigmoid: bool = False, want_count: bool = False,
-                   cap: int | None = None, use_values: bool = True):
+                   cap: int | None = None, use_values: bool = True, want_offsets: bool = False):
     """K6+K3 fused: the candidates of owners [v_lo, v_hi) AND their heuristic scores from one walk
     over the owners' 2-paths (``wtable=None`` -> CN count, else sum of ``wtable[k]`` over the common
     neighbours: AA with 1/log deg, RA with 1/deg).  Returns ``(edges int32 [2,N], score fp32 [N])``
@@ -161,7 +164,8 @@ def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int
     same pairs.  A weighted adjacency (collab, ``use_values``) contributes A[u,k]*(A[v,k]*wtable[k]) per
     2-path on the one-pass kernel; ``use_values=False`` ignores the values ('adamic', models.py:544-554).
     Without ``counts`` the one-pass kernel runs: no count pass, outputs are views of buffers sized by
-    the owner_bounds sum of the range."""
+    the owner_bounds sum of the range.  ``want_offsets`` appends the per-owner offsets (int64
+    [v_hi - v_lo + 1], as in ``two_hop``) to the returned tuple."""
     _need_cuda(adj.col, wtable)
     val = adj.val if use_values else None
     check_fixed_point_range(adj, wtable, use_values)
@@ -171,8 +175,9 @@ def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int
     lib = _lib.load()
     v_hi = adj.n if v_hi is None else v_hi
     if counts is None:
-        edges, score, count, _ = _onepass(adj, wtable, v_lo, v_hi, None, sigmoid, True, want_count, cap, val)
-        return (edges, score, count) if want_count else (edges, score)
+        edges, score, count, offsets = _onepass(adj, wtable, v_lo, v_hi, None, sigmoid, True, want_count, cap, val)
+        out = (edges, score, count) if want_count else (edges, score)
+        return out + (offsets,) if want_offsets else out
     offsets = torch.zeros(counts.numel() + 1, dtype=torch.int64, device=adj.device)
     torch.cumsum(counts, 0, out=offsets[1:])
     N = int(offsets[-1].item())
@@ -189,7 +194,8 @@ def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int
                                     _ptr(count), _ptr(ws), ws.numel(), _stream()), "eps_twohop_scored")
         from . import ops as _ops
         _ops.LAUNCHES["n"] += 2
-    return (edges, score, count) if want_count else (edges, score)
+    out = (edges, score, count) if want_count else (edges, score)
+    return out + (offsets,) if want_offsets else out
 
 
 def two_path_work(adj: SparseAdj) -> torch.Tensor:

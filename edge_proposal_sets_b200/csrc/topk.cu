@@ -769,3 +769,329 @@ extern "C" int eps_pack_edges(const int32_t *pair_u, const int32_t *pair_v, cons
   EPS_LAUNCH_CHECK();
   return EPS_OK;
 }
+
+
+// ---------------- K4c: segmented top-m select over owner slabs (per-node proposal budgets) ----------------
+// Segments are the owners of a slab: offsets[s] .. offsets[s+1] of the candidate list, contiguous and in candidate
+// order.  Per segment, the same three radix passes as K4 (11+11+10 bits, same keys, same tie rule) find the m-th key
+// T and r = how many elements equal to T are still needed; the write pass is K4's ordered compaction restricted to
+// the segment.  Band mode keeps every element whose key is <= threshold_last_key(T, margin, inclusive) — the bound of
+// K4b, so both prefilter paths round the same way.
+//   select: persistent CTAs take segments from a list with the large ones first (a hub left for last would be the tail
+//           of the launch); a segment of <= m elements passes through without a histogram, one of <= SEG_SMEM_KEYS
+//           keys is loaded into shared memory once, larger ones are streamed from L2 / HBM by every pass.
+//   scan:   the per-segment kept counts -> output offsets (the last entry is the survivor count the host reads).
+//   write:  persistent CTAs again; each copies its segment's survivors (u, v, score) in position order.
+namespace eps {
+
+constexpr int SEG_THREADS = 256;
+constexpr int SEG_SMEM_KEYS = 6144;          // 24 KB of keys next to the 8 KB histogram
+constexpr long long SEG_BIG = 16384;         // segments above this go to the front of the work list
+
+struct SegCtl {
+  uint32_t n_big, n_small, next_select, next_write;
+};
+
+__device__ __forceinline__ void seg_bounds(const long long *__restrict__ off, long long s, long long M,
+                                           long long &lo, long long &hi) {
+  lo = min(max(off[s], 0ll), M);
+  hi = min(max(off[s + 1], lo), M);
+}
+
+// work list: segments larger than SEG_BIG at the front, the others behind them (order inside a group is irrelevant:
+// every segment's result depends on its own elements only)
+__global__ void seg_order_kernel(const long long *__restrict__ off, long long n_seg, long long M, SegCtl *ctl,
+                                 uint32_t *__restrict__ order) {
+  const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n_seg) return;
+  long long lo, hi;
+  seg_bounds(off, s, M, lo, hi);
+  if (hi - lo > SEG_BIG) order[atomicAdd(&ctl->n_big, 1u)] = (uint32_t)s;
+  else order[n_seg - 1 - atomicAdd(&ctl->n_small, 1u)] = (uint32_t)s;
+}
+
+// one 256-thread block: the bin d of hist[NB] that holds the k_rem-th element (1-based) and cum = #elements in the
+// bins below d (topk_pick_kernel's search, inside the CTA that built the histogram)
+template <int NB>
+__device__ __forceinline__ void seg_pick(const uint32_t *hist, uint32_t k_rem, uint32_t *wtot, uint32_t *s_pick) {
+  constexpr int PER = NB / SEG_THREADS;
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  uint32_t c[PER], mine = 0;
+#pragma unroll
+  for (int q = 0; q < PER; ++q) { c[q] = hist[t * PER + q]; mine += c[q]; }
+  uint32_t inc = mine;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const uint32_t y = __shfl_up_sync(FULL, inc, d);
+    if (lane >= d) inc += y;
+  }
+  if (lane == 31) wtot[warp] = inc;
+  __syncthreads();
+  uint32_t base = 0;
+  for (int w = 0; w < warp; ++w) base += wtot[w];
+  const uint32_t before = base + inc - mine;
+  if (before < k_rem && k_rem <= before + mine) {
+    uint32_t cum = before;
+    int q = 0;
+    for (; q < PER - 1; ++q) {
+      if (cum + c[q] >= k_rem) break;
+      cum += c[q];
+    }
+    s_pick[0] = (uint32_t)(t * PER + q);
+    s_pick[1] = cum;
+  }
+  __syncthreads();
+}
+
+// one radix pass over a segment: histogram of the PASS digit of the keys inside the current prefix bucket, then the
+// bucket of the k_rem-th key.  Keys come from shared memory (small segments) or from `score` (hubs).
+template <int PASS>
+__device__ __forceinline__ void seg_pass(const float *__restrict__ seg, const uint32_t *keys_sh, long long n,
+                                         uint32_t *hist, uint32_t *wtot, uint32_t *s_pick, uint32_t &prefix,
+                                         uint32_t &k_rem) {
+  constexpr int NB = (PASS == 2) ? 1024 : 2048;
+  constexpr int SHIFT = (PASS == 0) ? 21 : (PASS == 1 ? 10 : 0);
+  for (int i = threadIdx.x; i < NB; i += SEG_THREADS) hist[i] = 0;
+  __syncthreads();
+  const int lane = lane_id();
+  for (long long b = 0; b < n; b += SEG_THREADS) {          // warp-uniform trip count
+    const long long i = b + threadIdx.x;
+    uint32_t key = 0;
+    bool ok = false;
+    if (i < n) {
+      key = keys_sh ? keys_sh[i] : score_key(__ldg(seg + i));
+      ok = pass_match<PASS>(key, prefix);
+    }
+    const unsigned part = __ballot_sync(FULL, ok);
+    if (part == 0) continue;
+    const uint32_t d = ok ? pass_digit<PASS>(key) : 0x10000u;
+    if (__popc(part) <= 8) {
+      if (ok) atomicAdd(&hist[d], 1u);
+    } else {                                                  // tie-heavy (CN) keys: one atomic per distinct digit
+      const unsigned peers = __match_any_sync(FULL, d);
+      if (ok && lane == (__ffs(peers) - 1)) atomicAdd(&hist[d], (uint32_t)__popc(peers));
+    }
+  }
+  __syncthreads();
+  seg_pick<NB>(hist, k_rem, wtot, s_pick);
+  prefix |= s_pick[0] << SHIFT;
+  k_rem -= s_pick[1];
+  __syncthreads();
+}
+
+// per segment: keep-rule (T, r) — keep key < T, and the first r keys == T — and the kept count
+__global__ void __launch_bounds__(SEG_THREADS)
+seg_select_kernel(const float *__restrict__ score, long long M, const long long *__restrict__ off, long long n_seg,
+                  uint32_t m, float margin, int band, SegCtl *ctl, const uint32_t *__restrict__ order,
+                  uint32_t *__restrict__ seg_T, uint32_t *__restrict__ seg_r, uint32_t *__restrict__ count) {
+  __shared__ uint32_t hist[2048];
+  __shared__ uint32_t keys_sh[SEG_SMEM_KEYS];
+  __shared__ uint32_t wtot[SEG_THREADS / 32], s_pick[2], s_item, s_cnt;
+  for (;;) {
+    if (threadIdx.x == 0) s_item = atomicAdd(&ctl->next_select, 1u);
+    __syncthreads();
+    const uint32_t item = s_item;
+    __syncthreads();
+    if (item >= n_seg) return;
+    const long long s = order[item];
+    long long lo, hi;
+    seg_bounds(off, s, M, lo, hi);
+    const long long n = hi - lo;
+    if (n <= (long long)m) {                                  // the whole segment is kept
+      if (threadIdx.x == 0) { seg_T[s] = 0xffffffffu; seg_r[s] = 0xffffffffu; count[s] = (uint32_t)n; }
+      continue;
+    }
+    const float *seg = score + lo;
+    const uint32_t *ks = nullptr;
+    if (n <= SEG_SMEM_KEYS) {
+      for (long long i = threadIdx.x; i < n; i += SEG_THREADS) keys_sh[i] = score_key(__ldg(seg + i));
+      ks = keys_sh;
+      __syncthreads();
+    }
+    uint32_t prefix = 0, k_rem = m;
+    seg_pass<0>(seg, ks, n, hist, wtot, s_pick, prefix, k_rem);
+    seg_pass<1>(seg, ks, n, hist, wtot, s_pick, prefix, k_rem);
+    seg_pass<2>(seg, ks, n, hist, wtot, s_pick, prefix, k_rem);
+    if (!band) {
+      if (threadIdx.x == 0) { seg_T[s] = prefix; seg_r[s] = k_rem; count[s] = m; }
+      continue;
+    }
+    const uint32_t last = threshold_last_key(prefix, margin, 1);
+    if (threadIdx.x == 0) s_cnt = 0;
+    __syncthreads();
+    uint32_t c = 0;
+    for (long long i = threadIdx.x; i < n; i += SEG_THREADS)
+      c += (ks ? ks[i] : score_key(__ldg(seg + i))) <= last;
+#pragma unroll
+    for (int o = 16; o; o >>= 1) c += __shfl_xor_sync(FULL, c, o);
+    if (lane_id() == 0 && c) atomicAdd(&s_cnt, c);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      seg_T[s] = last == 0xffffffffu ? last : last + 1;       // key <= last  <=>  key < last + 1
+      seg_r[s] = last == 0xffffffffu ? last : 0u;
+      count[s] = s_cnt;
+    }
+  }
+}
+
+// per segment: its survivors, in position order, at out_off[s] (K4's ordered compaction inside the segment)
+__global__ void __launch_bounds__(SEG_THREADS)
+seg_write_kernel(const float *__restrict__ score, const int *__restrict__ pu, const int *__restrict__ pv, long long M,
+                 const long long *__restrict__ off, long long n_seg, SegCtl *ctl, const uint32_t *__restrict__ order,
+                 const uint32_t *__restrict__ seg_T, const uint32_t *__restrict__ seg_r,
+                 const uint32_t *__restrict__ out_off, int *__restrict__ out_u, int *__restrict__ out_v,
+                 float *__restrict__ out_score) {
+  __shared__ uint32_t wsum[SEG_THREADS / 32];
+  __shared__ uint32_t s_tot, s_item;
+  const int lane = lane_id(), warp = threadIdx.x >> 5;
+  const ScoreSrc src{nullptr, 0, score};
+  for (;;) {
+    if (threadIdx.x == 0) s_item = atomicAdd(&ctl->next_write, 1u);
+    __syncthreads();
+    const uint32_t item = s_item;
+    __syncthreads();
+    if (item >= n_seg) return;
+    const long long s = order[item];
+    const uint32_t obase = out_off[s];
+    if (out_off[s + 1] == obase) continue;
+    long long lo, hi;
+    seg_bounds(off, s, M, lo, hi);
+    const uint32_t T = seg_T[s], r = seg_r[s];
+    uint32_t run_less = 0, run_eq = 0;
+    for (long long sub = lo; sub < hi; sub += SEG_THREADS * 4) {
+      const long long i0 = sub + (long long)threadIdx.x * 4;
+      float v4[4];
+      src.load4(i0, hi, v4);
+      uint32_t cls[4], mine = 0;                              // 1 = less, 0x10000 = eq
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        cls[q] = 0;
+        if (i0 + q < hi) {
+          const uint32_t key = score_key(v4[q]);
+          cls[q] = key < T ? 1u : (key == T ? 0x10000u : 0u);
+        }
+        mine += cls[q];
+      }
+      uint32_t inc = mine;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t t = __shfl_up_sync(FULL, inc, d);
+        if (lane >= d) inc += t;
+      }
+      if (lane == 31) wsum[warp] = inc;
+      __syncthreads();
+      if (threadIdx.x == 0) {
+        uint32_t acc = 0;
+        for (int w = 0; w < SEG_THREADS / 32; ++w) { const uint32_t v = wsum[w]; wsum[w] = acc; acc += v; }
+        s_tot = acc;
+      }
+      __syncthreads();
+      const uint32_t ex = wsum[warp] + inc - mine;
+      uint32_t lb = run_less + (ex & 0xffffu), eb = run_eq + (ex >> 16);
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        long long pos = -1;
+        if (cls[q] == 1u) { pos = lb + min(eb, r); ++lb; }
+        else if (cls[q] == 0x10000u) { if (eb < r) pos = lb + eb; ++eb; }
+        if (pos >= 0) {
+          const long long o = obase + pos;
+          out_u[o] = pu[i0 + q];
+          out_v[o] = pv[i0 + q];
+          out_score[o] = v4[q];
+        }
+      }
+      const uint32_t tot = s_tot;
+      run_less += tot & 0xffffu;
+      run_eq += tot >> 16;
+      __syncthreads();
+    }
+  }
+}
+
+struct SegLayout {
+  size_t ctl, order, T, r, scan_tmp, total;
+};
+
+static SegLayout seg_layout(int64_t n_seg) {
+  SegLayout L;
+  const size_t ns = (size_t)std::max<int64_t>(n_seg, 1);
+  size_t o = 0;
+  L.ctl = o; o += 256;
+  L.order = o; o += align256(ns * 4);
+  L.T = o; o += align256(ns * 4);
+  L.r = o; o += align256(ns * 4);
+  L.scan_tmp = o; o += align256(2 * ((ns + 1 + SCAN_CHUNK - 1) / SCAN_CHUNK + 1) * 4);
+  L.total = o;
+  return L;
+}
+
+static int seg_grid(int64_t n_seg) {
+  return (int)std::max<long long>(1, std::min<long long>(n_seg, (long long)sm_count() * 4));
+}
+
+}  // namespace eps
+
+extern "C" size_t eps_segment_topk_workspace_bytes(int64_t n_seg) {
+  return eps::seg_layout(n_seg < 0 ? 0 : n_seg).total;
+}
+
+extern "C" int eps_segment_topk_select(const float *score, int64_t M, const int64_t *seg_offsets, int64_t n_seg,
+                                       int64_t m, float margin, int band, uint32_t *out_offsets, void *workspace,
+                                       size_t workspace_bytes, void *stream_) {
+  using namespace eps;
+  EPS_CHECK_ARG(M >= 0 && M < 0xffffffffll, "M out of range [0, 2^32-1)");
+  EPS_CHECK_ARG(n_seg >= 0 && n_seg < 0xffffffffll, "n_seg out of range [0, 2^32-1)");
+  EPS_CHECK_ARG(m >= 1 && m < 0xffffffffll, "m out of range [1, 2^32-1)");
+  EPS_CHECK_ARG(out_offsets != nullptr && workspace != nullptr, "null pointer (out_offsets / workspace)");
+  EPS_CHECK_ARG(n_seg == 0 || seg_offsets != nullptr, "null pointer (seg_offsets)");
+  EPS_CHECK_ARG(M == 0 || score != nullptr, "null pointer (score)");
+  EPS_CHECK_ARG(n_seg > 0 || M == 0, "inconsistent offsets: M > 0 elements in no segment");
+  EPS_CHECK_ARG(!band || margin >= 0.f, "band mode needs margin >= 0");
+  const SegLayout L = seg_layout(n_seg);
+  if (workspace_bytes < L.total) {
+    set_error("eps_segment_topk_select: workspace too small (%zu < %zu)", workspace_bytes, L.total);
+    return EPS_ERR_WORKSPACE;
+  }
+  cudaStream_t stream = (cudaStream_t)stream_;
+  if (sm_count() <= 0) { set_error("eps_segment_topk_select: no CUDA device"); return EPS_ERR_CUDA; }
+  char *ws = (char *)workspace;
+  SegCtl *ctl = (SegCtl *)(ws + L.ctl);
+  uint32_t *order = (uint32_t *)(ws + L.order);
+  EPS_CUDA(cudaMemsetAsync(ctl, 0, sizeof(SegCtl), stream));
+  EPS_CUDA(cudaMemsetAsync(out_offsets + n_seg, 0, 4, stream));
+  if (n_seg == 0) return EPS_OK;
+  const long long *off = (const long long *)seg_offsets;
+  seg_order_kernel<<<(unsigned)((n_seg + 255) / 256), 256, 0, stream>>>(off, n_seg, M, ctl, order);
+  seg_select_kernel<<<seg_grid(n_seg), SEG_THREADS, 0, stream>>>(
+      score, M, off, n_seg, (uint32_t)m, margin, band, ctl, order, (uint32_t *)(ws + L.T),
+      (uint32_t *)(ws + L.r), out_offsets);
+  scan_exclusive(out_offsets, nullptr, n_seg + 1, (uint32_t *)(ws + L.scan_tmp), stream);
+  EPS_LAUNCH_CHECK();
+  return EPS_OK;
+}
+
+extern "C" int eps_segment_topk_write(const float *score, const int32_t *pair_u, const int32_t *pair_v, int64_t M,
+                                      const int64_t *seg_offsets, int64_t n_seg, const uint32_t *out_offsets,
+                                      int32_t *out_u, int32_t *out_v, float *out_score, void *workspace,
+                                      size_t workspace_bytes, void *stream_) {
+  using namespace eps;
+  EPS_CHECK_ARG(M >= 0 && M < 0xffffffffll, "M out of range [0, 2^32-1)");
+  EPS_CHECK_ARG(n_seg >= 0 && n_seg < 0xffffffffll, "n_seg out of range [0, 2^32-1)");
+  EPS_CHECK_ARG(n_seg > 0 || M == 0, "inconsistent offsets: M > 0 elements in no segment");
+  if (n_seg == 0) return EPS_OK;
+  EPS_CHECK_ARG(score && pair_u && pair_v && seg_offsets && out_offsets && workspace, "null pointer (inputs)");
+  EPS_CHECK_ARG(out_u && out_v && out_score, "null pointer (outputs)");
+  const SegLayout L = seg_layout(n_seg);
+  if (workspace_bytes < L.total) {
+    set_error("eps_segment_topk_write: workspace too small (%zu < %zu)", workspace_bytes, L.total);
+    return EPS_ERR_WORKSPACE;
+  }
+  cudaStream_t stream = (cudaStream_t)stream_;
+  char *ws = (char *)workspace;
+  seg_write_kernel<<<seg_grid(n_seg), SEG_THREADS, 0, stream>>>(
+      score, pair_u, pair_v, M, (const long long *)seg_offsets, n_seg, (SegCtl *)(ws + L.ctl),
+      (const uint32_t *)(ws + L.order), (const uint32_t *)(ws + L.T), (const uint32_t *)(ws + L.r), out_offsets,
+      out_u, out_v, out_score);
+  EPS_LAUNCH_CHECK();
+  return EPS_OK;
+}

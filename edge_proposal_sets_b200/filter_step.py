@@ -300,12 +300,12 @@ def tc_arm_supported(model) -> bool:
 @torch.no_grad()
 def filter_topk_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: int = 1 << 27,
                       distributed: bool = False, stats: Optional[dict] = None, pushdown: bool = True,
-                      owners: Optional[Tuple[int, int]] = None):
+                      owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None):
     """``_filter_multi`` (see there) with the prefilter's safety net: when a job's tensor-core scores leave the
     calibrated tolerance, or its band cannot prune, the call is repeated with that job on the fp32 arm."""
     jobs = [j if isinstance(j, FilterJob) else FilterJob(*j) for j in jobs]
     try:
-        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners)
+        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners, per_node)
     except PrefilterToleranceError as exc:
         import warnings
         warnings.warn(f"{exc}; re-running the filter step on the fp32 arm")
@@ -314,13 +314,13 @@ def filter_topk_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pai
                 j.precision = "fp32"
         if stats is not None:
             stats["prefilter_fallback"] = str(exc)
-        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners)
+        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners, per_node)
 
 
 @torch.no_grad()
 def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: int = 1 << 27,
                   distributed: bool = False, stats: Optional[dict] = None, pushdown: bool = True,
-                  owners: Optional[Tuple[int, int]] = None):
+                  owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None):
     """The filter step for several filter models over ONE enumeration of the 2-hop candidates: a list of
     sorted proposal lists (float32 ``[k,3]`` rows (u, v, score) on the device; score descending, ties by
     the reference's candidate order), one per job.  ``k=None`` keeps every candidate like the reference.
@@ -336,8 +336,26 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
     a violation, or a band so wide that it cannot prune, raises ``PrefilterToleranceError``
     (``filter_topk_multi`` then re-runs the call with the job on the fp32 arm).
 
-    ``owners=(lo, hi)`` restricts the candidates to those owned by v in [lo, hi) (a sample of the job)."""
+    ``owners=(lo, hi)`` restricts the candidates to those owned by v in [lo, hi) (a sample of the job).
+
+    ``per_node=m`` (per-node proposal budgets): only the m best candidates (u, v) of every owner v — score
+    descending, ties by u ascending — take part; the list is then ordered by the same rule and cut to k (``k=None``
+    keeps every owner's m).  The budget is per v, the second column of a row: keeping (u, v) in v's list says nothing
+    about (v, u) in u's list (``add_edges`` symmetrises the graph, so either adds the undirected edge).  An owner's
+    candidates are contiguous inside one slab, so K4c (``ops.segment_topk``) selects them slab by slab and its
+    survivors, still in candidate order, feed the unchanged running top-k.  With m >= every owner's candidate count
+    the result is the global list.  GNN jobs on the prefilter: per slab, the band select keeps every candidate whose
+    tensor-core score s16 is >= (its owner's m-th best s16) - 2 tol; the pool is re-scored in fp32, the tolerance
+    verified on it, and the exact per-owner select runs on the fp32 scores.  Sound because, with |s16 - s32| <= tol
+    for every pair, an owner's j-th best s32 is >= its j-th best s16 - tol for every j <= m (its j best candidates by
+    s16 all have s32 >= that value): a candidate with s16 < S16_m - 2 tol has s32 < S16_m - tol <= S32_m, strictly
+    below the owner's m-th best fp32 score, so it cannot be among the owner's exact m best.  No band is exchanged or
+    pruned across owners (each rank's per-owner lists are complete), and the prefilter stays on with ``k=None``:
+    the n * m budget bounds the pool."""
     rank, world = parallel.world_info() if distributed else (0, 1)
+    if per_node is not None and int(per_node) < 1:
+        raise ValueError(f"per_node must be >= 1 (got {per_node})")
+    m = None if per_node is None else int(per_node)
     if world > 1 and k is None:
         raise ValueError("distributed filter needs a proposal size k")
     jobs = [j if isinstance(j, FilterJob) else FilterJob(*j) for j in jobs]
@@ -356,34 +374,43 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
             prec = j.precision
             if prec in ("prefilter", "f16", "bf16", "tc") and not tc_arm_supported(j.model):
                 prec = "fp32"                                # shapes the tcgen05 arm is not built for (H=300)
-            if prec == "prefilter" and k is None:
+            if prec == "prefilter" and k is None and m is None:
                 prec = "fp32"                                # keeping every candidate: nothing to prefilter
             h = j.model.embed(x, adj, distributed=world > 1)
+            band = prec == "prefilter" and m is None
             plans.append(dict(kind="gnn", prec=prec, h=h, ctx=None if prec == "fp32" else j.model.linkpred.tc_context(h),
-                              tol=None, cal=None,
-                              run=RunningTopK(k, 2.0 * PREFILTER_TOL if prec == "prefilter" else None, pushdown)))
+                              tol=None, cal=None, pn_kept=0,
+                              pool=dict(e=[], s=[], cnt=[], size=0, owners=0, budget=None, overflow=False)
+                              if (prec == "prefilter" and m is not None) else None,
+                              run=RunningTopK(k, 2.0 * PREFILTER_TOL if band else None, pushdown)))
         else:
             table = heuristic_table(j.name, adj, j.ra_adj)
             if table is not None and fused_job is None:
                 fused_job = len(plans)
-            plans.append(dict(kind="heuristic", table=table, run=RunningTopK(k, None, pushdown)))
+            plans.append(dict(kind="heuristic", table=table, pn_kept=0, pool=None, run=RunningTopK(k, None, pushdown)))
     ph.mark("embed")
     n_slabs = 0
+    n_cand = 0
     for lo, hi, cap in iter_slabs(adj, v_lo, v_hi, slab_pairs):
         n_slabs += 1
         scores = {}
+        offsets = None
         if fused_job is not None:
             # CN / AA / RA are the values of A@A: one walk over the owners' 2-paths yields the
             # candidates and their scores together (bit-identical to scoring the pairs with K3)
             t = plans[fused_job]["table"]
-            edges, scores[fused_job] = candidates.two_hop_scored(t[0], t[1], lo, hi, sigmoid=t[2], cap=cap,
-                                                                 use_values=t[3])
+            r = candidates.two_hop_scored(t[0], t[1], lo, hi, sigmoid=t[2], cap=cap, use_values=t[3],
+                                          want_offsets=m is not None)
+            edges, scores[fused_job] = r[0], r[1]
+            offsets = r[2] if m is not None else None
             ph.mark("enum_score")
         else:
-            edges = candidates.two_hop(adj, lo, hi, cap=cap)
+            r = candidates.two_hop(adj, lo, hi, cap=cap, want_offsets=m is not None)
+            edges, offsets = r if m is not None else (r, None)
             ph.mark("enum")
         if edges.shape[1] == 0:
             continue
+        n_cand += edges.shape[1]
         for i, (j, p) in enumerate(zip(jobs, plans)):
             if i in scores:
                 continue
@@ -397,16 +424,24 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
             else:
                 scores[i] = score_edges(j.name, j.model, x, adj, edges, True, j.ra_adj)
                 ph.mark("score")
-        for i, p in enumerate(plans):
-            p["run"].update(edges, scores[i])
-        ph.mark("topk")
-        del edges, scores
+        if m is None:
+            for i, p in enumerate(plans):
+                p["run"].update(edges, scores[i])
+            ph.mark("topk")
+        else:
+            _per_node_slab(plans, edges, scores, offsets, m, hi - lo, ph)
+        del edges, scores, offsets
     out = []
     for j, p in zip(jobs, plans):
         run = p["run"]
         if p["kind"] == "gnn" and p["prec"] == "prefilter" and p["tol"] is None:
             _calibrate(j.model, p, None, None, world)        # this rank owned no candidates: still one collective
-        if p["kind"] == "gnn" and p["prec"] == "prefilter":
+        if p["pool"] is not None:
+            res, info = _rescore_pool_per_node(j.model, p["h"], p["pool"], k, m, world, p["tol"], p["cal"])
+            if stats is not None:
+                stats.setdefault("prefilter", {})[j.name] = info
+            ph.mark("rescore")
+        elif p["kind"] == "gnn" and p["prec"] == "prefilter":
             res, info = _rescore_pool(j.model, p["h"], run, k, world, p["tol"], p["cal"])
             if stats is not None:
                 stats.setdefault("prefilter", {})[j.name] = info
@@ -419,7 +454,9 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
             ph.mark("merge")
         out.append(res)
     if stats is not None:
-        stats["candidates_scored"] = plans[0]["run"].seen if plans else 0
+        stats["candidates_scored"] = (plans[0]["run"].seen if m is None else n_cand) if plans else 0
+        if m is not None:
+            stats["per_node"] = dict(m=m, survivors=[p["pn_kept"] for p in plans])
         stats["slabs"] = n_slabs
         stats["owners"] = [v_lo, v_hi]
         stats["pushdown_survivors"] = [p["run"].survivors for p in plans]
@@ -427,6 +464,77 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
             torch.cuda.synchronize()
             stats["phase_ms"] = ph.totals()
     return out
+
+
+def _per_node_slab(plans, edges, scores, offsets, m: int, n_owners: int, ph) -> None:
+    """Per-node mode, one slab: K4c per job — the exact per-owner top-m, or for a prefilter job the band of every
+    owner's m-th tensor-core score, appended to the job's pool — then the exact survivors into the running top-k."""
+    kept = []
+    for i, p in enumerate(plans):
+        pool = p["pool"]
+        if pool is not None and pool["overflow"]:
+            kept.append(None)
+            continue
+        margin = None if pool is None else 2.0 * p["tol"]
+        kept.append(ops.segment_topk(scores[i], edges, offsets, m, margin=margin))
+        p["pn_kept"] += kept[-1][1].numel()
+        if pool is not None:
+            b = torch.clamp(offsets[1:] - offsets[:-1], max=m).sum()     # this slab's exact budget, on the device
+            pool["budget"] = b if pool["budget"] is None else pool["budget"] + b
+    ph.mark("per_node")
+    for p, kp in zip(plans, kept):
+        if kp is None:
+            continue
+        e, s, off = kp
+        pool = p["pool"]
+        if pool is None:
+            p["run"].update(e, s)
+            continue
+        pool["e"].append(e)
+        pool["s"].append(s)
+        pool["cnt"].append(off[1:] - off[:-1])
+        pool["size"] += s.numel()
+        pool["owners"] += n_owners
+        if pool["size"] > max(PREFILTER_POOL_CAP, 4 * m * pool["owners"]):
+            # the band holds more than 4x every owner's budget: it cannot prune (decided collectively at the end)
+            pool.update(e=[], s=[], cnt=[], overflow=True)
+    ph.mark("topk")
+
+
+def _rescore_pool_per_node(model, h, pool, k: Optional[int], m: int, world: int, tol: float, cal=None):
+    """Per-node prefilter epilogue: fp32 scores of the pool, tolerance check on it, exact per-owner top-m of the fp32
+    scores (K4c over the pool's owner segments), then the first k rows by score.  No exchange between ranks but the
+    decision flags: owners are partitioned, so every rank's pool holds its owners' complete bands."""
+    dev = h.device
+    margin = 2.0 * tol
+    P = pool["size"] if not pool["overflow"] else 0
+    budget = 0 if pool["budget"] is None else int(pool["budget"].item())
+    overflow = pool["overflow"] or P > max(PREFILTER_POOL_CAP, 4 * budget)
+    info = dict(m=int(m), k=None if k is None else int(k), pool=int(pool["size"]), budget=budget, tol=tol,
+                margin=margin, tol_ceiling=PREFILTER_TOL, calibration=cal, band_occupancy=float(P) / max(budget, 1))
+    res = torch.empty((0, 3), dtype=torch.float32, device=dev)
+    flags = torch.zeros(2, dtype=torch.float32, device=dev)       # [max deviation on the pool, pool overflow]
+    if P and not overflow:
+        edges, s16, cnt = torch.cat(pool["e"], 1), torch.cat(pool["s"]), torch.cat(pool["cnt"])
+        s32 = model.linkpred.score_pairs(h, edges, "fp32")
+        flags[0] = (s32 - s16).abs().max()
+        off = torch.zeros(cnt.numel() + 1, dtype=torch.int64, device=dev)
+        torch.cumsum(cnt, 0, out=off[1:])
+        e, s, _ = ops.segment_topk(s32, edges, off, m)
+        res = ops.topk_edges(e, s, s.numel() if k is None else min(int(k), s.numel()))
+    pool.update(e=[], s=[], cnt=[])
+    flags[1] = 1.0 if overflow else 0.0
+    if world > 1:                                            # every rank must take the same decision
+        torch.distributed.all_reduce(flags, op=torch.distributed.ReduceOp.MAX)
+    info["max_abs_dev_tc_vs_fp32"] = float(flags[0].item())
+    if float(flags[1].item()) > 0:
+        raise PrefilterToleranceError(f"the per-node prefilter band (margin {margin:.2e}) holds more than "
+                                      f"{max(PREFILTER_POOL_CAP, 4 * budget)} candidates: this model's scores are too "
+                                      "close together for a reduced-precision prefilter")
+    if not info["max_abs_dev_tc_vs_fp32"] <= tol:
+        raise PrefilterToleranceError(f"tensor-core prefilter scores deviate {info['max_abs_dev_tc_vs_fp32']:.3e} from fp32 "
+                                      f"on the pool (> calibrated tolerance {tol:.2e})")
+    return res, info
 
 
 def _calibrate(model, plan, edges, s16, world: int) -> None:
@@ -493,12 +601,13 @@ def _rescore_pool(model, h, run: RunningTopK, k: int, world: int, tol: float, ca
 def filter_topk(model_name: str, model, x, adj: SparseAdj, k: Optional[int] = None,
                 slab_pairs: int = 1 << 27, distributed: bool = False, ra_adj: Optional[SparseAdj] = None,
                 stats: Optional[dict] = None, precision: Optional[str] = None,
-                owners: Optional[Tuple[int, int]] = None) -> torch.Tensor:
+                owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None) -> torch.Tensor:
     """Sorted proposal list of one filter model, float32 ``[k,3]`` rows (u, v, score) on the device: score
     descending, ties by the reference's candidate order.  ``k=None`` keeps every candidate like the
-    reference.  ``precision`` (GNN models): see ``FilterJob``; default = the model's ``linkpred.precision``."""
+    reference.  ``precision`` (GNN models): see ``FilterJob``; default = the model's ``linkpred.precision``.
+    ``per_node=m``: only the m best candidates of every owner v (see ``_filter_multi``)."""
     job = FilterJob(model_name, model, ra_adj, precision)
-    return filter_topk_multi([job], x, adj, k, slab_pairs, distributed, stats, owners=owners)[0]
+    return filter_topk_multi([job], x, adj, k, slab_pairs, distributed, stats, owners=owners, per_node=per_node)[0]
 
 
 def load_extra_edges(path: str, num_sorted_edge: int) -> torch.Tensor:

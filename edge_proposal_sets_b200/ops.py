@@ -374,3 +374,46 @@ def gather_pairs2(pairs_a, pairs_b, idx: torch.Tensor):
                                 _stream()), "eps_gather_pairs2")
     LAUNCHES["n"] += 1 if k else 0
     return ou, ov
+
+
+def segment_topk(score: torch.Tensor, edges: torch.Tensor, offsets: torch.Tensor, m: int,
+                 margin: Optional[float] = None):
+    """K4c.  Per-segment top-m of ``score`` with segments ``offsets`` (int64 [S+1], device; an owner slab's
+    per-owner offsets): ``(edges int32 [2,R], score fp32 [R], kept offsets int64 [S+1])``, the survivors in
+    position order.  ``margin=None``: the m best of every segment (score descending, ties by position); a number:
+    every element with score >= (the segment's m-th best score) - margin (the prefilter band, bounded like K4b's
+    ``threshold_compact``).  One host sync (the survivor count sizes the outputs)."""
+    _need_cuda(score, edges, offsets)
+    lib = _lib.load()
+    m = int(m)
+    if m < 1:
+        raise EpsError(f"segment_topk: m must be >= 1 (got {m})")
+    dev = score.device
+    score = score.contiguous().float()
+    M = score.numel()
+    pu, pv = _pairs(edges)
+    if pu.numel() != M:
+        raise EpsError(f"segment_topk: {pu.numel()} pairs for {M} scores")
+    if offsets.dim() != 1 or offsets.numel() < 1:
+        raise EpsError("segment_topk: offsets must be a 1-D tensor of n_seg + 1 entries")
+    off = offsets.contiguous().to(torch.int64)
+    n_seg = off.numel() - 1
+    kept32 = torch.empty(n_seg + 1, dtype=torch.int32, device=dev)     # uint32 payload
+    ws = _ws(lib.eps_segment_topk_workspace_bytes(n_seg), dev)
+    band = margin is not None
+    ev = _event_pair("segment_topk")
+    check(lib.eps_segment_topk_select(_ptr(score), M, _ptr(off), n_seg, m, float(margin or 0.0), int(band),
+                                      _ptr(kept32), _ptr(ws), ws.numel(), _stream()), "eps_segment_topk_select")
+    LAUNCHES["n"] += (3 + (2 if n_seg + 1 > 8192 else 0)) if n_seg else 0
+    kept = kept32.long() & 0xFFFFFFFF
+    R = int(kept[-1].item())
+    out = torch.empty((2, R), dtype=torch.int32, device=dev)
+    osc = torch.empty(R, dtype=torch.float32, device=dev)
+    if R:
+        check(lib.eps_segment_topk_write(_ptr(score), _ptr(pu), _ptr(pv), M, _ptr(off), n_seg, _ptr(kept32),
+                                         _ptr(out[0]), _ptr(out[1]), _ptr(osc), _ptr(ws), ws.numel(), _stream()),
+              "eps_segment_topk_write")
+        LAUNCHES["n"] += 1
+    if ev is not None:
+        ev[1].record()
+    return out, osc, kept

@@ -17,6 +17,11 @@ Differences from the reference, all on the fast side of the same semantics:
   * with ``--topk`` a GNN filter scores every candidate on the tcgen05 tensor cores (fp16 operands) and
     re-scores the band around the k-th score in fp32: the saved list is the fp32 list, bit for bit
     (``--mlp_precision``, filter_step.filter_topk_multi);
+  * ``--per_node_topk M`` keeps only the M best candidates (u, v) of every node v (score descending, ties by u):
+    every node gets proposals, not just the neighbourhoods of the hubs, and the list has at most n * M rows.  The
+    kept rows are ordered like the global list (and cut to ``--topk`` when given), so the file is read the same way.
+    The budget belongs to v, the second column; (v, u) need not be in u's list (the rank graph is symmetrised, so
+    either row adds the undirected edge);
   * under ``torchrun`` the owners are sharded across the GPUs and merged with one all-gather.
 """
 from __future__ import annotations
@@ -26,6 +31,13 @@ import os
 from pathlib import Path
 
 import torch
+
+
+def _budget(text: str) -> int:
+    m = int(text)
+    if m < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1 (got {m})")
+    return m
 
 
 def parse_args(argv=None):
@@ -49,6 +61,9 @@ def parse_args(argv=None):
                    help="GNN filters: 'prefilter' = tcgen05 fp16-operand scores select a band around the top-k that is "
                         "re-scored in fp32 (the fp32 list, bit for bit); 'fp32' = FFMA arm for every candidate; "
                         "'f16' (alias 'bf16') = tensor-core scores only (approximate list)")
+    p.add_argument("--per_node_topk", type=_budget, default=None, metavar="M",
+                   help="per-node proposal budget: keep only the M best candidates (u, v) of every node v, then order "
+                        "them like the global list (and keep the first --topk rows when given); default: off")
     p.add_argument("--slab_pairs", type=int, default=1 << 27)
     p.add_argument("--random_init", action="store_true",
                    help="score with seeded random weights when models/{checkpoint} does not exist")
@@ -109,7 +124,8 @@ def main(argv=None):
     if distributed and k is None:
         raise SystemExit("filter.py: --topk is required under torchrun (only top-k lists are merged)")
     sorted_edges = filter_step.filter_topk(args.model, model, data.x, data.adj_t, k=k, slab_pairs=args.slab_pairs,
-                                           distributed=distributed, ra_adj=ra_adj, stats=stats).cpu()
+                                           distributed=distributed, ra_adj=ra_adj, stats=stats,
+                                           per_node=args.per_node_topk).cpu()
     print(f"using {stats.get('candidates_scored')} edges" + (" (this rank)" if distributed else ""))
     if rank == 0:
         print(sorted_edges)

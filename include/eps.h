@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define EPS_VERSION 201 /* 0.2.1; edge_proposal_sets_b200/_lib.py checks it at load time */
+#define EPS_VERSION 202 /* 0.2.2; edge_proposal_sets_b200/_lib.py checks it at load time */
 
 typedef enum {
   EPS_OK = 0,
@@ -234,6 +234,42 @@ int eps_threshold_write(const float *score, const int32_t *pair_u, const int32_t
                         const uint32_t *bound_key, float margin, int inclusive,
                         const uint32_t *tile_offsets, int32_t *out_u, int32_t *out_v, float *out_score,
                         uint32_t *out_pos, void *stream);
+
+/* ---------------------------------------------------------------------------
+ * K4c  segmented top-m select: per-owner proposal budgets
+ * replaces: no reference counterpart (the reference keeps a global sort,
+ *           filter.py:160-161); "the m best new edges of every node" from one
+ *           pass over each owner slab instead of a sort of all candidates.
+ * Segments are given by seg_offsets int64[n_seg + 1] (device): segment s is
+ * score[seg_offsets[s] .. seg_offsets[s+1]), nondecreasing, seg_offsets[0] == 0
+ * and seg_offsets[n_seg] == M (an owner slab's offsets_out of
+ * eps_twohop_onepass).  Keys and tie rule are K4's: score descending, ties by
+ * position ascending, -0.0 == +0.0.
+ *   band == 0 (exact): keep the m best elements of every segment (all of a
+ *              segment of <= m elements) - every element whose key is below the
+ *              segment's m-th key, plus the first r elements tied with it.
+ *   band != 0 : keep every element with score >= s_m - margin (margin >= 0,
+ *              s_m = the segment's m-th best score), bounded exactly as K4b's
+ *              inclusive threshold (one ulp of slack below the rounded
+ *              difference); a segment of <= m elements is kept whole.
+ *   select: out_offsets uint32[n_seg + 1] (caller-owned, device) = exclusive
+ *           scan of the per-segment kept counts; out_offsets[n_seg] is the
+ *           survivor count S, which the host reads to size the outputs.
+ *   write : the survivors (u, v, score) in POSITION ORDER, segment s at
+ *           out_offsets[s]; out_u / out_v / out_score hold S elements.
+ * The per-segment results of select live in the workspace
+ * (eps_segment_topk_workspace_bytes(n_seg) bytes, caller-owned) and are read
+ * by write: pass the same, unmodified workspace to both calls, in stream order.
+ * Requires M < 2^32 - 1, 1 <= m < 2^32 - 1.
+ * ------------------------------------------------------------------------- */
+size_t eps_segment_topk_workspace_bytes(int64_t n_seg);
+int eps_segment_topk_select(const float *score, int64_t M, const int64_t *seg_offsets, int64_t n_seg,
+                            int64_t m, float margin, int band, uint32_t *out_offsets, void *workspace,
+                            size_t workspace_bytes, void *stream);
+int eps_segment_topk_write(const float *score, const int32_t *pair_u, const int32_t *pair_v, int64_t M,
+                           const int64_t *seg_offsets, int64_t n_seg, const uint32_t *out_offsets,
+                           int32_t *out_u, int32_t *out_v, float *out_score, void *workspace,
+                           size_t workspace_bytes, void *stream);
 
 /* ---------------------------------------------------------------------------
  * K6  2-hop candidate enumeration for the owner range [v_lo, v_hi)
