@@ -13,9 +13,10 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libeps_b200.so")
 
 EPS_OK = 0
-EPS_VERSION = 202          # must equal EPS_VERSION in include/eps.h (checked by load())
+EPS_VERSION = 203          # must equal EPS_VERSION in include/eps.h (checked by load())
 EPS_REDUCE_SUM, EPS_REDUCE_MEAN = 0, 1
 EPS_CN_SIGMOID, EPS_CN_GROUPED_BY_V = 1, 2
+EPS_TWOHOP_UPPER = 4       # eps_twohop_onepass: only the candidates u > v of every owner v
 EPS_MLP_FP32, EPS_MLP_TC_F16 = 0, 1
 EPS_MLP_TC_BF16 = EPS_MLP_TC_F16       # round-1 name
 EPS_MLP_REUSE_WORKSPACE = 0x100

@@ -12,7 +12,7 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import EPS_CN_SIGMOID, EpsError, check
+from ._lib import EPS_CN_SIGMOID, EPS_TWOHOP_UPPER, EpsError, check
 from .graph import SparseAdj
 from .ops import _need_cuda, _ptr, _stream, _ws
 
@@ -33,11 +33,14 @@ def owner_counts(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None) -> torc
     return counts.long() & 0xFFFFFFFF
 
 
-def owner_bounds(adj: SparseAdj) -> torch.Tensor:
+def owner_bounds(adj: SparseAdj, upper: bool = False) -> torch.Tensor:
     """Upper bound of every owner's candidate count, int64 [n]: a candidate of v is the end point of
     a 2-path from v (<= #2-paths) and is neither v nor a neighbour of v: <= n - |N(v) U {v}|, i.e.
     n - 1 - deg v, or n - deg v when v carries a self loop (add_edges keeps them; v is then in N(v)).
-    Torch ops only; sizes the outputs of the one-pass kernel and cuts owner ranges into slabs / GPU shards."""
+    Torch ops only; sizes the outputs of the one-pass kernel and cuts owner ranges into slabs / GPU shards.
+    ``upper``: the bound of the half candidates u > v (``half_bounds``)."""
+    if upper:
+        return half_bounds(adj)
     if "owner_bounds" not in adj._cache:
         deg = adj.degree().long()
         rp = adj.rowptr.long()
@@ -51,6 +54,56 @@ def owner_bounds(adj: SparseAdj) -> torch.Tensor:
             loop = torch.ones_like(deg)                 # large graphs: the looser n - deg for everyone
         adj._cache["owner_bounds"] = torch.minimum(two_path_work(adj), (adj.n - 1 - deg + loop).clamp_(min=0))
     return adj._cache["owner_bounds"]
+
+
+def _mirror_search(adj: SparseAdj):
+    """(key, mirror, pos): key = row * n + col of every entry (int64 [nnz], ascending: rows are stored in order with
+    sorted columns), mirror = col * n + row, pos = the first key > mirror.  Keys are integers, so pos is also the first
+    key >= k * n + v + 1 for the entry (v, k), i.e. where the suffix of N(k) above v starts; and (k, v) is an entry
+    exactly when key[pos - 1] == mirror.  One search serves the symmetry check and the half bounds."""
+    if "mirror_search" not in adj._cache:
+        row, col = adj.row(), adj.col.long()
+        key = row * adj.n + col
+        mirror = col * adj.n + row
+        adj._cache["mirror_search"] = (key, mirror, torch.searchsorted(key, mirror, right=True))
+    return adj._cache["mirror_search"]
+
+
+def half_bounds(adj: SparseAdj) -> torch.Tensor:
+    """Upper bound of every owner's count of HALF candidates u > v (the upper-triangle mode of the one-pass kernel),
+    int64 [n]: min(#2-paths v - k - u with u > v, (n - 1 - v) - |N(v) & (v, n)|).  The 2-path term is
+    sum_{k in N(v)} |N(k) & (v, n)|; one searchsorted of k * n + v + 1 over the sorted entry keys gives each
+    |N(k) & (v, n)| (``_mirror_search``).  With the full bound every slab of the half stream would be about half empty."""
+    if "half_bounds" not in adj._cache:
+        n = adj.n
+        rp = adj.rowptr.long()
+        if adj.nnz == 0:
+            adj._cache["half_bounds"] = torch.zeros(n, dtype=torch.int64, device=adj.device)
+            adj._cache["half_two_path_work"] = adj._cache["half_bounds"]
+            return adj._cache["half_bounds"]
+        key, _, pos = _mirror_search(adj)
+        # entry (v, k): the suffix of N(k) above v starts at the first key >= k * n + v + 1
+        suffix = rp[adj.col.long() + 1] - pos
+        cs = torch.zeros(adj.nnz + 1, dtype=torch.int64, device=adj.device)
+        torch.cumsum(suffix, 0, out=cs[1:])
+        paths = cs[rp[1:]] - cs[rp[:-1]]
+        ar = torch.arange(n, device=adj.device)
+        above = rp[1:] - torch.searchsorted(key, ar * n + ar + 1)          # |N(v) & (v, n)|
+        adj._cache["half_two_path_work"] = paths
+        adj._cache["half_bounds"] = torch.minimum(paths, (n - 1 - ar - above).clamp_(min=0))
+    return adj._cache["half_bounds"]
+
+
+def structurally_symmetric(adj: SparseAdj) -> bool:
+    """True when (u, k) is an entry exactly when (k, u) is (``add_edges`` graphs always are) and no entry repeats: then
+    u is a candidate of v exactly when v is a candidate of u.  Checked once per graph."""
+    if "struct_sym" not in adj._cache:
+        ok = True
+        if adj.nnz:
+            key, mirror, pos = _mirror_search(adj)
+            ok = bool(torch.equal(key[(pos - 1).clamp_(min=0)], mirror)) and bool((key[1:] > key[:-1]).all())
+        adj._cache["struct_sym"] = ok
+    return adj._cache["struct_sym"]
 
 
 def check_fixed_point_range(adj: SparseAdj, wtable, use_values: bool) -> None:
@@ -86,10 +139,11 @@ def values_symmetric(adj: SparseAdj) -> bool:
 
 
 def _onepass(adj: SparseAdj, wtable, v_lo: int, v_hi: int, bounds, sigmoid: bool, want_score: bool, want_count: bool,
-             cap: int | None = None, val: torch.Tensor | None = None):
+             cap: int | None = None, val: torch.Tensor | None = None, upper: bool = False):
     """eps_twohop_onepass: (edges int32 [2,N] view, score | None, count | None, offsets int64 [n_own+1]).
-    ``bounds``: per-owner upper bounds of the candidate counts (default ``owner_bounds``); ``cap``: their
-    sum when the caller already knows it (filter_step.iter_slabs) — saves a host sync."""
+    ``bounds``: per-owner upper bounds of the candidate counts (default ``owner_bounds(adj, upper)``); ``cap``: their
+    sum when the caller already knows it (filter_step.iter_slabs) — saves a host sync.  ``upper``: only the
+    candidates u > v of every owner v (EPS_TWOHOP_UPPER)."""
     lib = _lib.load()
     dev = adj.device
     n_own = v_hi - v_lo
@@ -99,7 +153,7 @@ def _onepass(adj: SparseAdj, wtable, v_lo: int, v_hi: int, bounds, sigmoid: bool
                 torch.empty(0, dtype=torch.float32, device=dev) if want_score else None,
                 torch.empty(0, dtype=torch.int32, device=dev) if want_count else None, z)
     if bounds is None:
-        bounds = owner_bounds(adj)[v_lo:v_hi]
+        bounds = owner_bounds(adj, upper)[v_lo:v_hi]
     boff = torch.zeros(n_own + 1, dtype=torch.int64, device=dev)
     torch.cumsum(bounds, 0, out=boff[1:])
     cap = int(boff[-1].item()) if cap is None else int(cap)
@@ -112,7 +166,7 @@ def _onepass(adj: SparseAdj, wtable, v_lo: int, v_hi: int, bounds, sigmoid: bool
     wt = None if wtable is None else wtable.contiguous().float()
     ws = _ws(lib.eps_twohop_onepass_workspace_bytes(cap, n_own), dev)
     check(lib.eps_twohop_onepass(_ptr(adj.rowptr), _ptr(adj.col), _ptr(val), _ptr(wt), adj.n, v_lo, v_hi, _ptr(boff), cap,
-                                 EPS_CN_SIGMOID if sigmoid else 0, _ptr(buf[0]), _ptr(buf[1]), _ptr(score),
+                                 (EPS_CN_SIGMOID if sigmoid else 0) | (EPS_TWOHOP_UPPER if upper else 0), _ptr(buf[0]), _ptr(buf[1]), _ptr(score),
                                  _ptr(count), _ptr(offsets), _ptr(ws), ws.numel(), _stream()), "eps_twohop_onepass")
     from . import ops as _ops
     _ops.LAUNCHES["n"] += 3
@@ -123,19 +177,23 @@ def _onepass(adj: SparseAdj, wtable, v_lo: int, v_hi: int, bounds, sigmoid: bool
 
 
 def two_hop(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, counts: torch.Tensor | None = None,
-            cap: int | None = None, want_offsets: bool = False):
+            cap: int | None = None, want_offsets: bool = False, upper: bool = False):
     """(u, v) candidate list of owners [v_lo, v_hi): int32 [2, N], column-major reference order.
     ``counts`` (from ``owner_counts``) selects the two-pass kernels; without it the one-pass kernel
     runs (no count pass) and the result is a [2, N] view of a buffer sized by the owner_bounds sum
     (``cap`` = that sum, when the caller already has it on the host).  ``want_offsets`` returns
     ``(edges, offsets)``: offsets int64 [v_hi - v_lo + 1], owner v's candidates are
-    ``edges[:, offsets[v - v_lo]:offsets[v - v_lo + 1]]`` (the segments of ``ops.segment_topk``)."""
+    ``edges[:, offsets[v - v_lo]:offsets[v - v_lo + 1]]`` (the segments of ``ops.segment_topk``).
+    ``upper`` (one pass only): only the candidates u > v of every owner v — each unordered pair once on a
+    structurally symmetric graph; ``cap`` is then the sum of ``half_bounds``."""
     _need_cuda(adj.col)
     lib = _lib.load()
     v_hi = adj.n if v_hi is None else v_hi
+    if upper and counts is not None:
+        raise EpsError("two_hop: the upper-triangle mode is one-pass only (no `counts`)")
     if counts is None:
         # one pass: padded per-owner slots sized by owner_bounds, compacted by the finalize pass
-        r = _onepass(adj, None, v_lo, v_hi, None, False, False, False, cap)
+        r = _onepass(adj, None, v_lo, v_hi, None, False, False, False, cap, upper=upper)
         return (r[0], r[3]) if want_offsets else r[0]
     offsets = torch.zeros(counts.numel() + 1, dtype=torch.int64, device=adj.device)
     torch.cumsum(counts, 0, out=offsets[1:])
@@ -156,7 +214,8 @@ def two_hop(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, counts: torc
 
 def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int = 0, v_hi: int | None = None,
                    counts: torch.Tensor | None = None, sigmoid: bool = False, want_count: bool = False,
-                   cap: int | None = None, use_values: bool = True, want_offsets: bool = False):
+                   cap: int | None = None, use_values: bool = True, want_offsets: bool = False,
+                   upper: bool = False):
     """K6+K3 fused: the candidates of owners [v_lo, v_hi) AND their heuristic scores from one walk
     over the owners' 2-paths (``wtable=None`` -> CN count, else sum of ``wtable[k]`` over the common
     neighbours: AA with 1/log deg, RA with 1/deg).  Returns ``(edges int32 [2,N], score fp32 [N])``
@@ -165,17 +224,20 @@ def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int
     2-path on the one-pass kernel; ``use_values=False`` ignores the values ('adamic', models.py:544-554).
     Without ``counts`` the one-pass kernel runs: no count pass, outputs are views of buffers sized by
     the owner_bounds sum of the range.  ``want_offsets`` appends the per-owner offsets (int64
-    [v_hi - v_lo + 1], as in ``two_hop``) to the returned tuple."""
+    [v_hi - v_lo + 1], as in ``two_hop``) to the returned tuple.  ``upper``: as in ``two_hop``."""
     _need_cuda(adj.col, wtable)
     val = adj.val if use_values else None
     check_fixed_point_range(adj, wtable, use_values)
     if val is not None and (counts is not None or not values_symmetric(adj)):
         raise EpsError("two_hop_scored: a weighted adjacency takes the one-pass kernel (no `counts`) and needs "
                        "bitwise symmetric values; otherwise score with two_hop + ops.cn_aa")
+    if upper and counts is not None:
+        raise EpsError("two_hop_scored: the upper-triangle mode is one-pass only (no `counts`)")
     lib = _lib.load()
     v_hi = adj.n if v_hi is None else v_hi
     if counts is None:
-        edges, score, count, offsets = _onepass(adj, wtable, v_lo, v_hi, None, sigmoid, True, want_count, cap, val)
+        edges, score, count, offsets = _onepass(adj, wtable, v_lo, v_hi, None, sigmoid, True, want_count, cap, val,
+                                                upper)
         out = (edges, score, count) if want_count else (edges, score)
         return out + (offsets,) if want_offsets else out
     offsets = torch.zeros(counts.numel() + 1, dtype=torch.int64, device=adj.device)
@@ -196,6 +258,14 @@ def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int
         _ops.LAUNCHES["n"] += 2
     out = (edges, score, count) if want_count else (edges, score)
     return out + (offsets,) if want_offsets else out
+
+
+def half_two_path_work(adj: SparseAdj) -> torch.Tensor:
+    """``two_path_work`` of the upper-triangle mode: the 2-paths v - k - u with u > v of every owner (the first term of
+    ``half_bounds``); low ids carry most of it."""
+    if "half_two_path_work" not in adj._cache:
+        half_bounds(adj)
+    return adj._cache["half_two_path_work"]
 
 
 def two_path_work(adj: SparseAdj) -> torch.Tensor:

@@ -31,6 +31,9 @@
 //     real count; a single-block scan turns the counts into compact offsets and the finalize pass —
 //     which has to read every accumulator anyway — moves (u, score, count) to the compact position and
 //     regenerates v from the owner id.  No count pass, no inter-CTA dependency.
+// Upper-triangle mode (EPS_TWOHOP_UPPER, one-pass only): only the candidates u > v of owner v.  The candidate relation
+// of a symmetric adjacency is symmetric, so this is every unordered pair once; both walks start each N(k) at its lower
+// bound of v + 1 and the rank / emission / cleanup passes start at the bitmap block that holds v + 1.
 #include "eps_common.cuh"
 
 namespace eps {
@@ -47,10 +50,11 @@ constexpr int TS_DEPTH = 8;   // ... with this many loads in flight per lane (a 
 // (ncu source counters, profiles/round2_e_twohop.md).  The caller picks the largest LG that still leaves ~4 groups
 // per warp to balance with.  `counter` is zero when the walk starts (the caller resets it behind a barrier).
 // f.visit(u, p) is called once per 2-path v - k - u (p = index of u in `col`, i.e. inside N(k)) after
-// f.select_slot*(lane that holds k's metadata).
+// f.select_slot*(lane that holds k's metadata).  Only end points u >= umin are visited: each N(k) is sorted, so its
+// walk starts at its lower bound of umin (one binary search per list) and the flattened prefix uses the suffix lengths.
 template <typename F>
 __device__ __forceinline__ void walk_two_paths(const int *__restrict__ rowptr, const int *__restrict__ col,
-                                               int vs, int ve, int lane, int LG, int *counter, F f) {
+                                               int vs, int ve, int lane, int LG, int *counter, int umin, F f) {
   for (;;) {
     int grp = 0;
     if (lane == 0) grp = atomicAdd(counter, 1);
@@ -61,7 +65,16 @@ __device__ __forceinline__ void walk_two_paths(const int *__restrict__ rowptr, c
     if (lane < LG && base + lane < ve) {
       k = __ldg(col + base + lane);
       s = __ldg(rowptr + k);
-      len = __ldg(rowptr + k + 1) - s;
+      const int e = __ldg(rowptr + k + 1);
+      if (umin > 0) {                                  // upper-triangle mode: first position with col >= umin
+        int lo = s, hi = e;
+        while (lo < hi) {
+          const int mid = (lo + hi) >> 1;
+          if (__ldg(col + mid) < umin) lo = mid + 1; else hi = mid;
+        }
+        s = lo;
+      }
+      len = e - s;
     }
     f.load_slot(k, base + lane);
     // ---- long lists: the whole warp streams one list, TS_DEPTH loads in flight per lane ----
@@ -174,7 +187,7 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
                     const long long *__restrict__ offsets, int *__restrict__ pair_u,
                     int *__restrict__ pair_v, unsigned long long *__restrict__ acc, int *__restrict__ cn,
                     unsigned int *owner_counter, unsigned int *__restrict__ counts_out,
-                    const int *__restrict__ owner_order, int n_order) {
+                    const int *__restrict__ owner_order, int n_order, int upper) {
   extern __shared__ uint32_t sm[];
   const int W = (n + 31) >> 5;       // bitmap words
   const int W2 = (W + 31) >> 5;      // blocks of 32 words
@@ -207,19 +220,23 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
     while (LG > 1 && (ve - vs + LG - 1) / LG < 4 * NW) LG >>= 1;
     const long long out_base = offsets[v - v_lo];
     if (offsets[v - v_lo + 1] == out_base) continue;   // no (room for) candidates (uniform): bitmap untouched
+    // upper-triangle mode (EPS_TWOHOP_UPPER): only candidates u > v, so every bit set below lies at or above umin and
+    // the rank pass, emission and cleanup start at the block that holds umin
+    const int umin = upper ? v + 1 : 0;
+    const int g0 = umin >> 10;                         // first block of 32 bitmap words that can hold a mark
     // ---- 1. mark ----
-    walk_two_paths(rowptr, col, vs, ve, lane, LG, &s_walk, MarkVisitor{bm, bm2});
+    walk_two_paths(rowptr, col, vs, ve, lane, LG, &s_walk, umin, MarkVisitor{bm, bm2});
     __syncthreads();
     // ---- 2. clear known edges and the diagonal ----
     for (int p = vs + tid; p < ve; p += THREADS) {
       const int k = __ldg(col + p);
-      atomicAnd(&bm[k >> 5], ~(1u << (k & 31)));
+      if (k >= umin) atomicAnd(&bm[k >> 5], ~(1u << (k & 31)));
     }
-    if (tid == 0) atomicAnd(&bm[v >> 5], ~(1u << (v & 31)));
+    if (tid == 0 && v >= umin) atomicAnd(&bm[v >> 5], ~(1u << (v & 31)));
     if (tid == 0) { s_carry = 0; s_walk = 0; }        // the first walk is over (barrier above): reset for the second
     __syncthreads();
     // ---- 3a. rank: thread t owns block c + t (32 bitmap words) ----
-    for (int c = 0; c < W2; c += THREADS) {
+    for (int c = g0; c < W2; c += THREADS) {
       const int g = c + tid;
       const uint32_t m2 = (g < W2) ? bm2[g] : 0u;
       uint32_t cnt = 0;
@@ -260,7 +277,7 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
       // padded slot: record the real count (a violated bound poisons N instead of overrunning the slot)
       if (tid == 0) counts_out[v - v_lo] = fits ? total : 0xffffffffu;
       if (!fits) {
-        for (int g = tid; g < W2; g += THREADS) {
+        for (int g = g0 + tid; g < W2; g += THREADS) {
           uint32_t m = bm2[g];
           while (m) {
             const int b = __ffs(m) - 1;
@@ -273,7 +290,7 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
       }
     }
     // ---- 3b. emit pair_u / pair_v in ascending u ----
-    for (int g = tid; g < W2; g += THREADS) {
+    for (int g = g0 + tid; g < W2; g += THREADS) {
       uint32_t m = bm2[g];
       long long o = out_base + blk[g];
       while (m) {
@@ -295,11 +312,11 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
       ScoreVisitor<HAS_W, WANT_CN, HAS_VAL> sv{bm, blk, pre, wtable, val,
                                                (HAS_W || HAS_VAL) ? acc + out_base : nullptr,
                                                WANT_CN ? cn + out_base : nullptr};
-      walk_two_paths(rowptr, col, vs, ve, lane, LG, &s_walk, sv);
+      walk_two_paths(rowptr, col, vs, ve, lane, LG, &s_walk, umin, sv);
     }
     __syncthreads();
     // ---- 5. cleanup ----
-    for (int c = 0; c < W2; c += THREADS) {
+    for (int c = g0; c < W2; c += THREADS) {
       const int g = c + tid;
       if (g < W2) {
         uint32_t m = bm2[g];
@@ -464,6 +481,7 @@ extern "C" int eps_twohop_scored(const int32_t *rowptr, const int32_t *col, cons
   cudaStream_t stream = (cudaStream_t)stream_;
   EPS_CHECK_ARG(rowptr && col && offsets, "null graph or offsets pointer");
   EPS_CHECK_ARG(n > 0 && v_lo >= 0 && v_hi <= n && v_lo <= v_hi && N >= 0, "bad owner range or N");
+  EPS_CHECK_ARG(!(flags & EPS_TWOHOP_UPPER), "EPS_TWOHOP_UPPER needs the one-pass entry point (eps_twohop_onepass)");
   if (v_lo == v_hi || N == 0) return EPS_OK;
   EPS_CHECK_ARG(pair_u && pair_v && (score || count), "missing output pointer");
   const int sms = sm_count();
@@ -490,7 +508,7 @@ extern "C" int eps_twohop_scored(const int32_t *rowptr, const int32_t *col, cons
   }
   if (cn) EPS_CUDA(cudaMemsetAsync(cn, 0, (size_t)N * 4, stream));
   void (*kern)(const int *, const int *, const float *, const float *, int, int, int, const long long *, int *,
-               int *, unsigned long long *, int *, unsigned int *, unsigned int *, const int *, int);
+               int *, unsigned long long *, int *, unsigned int *, unsigned int *, const int *, int, int);
   if (wtable) kern = cn ? twohop_score_kernel<true, true, false> : twohop_score_kernel<true, false, false>;
   else kern = twohop_score_kernel<false, true, false>;
   EPS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -500,7 +518,7 @@ extern "C" int eps_twohop_scored(const int32_t *rowptr, const int32_t *col, cons
   const int grid = (int)std::min<long long>((long long)(v_hi - v_lo), (long long)sms * occ);
   kern<<<grid, TS_THREADS, smem, stream>>>(rowptr, col, nullptr, wtable, n, v_lo, v_hi,
                                            (const long long *)offsets, pair_u, pair_v, acc, cn,
-                                           (unsigned int *)ws, nullptr, nullptr, 0);
+                                           (unsigned int *)ws, nullptr, nullptr, 0, 0);
   EPS_LAUNCH_CHECK();
   if (score) {
     const int fgrid = (int)std::min<long long>((N + 255) / 256, (long long)sms * 8);
@@ -566,7 +584,7 @@ extern "C" int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, con
   }
   if (cn) EPS_CUDA(cudaMemsetAsync(cn, 0, (size_t)cap * 4, stream));
   void (*kern)(const int *, const int *, const float *, const float *, int, int, int, const long long *, int *,
-               int *, unsigned long long *, int *, unsigned int *, unsigned int *, const int *, int);
+               int *, unsigned long long *, int *, unsigned int *, unsigned int *, const int *, int, int);
   // CTA size.  Measured (gpurun_out/r31, fused phase per step): 1024 threads help only where the bitmap limits
   // the kernel to 2 CTAs per SM (ppa 12.6 -> 11.6 ms) and hurt where 512-thread CTAs already fill the SM
   // (collab 4.6 -> 7.7 ms; ddi 8.1 -> 8.2): 512 stays the default, EPS_TS_THREADS=1024 overrides (A/B runs)
@@ -596,7 +614,8 @@ extern "C" int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, con
   }
   kern<<<grid, threads, smem, stream>>>(rowptr, col, val, wtable, n, v_lo, v_hi,
                                            (const long long *)bound_offsets, pad_u, nullptr, acc, cn,
-                                           (unsigned int *)ws, counts, order, n_own);
+                                           (unsigned int *)ws, counts, order, n_own,
+                                           (flags & EPS_TWOHOP_UPPER) ? 1 : 0);
   EPS_LAUNCH_CHECK();
   owner_scan_kernel<<<1, 1024, 0, stream>>>(counts, n_own, (long long *)offsets_out);
   EPS_LAUNCH_CHECK();

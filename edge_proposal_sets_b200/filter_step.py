@@ -18,6 +18,12 @@ single global stable sort.  Multi-GPU: each rank takes a contiguous owner range
 (parallel.partition_by_work), the GNN embeddings are computed row-sharded and all-gathered
 (models._ConvStack.embed_rows) and the per-rank lists are merged after an exchange of the global k-th
 score (parallel.merge_topk).
+
+Mirror mode (``mirror``, on by default where it is exact): on a structurally symmetric graph u is a candidate of v
+exactly when v is a candidate of u, and every fused heuristic score on an unweighted graph and every LinkPredictor
+score (h_u * h_v, one rounded product per feature) is a symmetric function bit for bit.  The slabs then stream only
+the half candidates u > v of every owner (K6 / K6+K3 upper-triangle mode), and the full list is rebuilt from the
+half top-k (``mirror_topk``).
 """
 from __future__ import annotations
 
@@ -88,14 +94,15 @@ def ra_graph_from_train_edges(train_edges: torch.Tensor, num_nodes: int) -> Spar
     return SparseAdj(rowptr.int(), (ukey - row * n).int(), None if bool((cnt == 1).all()) else val, n)
 
 
-def iter_slabs(adj: SparseAdj, v_lo: int, v_hi: int, slab_pairs: int) -> Iterator[Tuple[int, int, int]]:
+def iter_slabs(adj: SparseAdj, v_lo: int, v_hi: int, slab_pairs: int,
+               upper: bool = False) -> Iterator[Tuple[int, int, int]]:
     """Yield (lo, hi, cap) owner ranges whose candidate count is at most ``cap <= slab_pairs``
     (a single owner whose bound exceeds that gets a slab of its own).  ``cap`` is the sum of the
     per-owner upper bounds (candidates.owner_bounds) — it sizes the one-pass kernel's outputs, so no
-    count pass over the graph is needed to plan the slabs."""
+    count pass over the graph is needed to plan the slabs.  ``upper``: the bounds of the half candidates u > v."""
     if v_hi <= v_lo:
         return
-    cs = torch.cumsum(candidates.owner_bounds(adj)[v_lo:v_hi], 0).cpu()
+    cs = torch.cumsum(candidates.owner_bounds(adj, upper)[v_lo:v_hi], 0).cpu()
     lo = 0
     n_own = v_hi - v_lo
     base = 0
@@ -109,16 +116,56 @@ def iter_slabs(adj: SparseAdj, v_lo: int, v_hi: int, slab_pairs: int) -> Iterato
         lo = hi
 
 
-def owner_cost(adj: SparseAdj, jobs) -> torch.Tensor:
+def owner_cost(adj: SparseAdj, jobs, upper: bool = False) -> torch.Tensor:
     """Per-owner cost estimate that the multi-GPU owner ranges are balanced on.  Enumeration (K6) costs the owner's
     2-paths; scoring a candidate with a GNN filter model (K2) costs ~8 x a 2-path visit (measured on the ppa shape:
     0.218 ns per candidate against 0.029 ns per 2-path), and the candidate count is bounded by the owner's slot size
     (candidates.owner_bounds).  Balancing on 2-paths alone left the ranks with few hubs 5 % more candidates and the
-    others waiting at the merge (N = 4: 33 ms of a 615 ms step)."""
-    work = candidates.two_path_work(adj).double()
+    others waiting at the merge (N = 4: 33 ms of a 615 ms step).  ``upper`` (mirror mode): the same model on the half
+    work — the 2-paths that end above v and the half-candidate bound — which low owner ids carry most of."""
+    work = (candidates.half_two_path_work(adj) if upper else candidates.two_path_work(adj)).double()
     if any((j.name if hasattr(j, "name") else j[0]) in GNN_MODELS for j in jobs):
-        work = work + 8.0 * candidates.owner_bounds(adj).double()
+        work = work + 8.0 * candidates.owner_bounds(adj, upper).double()
     return work
+
+
+def mirror_eligible(jobs, adj: SparseAdj, k: Optional[int], owners=None, per_node: Optional[int] = None) -> bool:
+    """True when ``_filter_multi`` may score every unordered candidate pair once and rebuild the list (``mirror_topk``):
+    the whole graph (no ``owners``), a proposal size ``k`` and no per-node budgets (those need both directions of an
+    owner's list), a structurally symmetric adjacency, and a bit-symmetric score in every job — any GNN arm (the
+    LinkPredictor's input h_u * h_v is one rounded product per feature), or a fused heuristic on an unweighted graph
+    or without values (weighted AA / CN forms a_u * (a_v * w_k) in fp32, which is not symmetric)."""
+    if owners is not None or k is None or per_node is not None:
+        return False
+    for j in jobs:
+        if j.name in GNN_MODELS:
+            continue
+        t = heuristic_table(j.name, adj, j.ra_adj)
+        if t is None or (adj.val is not None and t[3]):
+            return False
+    return candidates.structurally_symmetric(adj)
+
+
+def mirror_topk(half: torch.Tensor, k: int, n: int, select=None) -> torch.Tensor:
+    """The full ``[k,3]`` list from the top-k of the half candidates.
+
+    The half stream holds every unordered pair {a, b} (a < b) once, as the row (b, a) of owner a: in candidate order
+    (column-major, by (v, u)) that is the position of the pair's FIRST full row, and the full stream's second row
+    (a, b) has the same score.  Claim: the full top-k rows use only pairs that lie in the half top-k.  Let P own a row
+    of the full top-k; P's first row precedes its second, so P's first row is in the full top-k too.  Every pair Q
+    ranked before P in half order (better score, or the same score and an earlier half position) has its first row
+    before P's first row in the full order, so fewer than k pairs precede P and P is in the half top-k.
+    Hence: the half top-k (``half``, k rows), its mirrored rows (v, u, s) added, the 2k rows put into candidate order
+    by one int64 key sort (v * n + u), and K4's select (score descending, ties by position) gives the full list.
+    ``select(edges, score, k)`` stands in for ``ops.topk_edges`` (the CPU tests pass a stable sort)."""
+    if half.shape[0] == 0:
+        return half
+    both = torch.cat([half, half[:, [1, 0, 2]]], 0)
+    ui, vi = both[:, 0].long(), both[:, 1].long()
+    order = torch.argsort(vi * n + ui)
+    both = both[order]
+    edges = torch.stack([both[:, 0].int(), both[:, 1].int()])
+    return (select or ops.topk_edges)(edges, both[:, 2].contiguous(), min(int(k), both.shape[0]))
 
 
 class PrefilterToleranceError(RuntimeError):
@@ -300,12 +347,13 @@ def tc_arm_supported(model) -> bool:
 @torch.no_grad()
 def filter_topk_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: int = 1 << 27,
                       distributed: bool = False, stats: Optional[dict] = None, pushdown: bool = True,
-                      owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None):
+                      owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None,
+                      mirror: Optional[bool] = None):
     """``_filter_multi`` (see there) with the prefilter's safety net: when a job's tensor-core scores leave the
     calibrated tolerance, or its band cannot prune, the call is repeated with that job on the fp32 arm."""
     jobs = [j if isinstance(j, FilterJob) else FilterJob(*j) for j in jobs]
     try:
-        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners, per_node)
+        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners, per_node, mirror)
     except PrefilterToleranceError as exc:
         import warnings
         warnings.warn(f"{exc}; re-running the filter step on the fp32 arm")
@@ -314,13 +362,14 @@ def filter_topk_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pai
                 j.precision = "fp32"
         if stats is not None:
             stats["prefilter_fallback"] = str(exc)
-        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners, per_node)
+        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners, per_node, mirror)
 
 
 @torch.no_grad()
 def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: int = 1 << 27,
                   distributed: bool = False, stats: Optional[dict] = None, pushdown: bool = True,
-                  owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None):
+                  owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None,
+                  mirror: Optional[bool] = None):
     """The filter step for several filter models over ONE enumeration of the 2-hop candidates: a list of
     sorted proposal lists (float32 ``[k,3]`` rows (u, v, score) on the device; score descending, ties by
     the reference's candidate order), one per job.  ``k=None`` keeps every candidate like the reference.
@@ -351,7 +400,16 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
     s16 all have s32 >= that value): a candidate with s16 < S16_m - 2 tol has s32 < S16_m - tol <= S32_m, strictly
     below the owner's m-th best fp32 score, so it cannot be among the owner's exact m best.  No band is exchanged or
     pruned across owners (each rank's per-owner lists are complete), and the prefilter stays on with ``k=None``:
-    the n * m budget bounds the pool."""
+    the n * m budget bounds the pool.
+
+    ``mirror=None`` (default) scores every unordered candidate pair once where that is exact (``mirror_eligible``),
+    ``mirror=True`` insists on it (ValueError where it is not exact), ``mirror=False`` always streams both directions.
+    In mirror mode the slabs stream the half candidates u > v (K6 / K6+K3 upper-triangle mode, slabs and GPU shares cut
+    on the half bounds and the half work; the bounds are planned with the symmetry check, phase ``mirror``); every job keeps
+    its running top-k over them by K4's rule — the prefilter's calibration, band, pool and fp32 re-scoring run
+    unchanged on the half pairs — the ranks merge the half lists as usual, and ``mirror_topk`` rebuilds the full list,
+    bit for bit the list of ``mirror=False``.  ``stats["candidates_scored"]`` still counts the directed candidates the
+    lists rank (2 x ``stats["pairs_evaluated"]``, the half pairs scored); ``stats["mirror"]`` says which path ran."""
     rank, world = parallel.world_info() if distributed else (0, 1)
     if per_node is not None and int(per_node) < 1:
         raise ValueError(f"per_node must be >= 1 (got {per_node})")
@@ -360,10 +418,17 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
         raise ValueError("distributed filter needs a proposal size k")
     jobs = [j if isinstance(j, FilterJob) else FilterJob(*j) for j in jobs]
     ph = _Phases(stats is not None and bool(stats.get("time_phases")))
+    half = mirror is not False and mirror_eligible(jobs, adj, k, owners, per_node)
+    if mirror and not half:
+        raise ValueError("mirror=True: this call cannot score each unordered pair once (it needs the whole graph, a k, "
+                         "no per-node budget, a structurally symmetric graph and bit-symmetric scores)")
+    if half:
+        candidates.owner_bounds(adj, upper=True)             # half slot bounds: planned with the symmetry check
+        ph.mark("mirror")                                    # (one search over the entries, once per graph)
     o_lo, o_hi = (0, adj.n) if owners is None else (max(int(owners[0]), 0), min(int(owners[1]), adj.n))
     v_lo, v_hi = o_lo, o_hi
     if world > 1:
-        bounds = parallel.partition_by_work(owner_cost(adj, jobs)[o_lo:o_hi], world)
+        bounds = parallel.partition_by_work(owner_cost(adj, jobs, half)[o_lo:o_hi], world)
         v_lo, v_hi = o_lo + bounds[rank], o_lo + bounds[rank + 1]
     # per job: scoring plan + running proposal set
     plans = []
@@ -391,7 +456,7 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
     ph.mark("embed")
     n_slabs = 0
     n_cand = 0
-    for lo, hi, cap in iter_slabs(adj, v_lo, v_hi, slab_pairs):
+    for lo, hi, cap in iter_slabs(adj, v_lo, v_hi, slab_pairs, half):
         n_slabs += 1
         scores = {}
         offsets = None
@@ -400,12 +465,12 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
             # candidates and their scores together (bit-identical to scoring the pairs with K3)
             t = plans[fused_job]["table"]
             r = candidates.two_hop_scored(t[0], t[1], lo, hi, sigmoid=t[2], cap=cap, use_values=t[3],
-                                          want_offsets=m is not None)
+                                          want_offsets=m is not None, upper=half)
             edges, scores[fused_job] = r[0], r[1]
             offsets = r[2] if m is not None else None
             ph.mark("enum_score")
         else:
-            r = candidates.two_hop(adj, lo, hi, cap=cap, want_offsets=m is not None)
+            r = candidates.two_hop(adj, lo, hi, cap=cap, want_offsets=m is not None, upper=half)
             edges, offsets = r if m is not None else (r, None)
             ph.mark("enum")
         if edges.shape[1] == 0:
@@ -452,9 +517,15 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
         if world > 1:
             res = parallel.merge_topk(res, k)
             ph.mark("merge")
+        if half:
+            res = mirror_topk(res, k, adj.n)
+            ph.mark("mirror")
         out.append(res)
     if stats is not None:
-        stats["candidates_scored"] = (plans[0]["run"].seen if m is None else n_cand) if plans else 0
+        seen = (plans[0]["run"].seen if m is None else n_cand) if plans else 0
+        stats["candidates_scored"] = 2 * seen if half else seen
+        stats["pairs_evaluated"] = seen
+        stats["mirror"] = half
         if m is not None:
             stats["per_node"] = dict(m=m, survivors=[p["pn_kept"] for p in plans])
         stats["slabs"] = n_slabs
@@ -601,13 +672,15 @@ def _rescore_pool(model, h, run: RunningTopK, k: int, world: int, tol: float, ca
 def filter_topk(model_name: str, model, x, adj: SparseAdj, k: Optional[int] = None,
                 slab_pairs: int = 1 << 27, distributed: bool = False, ra_adj: Optional[SparseAdj] = None,
                 stats: Optional[dict] = None, precision: Optional[str] = None,
-                owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None) -> torch.Tensor:
+                owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None,
+                mirror: Optional[bool] = None) -> torch.Tensor:
     """Sorted proposal list of one filter model, float32 ``[k,3]`` rows (u, v, score) on the device: score
     descending, ties by the reference's candidate order.  ``k=None`` keeps every candidate like the
     reference.  ``precision`` (GNN models): see ``FilterJob``; default = the model's ``linkpred.precision``.
-    ``per_node=m``: only the m best candidates of every owner v (see ``_filter_multi``)."""
+    ``per_node=m``: only the m best candidates of every owner v; ``mirror``: see ``_filter_multi``."""
     job = FilterJob(model_name, model, ra_adj, precision)
-    return filter_topk_multi([job], x, adj, k, slab_pairs, distributed, stats, owners=owners, per_node=per_node)[0]
+    return filter_topk_multi([job], x, adj, k, slab_pairs, distributed, stats, owners=owners, per_node=per_node,
+                             mirror=mirror)[0]
 
 
 def load_extra_edges(path: str, num_sorted_edge: int) -> torch.Tensor:

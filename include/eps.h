@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define EPS_VERSION 202 /* 0.2.2; edge_proposal_sets_b200/_lib.py checks it at load time */
+#define EPS_VERSION 203 /* 0.2.3; edge_proposal_sets_b200/_lib.py checks it at load time */
 
 typedef enum {
   EPS_OK = 0,
@@ -302,7 +302,7 @@ size_t eps_twohop_workspace_bytes(void);
  *   offsets  int64[v_hi - v_lo + 1] exclusive prefix of the per-owner counts
  *            returned by eps_twohop_candidates' count pass; N = offsets[last]
  *   wtable   NULL -> score = CN count; else score = sum of wtable[k]
- *   flags    EPS_CN_SIGMOID
+ *   flags    EPS_CN_SIGMOID  (EPS_TWOHOP_UPPER is rejected: one-pass only)
  *   score    fp32[N] or NULL;  count int32[N] or NULL (exact CN)
  * Unweighted adjacency only (weighted graphs: eps_twohop_candidates + eps_cn_aa).
  * Needs ~3n/16 bytes of shared memory (<= 200 KB, i.e. n <= ~1.0M).
@@ -337,8 +337,17 @@ size_t eps_twohop_scored_workspace_bytes(int64_t N);
  *                kernel reads A[k,u] for A[u,k], so A must be bitwise symmetric.
  *   wtable / flags / score / count as in eps_twohop_scored; score == NULL and
  *   count == NULL -> enumeration only (the GNN filter models).
+ *   flags |= EPS_TWOHOP_UPPER: upper-triangle mode, only the candidates u > v
+ *                of every owner v (each unordered pair once, under its smaller
+ *                end).  Both walks visit only the suffix u > v of every N(k)
+ *                and the bitmap work starts at word (v + 1) / 32; the bound
+ *                may then be min(#2-paths v-k-u with u > v,
+ *                n - 1 - v - |N(v) & (v, n)|).  Owner v's output is (u, v) in
+ *                ascending u, and every score equals the full kernel's score
+ *                of the same pair, bit for bit.
  * Results are bit-identical to the two-pass entry points.
  * ------------------------------------------------------------------------- */
+#define EPS_TWOHOP_UPPER 4
 int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, const float *val, const float *wtable,
                        int32_t n, int32_t v_lo, int32_t v_hi, const int64_t *bound_offsets, int64_t cap, int flags,
                        int32_t *pair_u, int32_t *pair_v, float *score, int32_t *count,
