@@ -17,6 +17,11 @@ EPS_VERSION = 203          # must equal EPS_VERSION in include/eps.h (checked by
 EPS_REDUCE_SUM, EPS_REDUCE_MEAN = 0, 1
 EPS_CN_SIGMOID, EPS_CN_GROUPED_BY_V = 1, 2
 EPS_TWOHOP_UPPER = 4       # eps_twohop_onepass: only the candidates u > v of every owner v
+# degree-normalised similarity scores: a 3-bit kind field at bit 8 of the eps_cn_aa / eps_twohop_* flags
+EPS_SCORE_KIND_SHIFT = 8
+EPS_SCORE_KIND_MASK = 7 << EPS_SCORE_KIND_SHIFT
+SCORE_KINDS = {"jaccard": 1, "sorensen": 2, "salton": 3, "hub_promoted": 4, "hub_depressed": 5,
+               "leicht_holme_newman": 6, "preferential_attachment": 7}
 EPS_MLP_FP32, EPS_MLP_TC_F16 = 0, 1
 EPS_MLP_TC_BF16 = EPS_MLP_TC_F16       # round-1 name
 EPS_MLP_REUSE_WORKSPACE = 0x100
@@ -34,6 +39,7 @@ SIGNATURES = {
     "eps_gcn_norm_fill": (_int, [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "eps_cn_aa": (_int, [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _i64, _int, _vp, _vp, _vp, _sz, _vp]),
     "eps_cn_aa_workspace_bytes": (_sz, []),
+    "eps_score_kinds": (_int, []),
     "eps_linkpred_mlp": (_int, [_vp, _i32, _i32, _vp, _vp, _i64, C.POINTER(_vp), C.POINTER(_vp), _i32,
                                 _int, _int, _vp, _vp, _sz, _vp]),
     "eps_linkpred_workspace_bytes": (_sz, [_i32, _i32, _i32, _i64, _int]),
@@ -86,7 +92,11 @@ def load(build: bool | None = None) -> C.CDLL:
         _b.build()
     lib = C.CDLL(LIB_PATH)
     for name, (res, args) in SIGNATURES.items():
-        fn = getattr(lib, name)  # AttributeError if the .so does not export a declared symbol
+        try:
+            fn = getattr(lib, name)
+        except AttributeError:
+            raise EpsError(f"{LIB_PATH} does not export {name} (built from an older eps.h): "
+                           "rebuild it with `python -m edge_proposal_sets_b200.build --force`") from None
         fn.restype = res
         fn.argtypes = args
     got = lib.eps_version()

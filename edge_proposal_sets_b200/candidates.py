@@ -12,7 +12,7 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import EPS_CN_SIGMOID, EPS_TWOHOP_UPPER, EpsError, check
+from ._lib import EPS_CN_SIGMOID, EPS_SCORE_KIND_SHIFT, EPS_TWOHOP_UPPER, SCORE_KINDS, EpsError, check
 from .graph import SparseAdj
 from .ops import _need_cuda, _ptr, _stream, _ws
 
@@ -127,6 +127,22 @@ def check_fixed_point_range(adj: SparseAdj, wtable, use_values: bool) -> None:
                        "CN/AA kernels (csrc/eps_common.cuh); rescale the edge weights or the weight table")
 
 
+def similarity_flags(adj: SparseAdj, kind: str | None) -> int:
+    """The flag bits of a similarity kind (``_lib.SCORE_KINDS``; ``None`` -> 0) for ``adj``.  The kernels divide
+    integers held in fp32, exact only below 2^24: raises when 2 * max degree >= 2^24 (a + b could reach it).  The
+    degree is checked once per graph."""
+    if kind is None:
+        return 0
+    if kind not in SCORE_KINDS:
+        raise EpsError(f"unknown similarity kind {kind!r} (known: {', '.join(SCORE_KINDS)})")
+    if "max_degree" not in adj._cache:
+        adj._cache["max_degree"] = int(adj.degree().max().item()) if adj.n else 0
+    if not 2 * adj._cache["max_degree"] < 2 ** 24:
+        raise EpsError(f"max degree {adj._cache['max_degree']}: deg u + deg v may reach 2^24, beyond the integers fp32 "
+                       f"holds exactly; the {kind} kernels cannot score this graph exactly")
+    return SCORE_KINDS[kind] << EPS_SCORE_KIND_SHIFT
+
+
 def values_symmetric(adj: SparseAdj) -> bool:
     """True when A[u,k] == A[k,u] bit for bit (always, for ``add_edges`` graphs with integer-valued
     weights: both directions receive the same exact sum).  Checked once per graph."""
@@ -139,11 +155,11 @@ def values_symmetric(adj: SparseAdj) -> bool:
 
 
 def _onepass(adj: SparseAdj, wtable, v_lo: int, v_hi: int, bounds, sigmoid: bool, want_score: bool, want_count: bool,
-             cap: int | None = None, val: torch.Tensor | None = None, upper: bool = False):
+             cap: int | None = None, val: torch.Tensor | None = None, upper: bool = False, kind_flags: int = 0):
     """eps_twohop_onepass: (edges int32 [2,N] view, score | None, count | None, offsets int64 [n_own+1]).
     ``bounds``: per-owner upper bounds of the candidate counts (default ``owner_bounds(adj, upper)``); ``cap``: their
     sum when the caller already knows it (filter_step.iter_slabs) — saves a host sync.  ``upper``: only the
-    candidates u > v of every owner v (EPS_TWOHOP_UPPER)."""
+    candidates u > v of every owner v (EPS_TWOHOP_UPPER).  ``kind_flags``: a similarity kind (``similarity_flags``)."""
     lib = _lib.load()
     dev = adj.device
     n_own = v_hi - v_lo
@@ -166,7 +182,8 @@ def _onepass(adj: SparseAdj, wtable, v_lo: int, v_hi: int, bounds, sigmoid: bool
     wt = None if wtable is None else wtable.contiguous().float()
     ws = _ws(lib.eps_twohop_onepass_workspace_bytes(cap, n_own), dev)
     check(lib.eps_twohop_onepass(_ptr(adj.rowptr), _ptr(adj.col), _ptr(val), _ptr(wt), adj.n, v_lo, v_hi, _ptr(boff), cap,
-                                 (EPS_CN_SIGMOID if sigmoid else 0) | (EPS_TWOHOP_UPPER if upper else 0), _ptr(buf[0]), _ptr(buf[1]), _ptr(score),
+                                 (EPS_CN_SIGMOID if sigmoid else 0) | (EPS_TWOHOP_UPPER if upper else 0) | kind_flags,
+                                 _ptr(buf[0]), _ptr(buf[1]), _ptr(score),
                                  _ptr(count), _ptr(offsets), _ptr(ws), ws.numel(), _stream()), "eps_twohop_onepass")
     from . import ops as _ops
     _ops.LAUNCHES["n"] += 3
@@ -215,7 +232,7 @@ def two_hop(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, counts: torc
 def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int = 0, v_hi: int | None = None,
                    counts: torch.Tensor | None = None, sigmoid: bool = False, want_count: bool = False,
                    cap: int | None = None, use_values: bool = True, want_offsets: bool = False,
-                   upper: bool = False):
+                   upper: bool = False, kind: str | None = None):
     """K6+K3 fused: the candidates of owners [v_lo, v_hi) AND their heuristic scores from one walk
     over the owners' 2-paths (``wtable=None`` -> CN count, else sum of ``wtable[k]`` over the common
     neighbours: AA with 1/log deg, RA with 1/deg).  Returns ``(edges int32 [2,N], score fp32 [N])``
@@ -224,8 +241,16 @@ def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int
     2-path on the one-pass kernel; ``use_values=False`` ignores the values ('adamic', models.py:544-554).
     Without ``counts`` the one-pass kernel runs: no count pass, outputs are views of buffers sized by
     the owner_bounds sum of the range.  ``want_offsets`` appends the per-owner offsets (int64
-    [v_hi - v_lo + 1], as in ``two_hop``) to the returned tuple.  ``upper``: as in ``two_hop``."""
+    [v_hi - v_lo + 1], as in ``two_hop``) to the returned tuple.  ``upper``: as in ``two_hop``.
+    ``kind`` (a name of ``_lib.SCORE_KINDS``, e.g. "jaccard"): a degree-normalised similarity of the exact count and
+    the degrees of both ends instead (include/eps.h, EPS_SCORE_*): structure only, so needs ``wtable=None`` and no
+    sigmoid, and ignores edge values."""
     _need_cuda(adj.col, wtable)
+    kind_flags = similarity_flags(adj, kind)
+    if kind_flags and (wtable is not None or sigmoid):
+        raise EpsError(f"two_hop_scored: the {kind} score takes no weight table and no sigmoid")
+    if kind_flags:
+        use_values = False
     val = adj.val if use_values else None
     check_fixed_point_range(adj, wtable, use_values)
     if val is not None and (counts is not None or not values_symmetric(adj)):
@@ -237,7 +262,7 @@ def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int
     v_hi = adj.n if v_hi is None else v_hi
     if counts is None:
         edges, score, count, offsets = _onepass(adj, wtable, v_lo, v_hi, None, sigmoid, True, want_count, cap, val,
-                                                upper)
+                                                upper, kind_flags)
         out = (edges, score, count) if want_count else (edges, score)
         return out + (offsets,) if want_offsets else out
     offsets = torch.zeros(counts.numel() + 1, dtype=torch.int64, device=adj.device)
@@ -252,7 +277,7 @@ def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int
         wt = None if wtable is None else wtable.contiguous().float()
         ws = _ws(lib.eps_twohop_scored_workspace_bytes(N), adj.device)
         check(lib.eps_twohop_scored(_ptr(adj.rowptr), _ptr(adj.col), _ptr(wt), adj.n, v_lo, v_hi, _ptr(offsets), N,
-                                    EPS_CN_SIGMOID if sigmoid else 0, _ptr(edges[0]), _ptr(edges[1]), _ptr(score),
+                                    (EPS_CN_SIGMOID if sigmoid else 0) | kind_flags, _ptr(edges[0]), _ptr(edges[1]), _ptr(score),
                                     _ptr(count), _ptr(ws), ws.numel(), _stream()), "eps_twohop_scored")
         from . import ops as _ops
         _ops.LAUNCHES["n"] += 2

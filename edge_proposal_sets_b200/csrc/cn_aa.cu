@@ -39,12 +39,14 @@ constexpr size_t CN_MAX_BITMAP_BYTES = 200 * 1024;
 // never depends on which phase handled the list or in which order the terms arrived.
 constexpr int CN_LONG = 64;
 
-template <bool HAS_W>
+// KIND != 0: a similarity score (EPS_SCORE_*) of the exact count, deg u (= len) and deg v (= *dv, in shared memory: a
+// register live across the walk spills) replaces the CN score.
+template <bool HAS_W, int KIND>
 __device__ __forceinline__ void grouped_batch(const int *__restrict__ rowptr,
                                               const int *__restrict__ col,
                                               const float *__restrict__ wtable,
                                               const uint32_t *bitmap, const int *__restrict__ pu,
-                                              long long base, int cnt, int flags,
+                                              long long base, int cnt, int flags, const int *dv,
                                               float *__restrict__ score, int *__restrict__ count) {
   const int lane = lane_id();
   const bool valid = lane < cnt;
@@ -139,14 +141,19 @@ __device__ __forceinline__ void grouped_batch(const int *__restrict__ rowptr,
   if (valid) {
     if (count) count[base + lane] = c_acc;
     if (score) {
-      float sc = HAS_W ? from_fixed(a_acc) : (float)c_acc;
-      if (flags & EPS_CN_SIGMOID) sc = sigmoidf_ref(sc);
+      float sc;
+      if (KIND) {
+        sc = similarity_score<KIND>(c_acc, len, *dv);
+      } else {
+        sc = HAS_W ? from_fixed(a_acc) : (float)c_acc;
+        if (flags & EPS_CN_SIGMOID) sc = sigmoidf_ref(sc);
+      }
       score[base + lane] = sc;
     }
   }
 }
 
-template <bool HAS_W>
+template <bool HAS_W, int KIND = 0>
 __global__ void __launch_bounds__(CN_THREADS)
 cn_grouped_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
                   const float *__restrict__ wtable, int n, const int *__restrict__ pu,
@@ -155,6 +162,7 @@ cn_grouped_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
   extern __shared__ uint32_t bitmap[];
   __shared__ long long s_tile;
   __shared__ long long s_end;
+  __shared__ int s_dv;               // deg v of the current run (similarity kinds)
   const int tid = threadIdx.x;
   const int warp = tid >> 5;
   const int nwarps = CN_THREADS / 32;
@@ -186,6 +194,7 @@ cn_grouped_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
         j += CN_THREADS;
       }
       const int vs = __ldg(rowptr + v), ve = __ldg(rowptr + v + 1);
+      if (KIND && tid == 0) s_dv = ve - vs;            // read after the barrier below
       for (int p = vs + tid; p < ve; p += CN_THREADS) {
         const int k = __ldg(col + p);
         atomicOr(&bitmap[k >> 5], 1u << (k & 31));
@@ -193,7 +202,7 @@ cn_grouped_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
       __syncthreads();
       for (long long base = i + (long long)warp * 32; base < j; base += (long long)nwarps * 32) {
         const int cnt = (int)min((long long)32, j - base);
-        grouped_batch<HAS_W>(rowptr, col, wtable, bitmap, pu, base, cnt, flags, score, count);
+        grouped_batch<HAS_W, KIND>(rowptr, col, wtable, bitmap, pu, base, cnt, flags, &s_dv, score, count);
       }
       __syncthreads();
       for (int p = vs + tid; p < ve; p += CN_THREADS) bitmap[__ldg(col + p) >> 5] = 0;
@@ -205,7 +214,7 @@ cn_grouped_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
 
 constexpr int PAIR_G = 8;
 
-template <bool HAS_VAL, bool HAS_W>
+template <bool HAS_VAL, bool HAS_W, int KIND = 0>
 __global__ void __launch_bounds__(256)
 cn_pairs_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
                 const float *__restrict__ val, const float *__restrict__ wtable,
@@ -268,13 +277,31 @@ cn_pairs_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
     if (gl == 0) {
       if (count) count[pair] = c_acc;
       if (score) {
-        float sc = (HAS_VAL || HAS_W) ? from_fixed(a_acc) : (float)c_acc;
-        if (flags & EPS_CN_SIGMOID) sc = sigmoidf_ref(sc);
+        float sc;
+        if (KIND) {
+          sc = similarity_score<KIND>(c_acc, lu, lv);
+        } else {
+          sc = (HAS_VAL || HAS_W) ? from_fixed(a_acc) : (float)c_acc;
+          if (flags & EPS_CN_SIGMOID) sc = sigmoidf_ref(sc);
+        }
         score[pair] = sc;
       }
     }
   }
 }
+
+using GroupedKernel = void (*)(const int *, const int *, const float *, int, const int *, const int *, long long, int,
+                               float *, int *, unsigned long long *);
+using PairsKernel = void (*)(const int *, const int *, const float *, const float *, const int *, const int *,
+                             long long, int, float *, int *);
+// index = similarity kind (EPS_SCORE_* >> EPS_SCORE_KIND_SHIFT); entry 0 is never used
+static const GroupedKernel kGroupedKinds[8] = {
+    cn_grouped_kernel<false, 0>, cn_grouped_kernel<false, 1>, cn_grouped_kernel<false, 2>, cn_grouped_kernel<false, 3>,
+    cn_grouped_kernel<false, 4>, cn_grouped_kernel<false, 5>, cn_grouped_kernel<false, 6>, cn_grouped_kernel<false, 7>};
+static const PairsKernel kPairsKinds[8] = {
+    cn_pairs_kernel<false, false, 0>, cn_pairs_kernel<false, false, 1>, cn_pairs_kernel<false, false, 2>,
+    cn_pairs_kernel<false, false, 3>, cn_pairs_kernel<false, false, 4>, cn_pairs_kernel<false, false, 5>,
+    cn_pairs_kernel<false, false, 6>, cn_pairs_kernel<false, false, 7>};
 
 }  // namespace eps
 
@@ -287,6 +314,10 @@ extern "C" int eps_cn_aa(const int32_t *rowptr, const int32_t *col, const float 
   using namespace eps;
   cudaStream_t stream = (cudaStream_t)stream_;
   EPS_CHECK_ARG(n > 0 && M >= 0, "bad n or M");
+  EPS_CHECK_ARG(!(flags & ~(EPS_CN_SIGMOID | EPS_CN_GROUPED_BY_V | EPS_SCORE_KIND_MASK)), "unknown flag bits");
+  const int kind = score_kind(flags);
+  EPS_CHECK_ARG(!kind || (!wtable && !val && !(flags & EPS_CN_SIGMOID)),
+                "a similarity kind (EPS_SCORE_*) needs wtable == NULL, val == NULL and no EPS_CN_SIGMOID");
   if (M == 0) return EPS_OK;  // empty pair list: nothing to read or write
   EPS_CHECK_ARG(rowptr && col && pair_u && pair_v, "null graph or pair pointer");
   EPS_CHECK_ARG(score || count, "score and count both NULL");
@@ -301,7 +332,7 @@ extern "C" int eps_cn_aa(const int32_t *rowptr, const int32_t *col, const float 
       return EPS_ERR_WORKSPACE;
     }
     EPS_CUDA(cudaMemsetAsync(workspace, 0, 8, stream));
-    auto kern = wtable ? cn_grouped_kernel<true> : cn_grouped_kernel<false>;
+    GroupedKernel kern = kind ? kGroupedKinds[kind] : wtable ? cn_grouped_kernel<true> : cn_grouped_kernel<false>;
     EPS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)bitmap_bytes));
     int occ = 0;
@@ -321,7 +352,9 @@ extern "C" int eps_cn_aa(const int32_t *rowptr, const int32_t *col, const float 
 #define EPS_LAUNCH_PAIRS(HV, HW)                                                             \
   cn_pairs_kernel<HV, HW><<<grid, 256, 0, stream>>>(rowptr, col, val, wtable, pair_u, pair_v, \
                                                     (long long)M, flags, score, count)
-  if (val && wtable) EPS_LAUNCH_PAIRS(true, true);
+  if (kind) kPairsKinds[kind]<<<grid, 256, 0, stream>>>(rowptr, col, val, wtable, pair_u, pair_v, (long long)M, flags,
+                                                       score, count);
+  else if (val && wtable) EPS_LAUNCH_PAIRS(true, true);
   else if (val) EPS_LAUNCH_PAIRS(true, false);
   else if (wtable) EPS_LAUNCH_PAIRS(false, true);
   else EPS_LAUNCH_PAIRS(false, false);

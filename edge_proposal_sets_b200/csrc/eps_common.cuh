@@ -74,6 +74,31 @@ __device__ __forceinline__ float from_fixed(unsigned long long s) {
   return __ll2float_rn((long long)s) * 3.637978807091713e-12f /* 2^-38 */;
 }
 
+// ---- degree-normalised similarity scores (include/eps.h, EPS_SCORE_*) ----
+__host__ __device__ constexpr int score_kind(int flags) { return (flags & EPS_SCORE_KIND_MASK) >> EPS_SCORE_KIND_SHIFT; }
+constexpr int SK_JACCARD = score_kind(EPS_SCORE_JACCARD), SK_SORENSEN = score_kind(EPS_SCORE_SORENSEN),
+              SK_SALTON = score_kind(EPS_SCORE_SALTON), SK_HUB_PROMOTED = score_kind(EPS_SCORE_HUB_PROMOTED),
+              SK_LHN = score_kind(EPS_SCORE_LHN), SK_PREF_ATTACH = score_kind(EPS_SCORE_PREF_ATTACH);
+
+// KIND = score_kind(flags), 1..7 (0 = the kernel's own CN / AA / RA score, which never reaches here).
+// c = exact common-neighbour count, a = deg u, b = deg v.  a + b < 2^24 (host check), so every integer below is exact in
+// fp32 and the fp32 divisions are the correctly rounded quotients.  A zero denominator gives 0.
+template <int KIND>
+__device__ __forceinline__ float similarity_score(int c, int a, int b) {
+  if (KIND == SK_PREF_ATTACH) return __ll2float_rn((long long)a * (long long)b);
+  if (KIND == SK_SALTON || KIND == SK_LHN) {
+    const double ab = (double)a * (double)b;                   // exact: < 2^48
+    if (ab == 0.0) return 0.f;
+    return (float)((double)c / (KIND == SK_SALTON ? sqrt(ab) : ab));
+  }
+  int num = c, den;
+  if (KIND == SK_JACCARD) den = a + b - c;
+  else if (KIND == SK_SORENSEN) { num = 2 * c; den = a + b; }
+  else if (KIND == SK_HUB_PROMOTED) den = min(a, b);
+  else den = max(a, b);                                         // EPS_SCORE_HUB_DEPRESSED
+  return den == 0 ? 0.f : __fdiv_rn((float)num, (float)den);
+}
+
 // streaming (read-once) loads that do not pollute L1
 __device__ __forceinline__ int ld_stream_s32(const int *p) {
   int r;

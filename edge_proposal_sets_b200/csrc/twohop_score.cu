@@ -20,7 +20,8 @@
 //               compact accumulator of that candidate (count as int32, weight as 64-bit fixed point,
 //               eps_common.cuh) — integer atomics, hence exact and order-independent
 //   5. cleanup  zero the touched bitmap words
-// A tiny element-wise pass then turns the fixed-point sums into fp32 scores (+ sigmoid).
+// A tiny element-wise pass then turns the fixed-point sums into fp32 scores (+ sigmoid), or the exact counts and the
+// degrees of both ends (two rowptr loads each) into a similarity score (EPS_SCORE_*, after the count-only walk).
 // Results are bit-identical to eps_cn_aa on the same pairs.
 //
 // Where an owner's output starts:
@@ -331,13 +332,21 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
   }
 }
 
+template <int KIND>
 __global__ void __launch_bounds__(256)
-twohop_finalize_kernel(const unsigned long long *__restrict__ acc, const int *__restrict__ cn,
+twohop_finalize_kernel(const int *__restrict__ rowptr, const int *__restrict__ pair_u, const int *__restrict__ pair_v,
+                       const unsigned long long *__restrict__ acc, const int *__restrict__ cn,
                        long long N, int flags, float *__restrict__ score) {
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += stride) {
-    float sc = acc ? from_fixed(acc[i]) : (float)cn[i];
-    if (flags & EPS_CN_SIGMOID) sc = sigmoidf_ref(sc);
+    float sc;
+    if (KIND) {
+      const int u = pair_u[i], v = pair_v[i];
+      sc = similarity_score<KIND>(cn[i], __ldg(rowptr + u + 1) - __ldg(rowptr + u), __ldg(rowptr + v + 1) - __ldg(rowptr + v));
+    } else {
+      sc = acc ? from_fixed(acc[i]) : (float)cn[i];
+      if (flags & EPS_CN_SIGMOID) sc = sigmoidf_ref(sc);
+    }
     score[i] = sc;
   }
 }
@@ -393,15 +402,17 @@ owner_scan_kernel(const unsigned int *__restrict__ counts, int n_own, long long 
   if (t == 1023) offsets[n_own] = (long long)part[1023];
 }
 
-// padded slot of owner v -> compact position; fixed-point sums -> fp32 scores on the way.
+// padded slot of owner v -> compact position; fixed-point sums -> fp32 scores on the way (KIND != 0: counts and the
+// degrees of u and v -> the similarity score).
 // Work is cut by COMPACT position (tiles of CP_TILE candidates), not by owner, so a hub with 10^5
 // candidates does not serialise on one CTA; the owner of a position is found by binary search over the
 // compact offsets of the (few) owners the tile touches.
 constexpr int CP_THREADS = 256, CP_PER = 8, CP_TILE = CP_THREADS * CP_PER;
 
+template <int KIND>
 __global__ void __launch_bounds__(CP_THREADS)
-twohop_compact_kernel(const long long *__restrict__ pad_off, const long long *__restrict__ cmp_off,
-                      int v_lo, int n_own, long long cap, const int *__restrict__ pad_u,
+twohop_compact_kernel(const int *__restrict__ rowptr, const long long *__restrict__ pad_off,
+                      const long long *__restrict__ cmp_off, int v_lo, int n_own, long long cap, const int *__restrict__ pad_u,
                       const unsigned long long *__restrict__ acc, const int *__restrict__ cn, int flags,
                       int *__restrict__ pair_u, int *__restrict__ pair_v, float *__restrict__ score,
                       int *__restrict__ count) {
@@ -450,6 +461,18 @@ twohop_compact_kernel(const long long *__restrict__ pad_off, const long long *__
         if (cn) cc[q] = cn[src[q]];
       }
     }
+    int du[CP_PER], dv[CP_PER];      // similarity kinds: deg u, deg v (rowptr is L2-resident)
+    if (KIND && score) {
+#pragma unroll
+      for (int q = 0; q < CP_PER; ++q) {
+        du[q] = dv[q] = 0;
+        if (src[q] >= 0) {
+          const int v = v_lo + own[q];
+          du[q] = __ldg(rowptr + uu[q] + 1) - __ldg(rowptr + uu[q]);
+          dv[q] = __ldg(rowptr + v + 1) - __ldg(rowptr + v);
+        }
+      }
+    }
 #pragma unroll
     for (int q = 0; q < CP_PER; ++q) {
       if (src[q] < 0) continue;
@@ -457,8 +480,13 @@ twohop_compact_kernel(const long long *__restrict__ pad_off, const long long *__
       pair_u[i] = uu[q];
       pair_v[i] = v_lo + own[q];
       if (score) {
-        float sc = acc ? from_fixed(aa[q]) : (float)cc[q];
-        if (flags & EPS_CN_SIGMOID) sc = sigmoidf_ref(sc);
+        float sc;
+        if (KIND) {
+          sc = similarity_score<KIND>(cc[q], du[q], dv[q]);
+        } else {
+          sc = acc ? from_fixed(aa[q]) : (float)cc[q];
+          if (flags & EPS_CN_SIGMOID) sc = sigmoidf_ref(sc);
+        }
         score[i] = sc;
       }
       if (count) count[i] = cc[q];
@@ -466,7 +494,26 @@ twohop_compact_kernel(const long long *__restrict__ pad_off, const long long *__
   }
 }
 
+using FinalizeKernel = void (*)(const int *, const int *, const int *, const unsigned long long *, const int *, long long,
+                                int, float *);
+using CompactKernel = void (*)(const int *, const long long *, const long long *, int, int, long long, const int *,
+                               const unsigned long long *, const int *, int, int *, int *, float *, int *);
+// index = score_kind(flags): 0 = CN / AA / RA, 1..7 = the similarity kinds
+static const FinalizeKernel kFinalizeKinds[8] = {
+    twohop_finalize_kernel<0>, twohop_finalize_kernel<1>, twohop_finalize_kernel<2>, twohop_finalize_kernel<3>,
+    twohop_finalize_kernel<4>, twohop_finalize_kernel<5>, twohop_finalize_kernel<6>, twohop_finalize_kernel<7>};
+static const CompactKernel kCompactKinds[8] = {
+    twohop_compact_kernel<0>, twohop_compact_kernel<1>, twohop_compact_kernel<2>, twohop_compact_kernel<3>,
+    twohop_compact_kernel<4>, twohop_compact_kernel<5>, twohop_compact_kernel<6>, twohop_compact_kernel<7>};
+
 }  // namespace eps
+
+extern "C" int eps_score_kinds(void) {
+  return (1 << eps::score_kind(EPS_SCORE_JACCARD)) | (1 << eps::score_kind(EPS_SCORE_SORENSEN)) |
+         (1 << eps::score_kind(EPS_SCORE_SALTON)) | (1 << eps::score_kind(EPS_SCORE_HUB_PROMOTED)) |
+         (1 << eps::score_kind(EPS_SCORE_HUB_DEPRESSED)) | (1 << eps::score_kind(EPS_SCORE_LHN)) |
+         (1 << eps::score_kind(EPS_SCORE_PREF_ATTACH));
+}
 
 extern "C" size_t eps_twohop_scored_workspace_bytes(int64_t N) {
   return 256 + (size_t)(N > 0 ? N : 0) * 8;
@@ -482,6 +529,10 @@ extern "C" int eps_twohop_scored(const int32_t *rowptr, const int32_t *col, cons
   EPS_CHECK_ARG(rowptr && col && offsets, "null graph or offsets pointer");
   EPS_CHECK_ARG(n > 0 && v_lo >= 0 && v_hi <= n && v_lo <= v_hi && N >= 0, "bad owner range or N");
   EPS_CHECK_ARG(!(flags & EPS_TWOHOP_UPPER), "EPS_TWOHOP_UPPER needs the one-pass entry point (eps_twohop_onepass)");
+  EPS_CHECK_ARG(!(flags & ~(EPS_CN_SIGMOID | EPS_SCORE_KIND_MASK)), "unknown flag bits");
+  const int kind = score_kind(flags);
+  EPS_CHECK_ARG(!kind || (!wtable && !(flags & EPS_CN_SIGMOID)),
+                "a similarity kind (EPS_SCORE_*) needs wtable == NULL and no EPS_CN_SIGMOID");
   if (v_lo == v_hi || N == 0) return EPS_OK;
   EPS_CHECK_ARG(pair_u && pair_v && (score || count), "missing output pointer");
   const int sms = sm_count();
@@ -522,7 +573,7 @@ extern "C" int eps_twohop_scored(const int32_t *rowptr, const int32_t *col, cons
   EPS_LAUNCH_CHECK();
   if (score) {
     const int fgrid = (int)std::min<long long>((N + 255) / 256, (long long)sms * 8);
-    twohop_finalize_kernel<<<fgrid, 256, 0, stream>>>(acc, cn, (long long)N, flags, score);
+    kFinalizeKinds[kind]<<<fgrid, 256, 0, stream>>>(rowptr, pair_u, pair_v, acc, cn, (long long)N, flags, score);
     EPS_LAUNCH_CHECK();
   }
   return EPS_OK;
@@ -551,6 +602,10 @@ extern "C" int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, con
   EPS_CHECK_ARG(cap == 0 || (pair_u && pair_v), "missing pair output pointer");
   EPS_CHECK_ARG(!(wtable && !score), "wtable given but no score output");
   EPS_CHECK_ARG(!(val && !score), "edge values given but no score output");
+  EPS_CHECK_ARG(!(flags & ~(EPS_CN_SIGMOID | EPS_TWOHOP_UPPER | EPS_SCORE_KIND_MASK)), "unknown flag bits");
+  const int kind = score_kind(flags);
+  EPS_CHECK_ARG(!kind || (!wtable && !val && !(flags & EPS_CN_SIGMOID)),
+                "a similarity kind (EPS_SCORE_*) needs wtable == NULL, val == NULL and no EPS_CN_SIGMOID");
   const int sms = sm_count();
   if (sms <= 0) { set_error("eps_twohop_onepass: no CUDA device"); return EPS_ERR_CUDA; }
   const int n_own = v_hi - v_lo;
@@ -621,7 +676,7 @@ extern "C" int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, con
   EPS_LAUNCH_CHECK();
   if (cap > 0) {
     const int cgrid = (int)std::min<long long>((cap + CP_TILE - 1) / CP_TILE, (long long)sms * 8);
-    twohop_compact_kernel<<<cgrid, CP_THREADS, 0, stream>>>((const long long *)bound_offsets,
+    kCompactKinds[kind]<<<cgrid, CP_THREADS, 0, stream>>>(rowptr, (const long long *)bound_offsets,
                                                      (const long long *)offsets_out, v_lo, n_own, (long long)cap,
                                                      pad_u, acc,
                                                      cn, flags, pair_u, pair_v, score, count);

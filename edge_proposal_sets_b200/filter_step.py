@@ -33,7 +33,7 @@ import torch
 
 from . import adamic_utils, candidates, ops, parallel
 from .graph import SparseAdj, add_edges
-from .models import GNN_MODELS, LinkGNN
+from .models import GNN_MODELS, SIMILARITY_MODELS, LinkGNN
 
 
 def score_edges(model_name: str, model, x, adj: SparseAdj, edges: torch.Tensor,
@@ -43,6 +43,8 @@ def score_edges(model_name: str, model, x, adj: SparseAdj, edges: torch.Tensor,
         assert isinstance(model, LinkGNN)
         h = model.embed(x, adj)
         return model.linkpred.score_pairs(h, edges)
+    if model_name in SIMILARITY_MODELS:
+        return ops.cn_aa(adj, edges, kind=model_name, grouped_by_v=grouped_by_v)
     if model_name in ("simple", "adamic"):
         model.grouped_by_v = grouped_by_v
         return model(x, edges, adj)
@@ -62,20 +64,23 @@ def same_structure(a: SparseAdj, b: SparseAdj) -> bool:
 
 
 def heuristic_table(model_name: str, adj: SparseAdj, ra_adj: Optional[SparseAdj] = None):
-    """(graph, weight table, sigmoid, use_values) of a heuristic filter model when it can take the fused
+    """(graph, weight table, sigmoid, use_values, kind) of a heuristic filter model when it can take the fused
     enumerate+score kernel (K6+K3, candidates.two_hop_scored): the scoring graph IS the graph whose 2-hop
     neighbourhood defines the candidates and, if weighted (collab), its values are bitwise symmetric.
-    ``None`` otherwise (RA on a rebuilt multigraph) -> two_hop + ops.cn_aa."""
+    ``None`` otherwise (RA on a rebuilt multigraph) -> two_hop + ops.cn_aa.  ``kind``: the similarity models
+    (structure only, so on weighted graphs too), else ``None``."""
+    if model_name in SIMILARITY_MODELS:
+        return adj, None, False, False, model_name
     if not candidates.values_symmetric(adj):
         return None
     if model_name == "simple":
-        return adj, None, False, True                        # models.py:536-542 (weighted on collab)
+        return adj, None, False, True, None                  # models.py:536-542 (weighted on collab)
     if model_name == "adamic":
-        return adj, adj.adamic_weights(), True, False        # models.py:544-554 (indices only)
+        return adj, adj.adamic_weights(), True, False, None  # models.py:544-554 (indices only)
     if model_name == "adamic_ogb":
-        return adj, adj.aa_ogb_weights(), False, True        # adamic_utils.py:13-25 (values of A)
+        return adj, adj.aa_ogb_weights(), False, True, None  # adamic_utils.py:13-25 (values of A)
     if model_name == "resource_allocation" and adj.val is None and (ra_adj is None or same_structure(ra_adj, adj)):
-        return adj, adj.ra_weights(), False, True            # train_and_eval.py:195-216
+        return adj, adj.ra_weights(), False, True, None      # train_and_eval.py:195-216
     return None
 
 
@@ -134,7 +139,8 @@ def mirror_eligible(jobs, adj: SparseAdj, k: Optional[int], owners=None, per_nod
     the whole graph (no ``owners``), a proposal size ``k`` and no per-node budgets (those need both directions of an
     owner's list), a structurally symmetric adjacency, and a bit-symmetric score in every job — any GNN arm (the
     LinkPredictor's input h_u * h_v is one rounded product per feature), or a fused heuristic on an unweighted graph
-    or without values (weighted AA / CN forms a_u * (a_v * w_k) in fp32, which is not symmetric)."""
+    or without values (weighted AA / CN forms a_u * (a_v * w_k) in fp32, which is not symmetric; the similarity
+    models are functions of (c, deg u, deg v) that are symmetric in the degrees, on any graph)."""
     if owners is not None or k is None or per_node is not None:
         return False
     for j in jobs:
@@ -462,10 +468,11 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
         offsets = None
         if fused_job is not None:
             # CN / AA / RA are the values of A@A: one walk over the owners' 2-paths yields the
-            # candidates and their scores together (bit-identical to scoring the pairs with K3)
+            # candidates and their scores together (bit-identical to scoring the pairs with K3); the
+            # similarity models take the exact counts of the same walk and the degrees
             t = plans[fused_job]["table"]
             r = candidates.two_hop_scored(t[0], t[1], lo, hi, sigmoid=t[2], cap=cap, use_values=t[3],
-                                          want_offsets=m is not None, upper=half)
+                                          want_offsets=m is not None, upper=half, kind=t[4])
             edges, scores[fused_job] = r[0], r[1]
             offsets = r[2] if m is not None else None
             ph.mark("enum_score")

@@ -6,7 +6,8 @@ reference's ``models.py`` so its checkpoints load unchanged and its callers
   LinkPredictor        /root/reference/models.py:461-485
   LinkGNN              /root/reference/models.py:487-506
   CommonNeighborsPredictor ('simple' | 'adamic' | 'adamic_ogb' | 'resource_allocation')
-                       /root/reference/models.py:508-554
+                       /root/reference/models.py:508-554, plus the degree-normalised similarities of
+                       SIMILARITY_MODELS (no reference counterpart; include/eps.h EPS_SCORE_*)
   build_model          /root/reference/models.py:578-670
   default_model_configs/root/reference/models.py:673-790
 
@@ -36,7 +37,11 @@ from . import autograd, ops, parallel
 from .graph import SparseAdj
 
 GNN_MODELS = ("gcn", "sage")
-HEURISTIC_MODELS = ("simple", "adamic", "adamic_ogb", "resource_allocation")
+# c / f(deg u, deg v) scores of the classic local-similarity table (Zhou, Lue & Zhang 2009) and a * b; structural and
+# symmetric, computed from the exact common-neighbour count by the same kernels (``ops.cn_aa(kind=...)``)
+SIMILARITY_MODELS = ("jaccard", "sorensen", "salton", "hub_promoted", "hub_depressed", "leicht_holme_newman",
+                     "preferential_attachment")
+HEURISTIC_MODELS = ("simple", "adamic", "adamic_ogb", "resource_allocation") + SIMILARITY_MODELS
 SUPPORTED_MODELS = GNN_MODELS + HEURISTIC_MODELS
 
 
@@ -277,6 +282,8 @@ class CommonNeighborsPredictor(nn.Module):
     def forward(self, x, edges, adj: SparseAdj):
         if self.type in ("adamic_ogb", "resource_allocation", "katz"):
             return None                            # reference behaviour (models.py:534-535)
+        if self.type in SIMILARITY_MODELS:
+            return ops.cn_aa(adj, edges, kind=self.type, grouped_by_v=self.grouped_by_v)
         if self.type == "simple":
             # sum_k adj[u,k]*adj[v,k]; raw value, no sigmoid (models.py:539-542)
             return ops.cn_aa(adj, edges, None, use_values=True, grouped_by_v=self.grouped_by_v)

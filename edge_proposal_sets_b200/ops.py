@@ -114,18 +114,25 @@ def pair_hadamard_bwd(h: torch.Tensor, edges: torch.Tensor, dz: torch.Tensor) ->
 
 def cn_aa(adj: SparseAdj, edges: torch.Tensor, wtable: Optional[torch.Tensor] = None,
           use_values: bool = True, sigmoid: bool = False, grouped_by_v: bool = False,
-          want_count: bool = False):
-    """K3.  score[i] = sum_{k in N(u)&N(v)} a_u (a_v w_k); optional exact int32 counts."""
+          want_count: bool = False, kind: Optional[str] = None):
+    """K3.  score[i] = sum_{k in N(u)&N(v)} a_u (a_v w_k); optional exact int32 counts.  ``kind`` (a name of
+    ``_lib.SCORE_KINDS``, e.g. "jaccard"): the degree-normalised similarity of the count and the degrees instead
+    (structure only: needs ``wtable=None`` and no sigmoid, ignores edge values)."""
     _need_cuda(adj.col, edges, wtable)
     lib = _lib.load()
-    from .candidates import check_fixed_point_range
+    from .candidates import check_fixed_point_range, similarity_flags
+    kind_flags = similarity_flags(adj, kind)
+    if kind_flags and (wtable is not None or sigmoid):
+        raise EpsError(f"cn_aa: the {kind} score takes no weight table and no sigmoid")
+    if kind_flags:
+        use_values = False
     check_fixed_point_range(adj, wtable, use_values)
     pu, pv = _pairs(edges)
     M = pu.numel()
     score = torch.empty(M, dtype=torch.float32, device=adj.device)
     count = torch.empty(M, dtype=torch.int32, device=adj.device) if want_count else None
     val = adj.val if use_values else None
-    flags = (EPS_CN_SIGMOID if sigmoid else 0) | (EPS_CN_GROUPED_BY_V if grouped_by_v else 0)
+    flags = (EPS_CN_SIGMOID if sigmoid else 0) | (EPS_CN_GROUPED_BY_V if grouped_by_v else 0) | kind_flags
     ws = _ws(lib.eps_cn_aa_workspace_bytes(), adj.device)
     check(lib.eps_cn_aa(_ptr(adj.rowptr), _ptr(adj.col), _ptr(val), _ptr(wtable), adj.n, _ptr(pu), _ptr(pv),
                         M, flags, _ptr(score), _ptr(count), _ptr(ws), ws.numel(), _stream()), "eps_cn_aa")

@@ -104,6 +104,29 @@ int eps_gcn_norm_fill(const int32_t *rowptr, const int32_t *col, const float *va
  * ------------------------------------------------------------------------- */
 #define EPS_CN_SIGMOID 1
 #define EPS_CN_GROUPED_BY_V 2
+/* Degree-normalised similarity scores (eps_cn_aa, eps_twohop_scored, eps_twohop_onepass): a 3-bit kind field at
+ * bit 8 of `flags`.  With c = |N(u) & N(v)| (the exact count), a = |N(u)|, b = |N(v)| (stored lists, self loops
+ * included, edge values ignored), score =
+ *   JACCARD        __fdiv_rn(c, a + b - c)             SORENSEN       __fdiv_rn(2c, a + b)
+ *   HUB_PROMOTED   __fdiv_rn(c, min(a, b))             HUB_DEPRESSED  __fdiv_rn(c, max(a, b))
+ *   SALTON         (float)((double)c / sqrt((double)a * (double)b))
+ *   LHN            (float)((double)c / ((double)a * (double)b))      (Leicht-Holme-Newman)
+ *   PREF_ATTACH    __ll2float_rn((int64)a * b)                         (preferential attachment)
+ * A zero denominator gives 0.  The four divisions are correctly rounded when 2 * max degree < 2^24 (the caller
+ * checks it).  A kind needs wtable == NULL, val == NULL and no EPS_CN_SIGMOID; every other combination, and any
+ * flag bit an entry point does not define, is rejected (EPS_ERR_INVALID). */
+#define EPS_SCORE_KIND_SHIFT 8
+#define EPS_SCORE_KIND_MASK (7 << EPS_SCORE_KIND_SHIFT)
+#define EPS_SCORE_JACCARD (1 << EPS_SCORE_KIND_SHIFT)
+#define EPS_SCORE_SORENSEN (2 << EPS_SCORE_KIND_SHIFT)
+#define EPS_SCORE_SALTON (3 << EPS_SCORE_KIND_SHIFT)
+#define EPS_SCORE_HUB_PROMOTED (4 << EPS_SCORE_KIND_SHIFT)
+#define EPS_SCORE_HUB_DEPRESSED (5 << EPS_SCORE_KIND_SHIFT)
+#define EPS_SCORE_LHN (6 << EPS_SCORE_KIND_SHIFT)
+#define EPS_SCORE_PREF_ATTACH (7 << EPS_SCORE_KIND_SHIFT)
+/* bit k set <=> kind code k (flags >> EPS_SCORE_KIND_SHIFT) is supported; a library without the kinds lacks the
+ * symbol, so a stale build fails at load time instead of ignoring the bits */
+int eps_score_kinds(void);
 int eps_cn_aa(const int32_t *rowptr, const int32_t *col, const float *val, const float *wtable,
               int32_t n, const int32_t *pair_u, const int32_t *pair_v, int64_t M, int flags,
               float *score, int32_t *count, void *workspace, size_t workspace_bytes,
@@ -302,7 +325,8 @@ size_t eps_twohop_workspace_bytes(void);
  *   offsets  int64[v_hi - v_lo + 1] exclusive prefix of the per-owner counts
  *            returned by eps_twohop_candidates' count pass; N = offsets[last]
  *   wtable   NULL -> score = CN count; else score = sum of wtable[k]
- *   flags    EPS_CN_SIGMOID  (EPS_TWOHOP_UPPER is rejected: one-pass only)
+ *   flags    EPS_CN_SIGMOID | a similarity kind (EPS_SCORE_*, see eps_cn_aa; degrees from rowptr)
+ *            (EPS_TWOHOP_UPPER is rejected: one-pass only)
  *   score    fp32[N] or NULL;  count int32[N] or NULL (exact CN)
  * Unweighted adjacency only (weighted graphs: eps_twohop_candidates + eps_cn_aa).
  * Needs ~3n/16 bytes of shared memory (<= 200 KB, i.e. n <= ~1.0M).
@@ -336,7 +360,9 @@ size_t eps_twohop_scored_workspace_bytes(int64_t N);
  *                A[u,k] * A[v,k] without wtable) — eps_cn_aa's products; the
  *                kernel reads A[k,u] for A[u,k], so A must be bitwise symmetric.
  *   wtable / flags / score / count as in eps_twohop_scored; score == NULL and
- *   count == NULL -> enumeration only (the GNN filter models).
+ *   count == NULL -> enumeration only (the GNN filter models).  A similarity
+ *   kind (EPS_SCORE_*) runs the count-only walk and applies its formula in the
+ *   compaction pass: weighted graphs pass val == NULL (structure only).
  *   flags |= EPS_TWOHOP_UPPER: upper-triangle mode, only the candidates u > v
  *                of every owner v (each unordered pair once, under its smaller
  *                end).  Both walks visit only the suffix u > v of every N(k)
