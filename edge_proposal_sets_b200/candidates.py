@@ -12,7 +12,7 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import EPS_CN_SIGMOID, EPS_SCORE_KIND_SHIFT, EPS_TWOHOP_UPPER, SCORE_KINDS, EpsError, check
+from ._lib import EPS_CN_GROUPED_BY_V, EPS_CN_SIGMOID, EPS_SCORE_KIND_SHIFT, EPS_TWOHOP_UPPER, SCORE_KINDS, EpsError, check
 from .graph import SparseAdj
 from .ops import _need_cuda, _ptr, _stream, _ws
 
@@ -244,7 +244,15 @@ def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int
     [v_hi - v_lo + 1], as in ``two_hop``) to the returned tuple.  ``upper``: as in ``two_hop``.
     ``kind`` (a name of ``_lib.SCORE_KINDS``, e.g. "jaccard"): a degree-normalised similarity of the exact count and
     the degrees of both ends instead (include/eps.h, EPS_SCORE_*): structure only, so needs ``wtable=None`` and no
-    sigmoid, and ignores edge values."""
+    sigmoid, and ignores edge values.  ``kind="local_path"``: the Local Path index (``two_hop_local_path``; the count is
+    c2)."""
+    if kind == LOCAL_PATH:
+        if wtable is not None or sigmoid or counts is not None:
+            raise EpsError("two_hop_scored: the local_path score takes no weight table, no sigmoid and no `counts` "
+                           "(one-pass only)")
+        e, s, c2, _, off = two_hop_local_path(adj, v_lo, v_hi, cap, upper, want_offsets=True)
+        out = (e, s, c2) if want_count else (e, s)
+        return out + (off,) if want_offsets else out
     _need_cuda(adj.col, wtable)
     kind_flags = similarity_flags(adj, kind)
     if kind_flags and (wtable is not None or sigmoid):
@@ -303,3 +311,110 @@ def two_path_work(adj: SparseAdj) -> torch.Tensor:
         rp = adj.rowptr.long()
         adj._cache["two_path_work"] = cs[rp[1:]] - cs[rp[:-1]]
     return adj._cache["two_path_work"]
+
+
+# ---------------------------------------------------------------------------------------------
+# Local Path index: LP(u, v) = (A^2)_uv + 1e-3 (A^3)_uv (include/eps.h, eps_local_path_*)
+# ---------------------------------------------------------------------------------------------
+LOCAL_PATH = "local_path"
+
+
+def require_symmetric(adj: SparseAdj, what: str) -> None:
+    """The Local Path kernels count 3-paths through the candidate relation, which needs a structurally symmetric graph
+    (``structurally_symmetric``, checked once per graph): raises before anything is launched otherwise."""
+    if not structurally_symmetric(adj):
+        raise EpsError(f"{what}: the local_path score needs a structurally symmetric adjacency ((u, k) stored exactly "
+                       "when (k, u) is, no repeated entry); add_edges graphs are")
+
+
+def arc_triangles(adj: SparseAdj) -> torch.Tensor:
+    """tri int32 [nnz]: tri[p] = |N(v) & N(k)| for the stored arc p = (v, k), i.e. the exact K3 counts of the pairs
+    (k, v) (grouped by v: rows are stored in order).  Structure only.  Built once per graph."""
+    if "arc_tri" not in adj._cache:
+        _need_cuda(adj.col)
+        lib = _lib.load()
+        tri = torch.empty(adj.nnz, dtype=torch.int32, device=adj.device)
+        if adj.nnz:
+            row = adj.row().to(torch.int32)
+            ws = _ws(lib.eps_cn_aa_workspace_bytes(), adj.device)
+            check(lib.eps_cn_aa(_ptr(adj.rowptr), _ptr(adj.col), None, None, adj.n, _ptr(adj.col), _ptr(row), adj.nnz,
+                                EPS_CN_GROUPED_BY_V, None, _ptr(tri), _ptr(ws), ws.numel(), _stream()), "eps_cn_aa")
+            from . import ops as _ops
+            _ops.LAUNCHES["n"] += 1
+        adj._cache["arc_tri"] = tri
+    return adj._cache["arc_tri"]
+
+
+def local_path_work(adj: SparseAdj, upper: bool = False) -> torch.Tensor:
+    """Per-owner pull work of the Local Path walk 3, int64 [n]: sum_{k in N(v)} sum_{u in N(k)} deg u (two products of A
+    with the degrees; a candidate reached by several 2-paths counts once per 2-path, so this bounds the work of its
+    N(u) stream).  ``upper``: only the end points u > v.  Torch ops only; device-agnostic."""
+    key = ("lp_work", bool(upper))
+    if key not in adj._cache:
+        deg = adj.degree().long()
+        rp = adj.rowptr.long()
+        cs = torch.zeros(adj.nnz + 1, dtype=torch.int64, device=adj.device)
+        if adj.nnz:
+            torch.cumsum(deg[adj.col.long()], 0, out=cs[1:])            # prefix of deg u over the entries
+        if upper and adj.nnz:
+            _, _, pos = _mirror_search(adj)                             # entry (v, k): N(k) above v starts at pos
+            per_entry = cs[rp[adj.col.long() + 1]] - cs[pos]
+        else:
+            per_entry = (cs[rp[1:]] - cs[rp[:-1]])[adj.col.long()]      # sum_{u in N(k)} deg u
+        ce = torch.zeros(adj.nnz + 1, dtype=torch.int64, device=adj.device)
+        if adj.nnz:
+            torch.cumsum(per_entry, 0, out=ce[1:])
+        adj._cache[key] = ce[rp[1:]] - ce[rp[:-1]]
+    return adj._cache[key]
+
+
+def _lp_ctas(device) -> int:
+    """Per-CTA scratch areas handed to eps_local_path_onepass: every CTA that can be resident (<= 4 per SM at 512
+    threads)."""
+    return 4 * torch.cuda.get_device_properties(device).multi_processor_count
+
+
+def two_hop_local_path(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, cap: int | None = None,
+                       upper: bool = False, want_offsets: bool = False):
+    """The candidates of owners [v_lo, v_hi) with their Local Path scores from one fused walk
+    (eps_local_path_onepass): ``(edges int32 [2,N], score fp32 [N], c2 int32 [N], c3 int32 [N])`` (+ offsets int64
+    [v_hi - v_lo + 1] with ``want_offsets``), candidates in the order of ``two_hop``.  c2 = |N(u) & N(v)|,
+    c3 = (A^3)_uv, score = fp32(c2 + 1e-3 * c3) rounded once from fp64.  ``upper`` / ``cap``: as in ``two_hop``.
+    Structure only (edge values ignored); raises on a graph that is not structurally symmetric."""
+    require_symmetric(adj, "two_hop_local_path")
+    _need_cuda(adj.col)
+    lib = _lib.load()
+    dev = adj.device
+    v_hi = adj.n if v_hi is None else v_hi
+    n_own = v_hi - v_lo
+    if n_own <= 0:
+        z = torch.zeros(1, dtype=torch.int64, device=dev)
+        i0 = torch.empty(0, dtype=torch.int32, device=dev)
+        out = (torch.empty((2, 0), dtype=torch.int32, device=dev), torch.empty(0, dtype=torch.float32, device=dev), i0, i0)
+        return out + (z,) if want_offsets else out
+    tri = arc_triangles(adj)
+    boff = torch.zeros(n_own + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(owner_bounds(adj, upper)[v_lo:v_hi], 0, out=boff[1:])
+    cap = int(boff[-1].item()) if cap is None else int(cap)
+    if cap >= 2**31:
+        raise EpsError(f"up to {cap} candidates in one slab; split the owner range (see filter_step.iter_slabs)")
+    if "max_bound" not in adj._cache:
+        adj._cache["max_bound"] = int(owner_bounds(adj).max().item()) if adj.n else 0
+    max_count, ctas = adj._cache["max_bound"], _lp_ctas(dev)
+    buf = torch.empty((2, max(cap, 1)), dtype=torch.int32, device=dev)
+    score = torch.empty(max(cap, 1), dtype=torch.float32, device=dev)
+    c2 = torch.empty(max(cap, 1), dtype=torch.int32, device=dev)
+    c3 = torch.empty(max(cap, 1), dtype=torch.int32, device=dev)
+    offsets = torch.empty(n_own + 1, dtype=torch.int64, device=dev)
+    ws = _ws(lib.eps_local_path_onepass_workspace_bytes(cap, n_own, max_count, ctas), dev)
+    check(lib.eps_local_path_onepass(_ptr(adj.rowptr), _ptr(adj.col), _ptr(tri), adj.n, v_lo, v_hi, _ptr(boff), cap,
+                                     max_count, ctas, EPS_TWOHOP_UPPER if upper else 0, _ptr(buf[0]), _ptr(buf[1]),
+                                     _ptr(score), _ptr(c2), _ptr(c3), _ptr(offsets), _ptr(ws), ws.numel(), _stream()),
+          "eps_local_path_onepass")
+    from . import ops as _ops
+    _ops.LAUNCHES["n"] += 6
+    N = int(offsets[-1].item())
+    if N > cap:
+        raise EpsError(f"eps_local_path_onepass: an owner's candidates exceed the caller's bound (N={N}, cap={cap})")
+    out = (buf[:, :N], score[:N], c2[:N], c3[:N])
+    return out + (offsets,) if want_offsets else out

@@ -506,6 +506,399 @@ static const CompactKernel kCompactKinds[8] = {
     twohop_compact_kernel<0>, twohop_compact_kernel<1>, twohop_compact_kernel<2>, twohop_compact_kernel<3>,
     twohop_compact_kernel<4>, twohop_compact_kernel<5>, twohop_compact_kernel<6>, twohop_compact_kernel<7>};
 
+// ---------------------------------------------------------------------------------------------
+// Local Path index (eps_local_path_onepass, eps_local_path_pairs; include/eps.h)
+//   LP(u, v) = c2 + 1e-3 * c3,  c2 = |N(u) & N(v)| = (A^2)_uv,  c3 = (A^3)_uv = sum_{j in N(u)} c2(j, v).
+// On a structurally symmetric graph every j in N(u) with c2(j, v) > 0 is a candidate of v or a neighbour k of v (never
+// v itself: a candidate u is not adjacent to v), so for a candidate u of owner v
+//   c3(u, v) = sum_{j in N(u) & C(v)} c2(j, v)  +  sum_{k in N(u) & N(v)} tri(v, k),     tri(v, k) = |N(v) & N(k)|.
+// The fused kernel gets both sums without a pass over all pairs of 3-paths:
+//   walks 1-2  the mark / score walks of twohop_score_kernel over ALL candidates of v (walk 3 looks up j < v in upper
+//              mode too); the score walk adds 1 to c2 and, for an emitted candidate, tri of the slot's arc (v, k) to c3;
+//   walk 3     while the bitmap is still in shared memory, the N(u) lists of the emitted candidates, 32 per warp,
+//              flattened as in cn_aa.cu's grouped_batch: a set bit j -> rank(j) -> c2(j, v) (term 1), summed per
+//              candidate in registers (segmented warp scan), one plain store per candidate.
+// c2 lives in a per-CTA scratch indexed by the full rank; u, c2 and c3 of the emitted candidates in the padded slot.
+// All sums are integers (c3 <= nnz < 2^31), the score is formed once in the compaction pass.
+// ---------------------------------------------------------------------------------------------
+constexpr int LP_THREADS = 512;
+constexpr int LP_LONG = 64;     // walk 3: lists at least this long are streamed warp-wide
+
+__device__ __forceinline__ float local_path_score(int c2, int c3) {
+  return __double2float_rn(__dadd_rn((double)c2, __dmul_rn(1e-3, (double)c3)));
+}
+
+__device__ __forceinline__ uint32_t bitmap_rank(const uint32_t *bm, const uint32_t *blk, const uint16_t *pre, int w, int b) {
+  return blk[w >> 5] + pre[w] + __popc(bm[w] & ((1u << b) - 1u));
+}
+
+struct LpScoreVisitor {
+  const uint32_t *bm, *blk;
+  const uint16_t *pre;
+  const int *__restrict__ tri;
+  int *c2;                 // per-CTA scratch, full rank
+  int *c3;                 // padded slot, rank - lo (candidates u >= umin)
+  int lo, umin;
+  int t_slot = 0, t = 0;
+  __device__ __forceinline__ void load_slot(int k, int pos) { t_slot = k >= 0 ? __ldg(tri + pos) : 0; }
+  __device__ __forceinline__ void select_slot(int b) { t = __shfl_sync(FULL, t_slot, b); }
+  __device__ __forceinline__ void select_slot_lane(int l) { t = __shfl_sync(FULL, t_slot, l); }
+  __device__ __forceinline__ void visit(int u, int) {
+    const int w = u >> 5, b = u & 31;
+    if ((bm[w] >> b) & 1u) {
+      const uint32_t idx = bitmap_rank(bm, blk, pre, w, b);
+      atomicAdd(c2 + idx, 1);
+      if (u >= umin && t) atomicAdd(c3 + (idx - lo), t);
+    }
+  }
+};
+
+// Walk 3 for the emitted candidates e0 .. e0 + cnt - 1 of the current owner (one warp).  c2 values were produced by L2
+// atomics of this CTA (possibly over lines an earlier owner left in L1): read with ld.global.cg.
+__device__ __forceinline__ void lp_walk3_batch(const int *__restrict__ rowptr, const int *__restrict__ col,
+                                               const uint32_t *bm, const uint32_t *blk, const uint16_t *pre,
+                                               const int *c2s, int lo, int *su, int *sc2, int *sc3, int e0, int cnt) {
+  const int lane = lane_id();
+  int s = 0, len = 0;
+  if (lane < cnt) {
+    const int u = __ldcg(su + e0 + lane);
+    s = __ldg(rowptr + u);
+    len = __ldg(rowptr + u + 1) - s;
+  }
+  int acc = 0;
+  // ---- long lists, warp-wide, four loads in flight per lane ----
+  unsigned longmask = __ballot_sync(FULL, len >= LP_LONG);
+  while (longmask) {
+    const int b = __ffs(longmask) - 1;
+    longmask &= longmask - 1;
+    const int sb = __shfl_sync(FULL, s, b);
+    const int lb = __shfl_sync(FULL, len, b);
+    int part = 0;
+    for (int off = 0; off < lb; off += 128) {
+      int j[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const int p = off + q * 32 + lane;
+        j[q] = p < lb ? __ldg(col + sb + p) : -1;
+      }
+#pragma unroll
+      for (int q = 0; q < 4; ++q)
+        if (j[q] >= 0 && ((bm[j[q] >> 5] >> (j[q] & 31)) & 1u))
+          part += __ldcg(c2s + bitmap_rank(bm, blk, pre, j[q] >> 5, j[q] & 31));
+    }
+    part = __reduce_add_sync(FULL, part);
+    if (lane == b) acc += part;
+  }
+  // ---- short lists, one flattened sequence; hits summed per list by a segmented scan ----
+  const int slen = len >= LP_LONG ? 0 : len;
+  int pin = slen;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const int t = __shfl_up_sync(FULL, pin, d);
+    if (lane >= d) pin += t;
+  }
+  const int pex = pin - slen;
+  const int total = __shfl_sync(FULL, pin, 31);
+  for (int jb = 0; jb < total; jb += 32) {
+    const int p = jb + lane;
+    int slot = 0;
+#pragma unroll
+    for (int step = 16; step >= 1; step >>= 1) {
+      const int t = __shfl_sync(FULL, pin, slot + step - 1);
+      if (t <= p) slot += step;
+    }
+    const int s_t = __shfl_sync(FULL, s, slot);
+    const int pe_t = __shfl_sync(FULL, pex, slot);
+    int x = 0;
+    if (p < total) {
+      const int j = __ldg(col + s_t + (p - pe_t));
+      if ((bm[j >> 5] >> (j & 31)) & 1u) x = __ldcg(c2s + bitmap_rank(bm, blk, pre, j >> 5, j & 31));
+    }
+    if (__ballot_sync(FULL, x != 0) == 0) continue;          // warp-uniform (a candidate has c2 >= 1)
+    // inclusive scan inside runs of equal slot (slots ascend with p, so equal ends mean one run)
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const int t = __shfl_up_sync(FULL, x, d);
+      const int sl = __shfl_up_sync(FULL, slot, d);
+      if (lane >= d && sl == slot) x += t;
+    }
+    const int lo_b = min(max(pex - jb, 0), 32), hi_b = min(max(pin - jb, 0), 32);
+    const int t = __shfl_sync(FULL, x, max(hi_b - 1, 0));   // the run of this lane's list ends at hi_b - 1
+    if (hi_b > lo_b) acc += t;
+  }
+  if (lane < cnt) {
+    const int e = e0 + lane;
+    sc3[e] = __ldcg(sc3 + e) + acc;
+    sc2[e] = __ldcg(c2s + lo + e);
+  }
+}
+
+__global__ void __launch_bounds__(LP_THREADS)
+local_path_onepass_kernel(const int *__restrict__ rowptr, const int *__restrict__ col, const int *__restrict__ tri,
+                          int n, int v_lo, int v_hi, const long long *__restrict__ offsets, int *pad_u, int *pad_c2,
+                          int *pad_c3, int *scratch, long long scratch_cap, unsigned int *owner_counter,
+                          unsigned int *__restrict__ counts_out, const int *__restrict__ owner_order, int n_order,
+                          int upper) {
+  extern __shared__ uint32_t sm[];
+  const int W = (n + 31) >> 5;
+  const int W2 = (W + 31) >> 5;
+  uint32_t *bm = sm;
+  uint32_t *bm2 = bm + W;
+  uint32_t *blk = bm2 + W2;
+  uint16_t *pre = reinterpret_cast<uint16_t *>(blk + W2);
+  __shared__ int s_owner, s_walk, s_walk3;
+  __shared__ uint32_t s_scan[LP_THREADS / 32];
+  __shared__ uint32_t s_carry, s_lo;
+  const int tid = threadIdx.x, lane = lane_id(), warp = tid >> 5;
+  constexpr int NW = LP_THREADS / 32;
+  int *c2s = scratch + (long long)blockIdx.x * scratch_cap;
+  for (int w = tid; w < W + W2; w += LP_THREADS) sm[w] = 0;
+  for (;;) {
+    __syncthreads();
+    if (tid == 0) {
+      const int t = (int)atomicAdd(owner_counter, 1u);
+      s_owner = (owner_order && t < n_order) ? v_lo + owner_order[t] : v_lo + t;
+      s_walk = 0;
+      s_walk3 = 0;
+    }
+    __syncthreads();
+    const int v = s_owner;
+    if (v >= v_hi) break;
+    const int vs = __ldg(rowptr + v), ve = __ldg(rowptr + v + 1);
+    int LG = 32;
+    while (LG > 1 && (ve - vs + LG - 1) / LG < 4 * NW) LG >>= 1;
+    const long long out_base = offsets[v - v_lo];
+    const long long slot = offsets[v - v_lo + 1] - out_base;
+    if (slot == 0) continue;                           // no candidate u >= umin (the bound says so): nothing to do
+    const int umin = upper ? v + 1 : 0;
+    // ---- walk 1: mark every candidate ----
+    walk_two_paths(rowptr, col, vs, ve, lane, LG, &s_walk, 0, MarkVisitor{bm, bm2});
+    __syncthreads();
+    for (int p = vs + tid; p < ve; p += LP_THREADS) {
+      const int k = __ldg(col + p);
+      atomicAnd(&bm[k >> 5], ~(1u << (k & 31)));
+    }
+    if (tid == 0) { atomicAnd(&bm[v >> 5], ~(1u << (v & 31))); s_carry = 0; s_walk = 0; }
+    __syncthreads();
+    // ---- rank (as twohop_score_kernel, from block 0) ----
+    for (int c = 0; c < W2; c += LP_THREADS) {
+      const int g = c + tid;
+      const uint32_t m2 = (g < W2) ? bm2[g] : 0u;
+      uint32_t cnt = 0;
+      for (uint32_t m = m2; m; m &= m - 1) {
+        const int w = g * 32 + __ffs(m) - 1;
+        pre[w] = (uint16_t)cnt;
+        cnt += __popc(bm[w]);
+      }
+      uint32_t inc = cnt;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t t = __shfl_up_sync(FULL, inc, d);
+        if (lane >= d) inc += t;
+      }
+      if (lane == 31) s_scan[warp] = inc;
+      __syncthreads();
+      uint32_t wbase = 0, tot = 0;
+#pragma unroll
+      for (int w = 0; w < NW; ++w) {
+        const uint32_t x = s_scan[w];
+        if (w < warp) wbase += x;
+        tot += x;
+      }
+      const uint32_t carry = s_carry;
+      if (g < W2) blk[g] = carry + wbase + (inc - cnt);
+      __syncthreads();
+      if (tid == 0) s_carry = carry + tot;
+    }
+    __syncthreads();
+    const uint32_t total = s_carry;
+    if (tid == 0) {                                    // lo = #candidates below umin
+      uint32_t r = total;
+      const int w0 = umin >> 5;
+      if (w0 < W) {
+        r = blk[w0 >> 5];
+        for (uint32_t m = bm2[w0 >> 5] & ((1u << (w0 & 31)) - 1u); m; m &= m - 1) r += __popc(bm[(w0 & ~31) + __ffs(m) - 1]);
+        r += __popc(bm[w0] & ((1u << (umin & 31)) - 1u));
+      }
+      s_lo = r;
+    }
+    __syncthreads();
+    const uint32_t lo = s_lo;
+    const bool fits = (long long)(total - lo) <= slot && (long long)total <= scratch_cap;
+    if (tid == 0) counts_out[v - v_lo] = fits ? total - lo : 0xffffffffu;
+    if (fits) {
+      // ---- emit u >= umin into the slot (c3 zeroed), zero the c2 scratch ----
+      for (int g = (umin >> 10) + tid; g < W2; g += LP_THREADS) {
+        for (uint32_t m = bm2[g]; m; m &= m - 1) {
+          const int w = g * 32 + __ffs(m) - 1;
+          uint32_t bits = bm[w];
+          uint32_t idx = blk[g] + pre[w];
+          const int below = umin - (w << 5);
+          if (below > 0) {
+            const uint32_t mask = below >= 32 ? 0xffffffffu : ((1u << below) - 1u);
+            idx += __popc(bits & mask);
+            bits &= ~mask;
+          }
+          for (; bits; bits &= bits - 1, ++idx) {
+            pad_u[out_base + (idx - lo)] = (w << 5) + __ffs(bits) - 1;
+            pad_c3[out_base + (idx - lo)] = 0;
+          }
+        }
+      }
+      for (uint32_t i = tid; i < total; i += LP_THREADS) c2s[i] = 0;
+      __syncthreads();
+      // ---- walk 2: c2 of every candidate, tri term of the emitted ones ----
+      LpScoreVisitor sv{bm, blk, pre, tri, c2s, pad_c3 + out_base, (int)lo, umin};
+      walk_two_paths(rowptr, col, vs, ve, lane, LG, &s_walk, 0, sv);
+      __syncthreads();
+      // ---- walk 3: 32 emitted candidates per warp, handed out dynamically ----
+      const int n_emit = (int)(total - lo);
+      for (;;) {
+        int b = 0;
+        if (lane == 0) b = atomicAdd(&s_walk3, 1);
+        const int e0 = __shfl_sync(FULL, b, 0) * 32;
+        if (e0 >= n_emit) break;
+        lp_walk3_batch(rowptr, col, bm, blk, pre, c2s, (int)lo, pad_u + out_base, pad_c2 + out_base,
+                       pad_c3 + out_base, e0, min(32, n_emit - e0));
+      }
+      __syncthreads();
+    }
+    // ---- cleanup ----
+    for (int g = tid; g < W2; g += LP_THREADS) {
+      for (uint32_t m = bm2[g]; m; m &= m - 1) bm[g * 32 + __ffs(m) - 1] = 0;
+      bm2[g] = 0;
+    }
+  }
+}
+
+// padded slot -> compact position, score from (c2, c3); work cut by compact position as in twohop_compact_kernel
+__global__ void __launch_bounds__(CP_THREADS)
+local_path_compact_kernel(const long long *__restrict__ pad_off, const long long *__restrict__ cmp_off, int v_lo,
+                          int n_own, long long cap, const int *__restrict__ pad_u, const int *__restrict__ pad_c2,
+                          const int *__restrict__ pad_c3, int *__restrict__ pair_u, int *__restrict__ pair_v,
+                          float *__restrict__ score, int *__restrict__ c2_out, int *__restrict__ c3_out) {
+  const long long N = cmp_off[n_own];
+  if (N > cap) return;
+  __shared__ int s_lo, s_hi;
+  const long long ntiles = (N + CP_TILE - 1) / CP_TILE;
+  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+    const long long base = tile * CP_TILE, end = min(base + (long long)CP_TILE, N);
+    __syncthreads();
+    if (threadIdx.x < 2) {
+      const long long x = threadIdx.x == 0 ? base : end - 1;
+      int lo = 0, hi = n_own;
+      while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (cmp_off[mid] <= x) lo = mid; else hi = mid;
+      }
+      if (threadIdx.x == 0) s_lo = lo; else s_hi = lo;
+    }
+    __syncthreads();
+    for (int q = 0; q < CP_PER; ++q) {
+      const long long i = base + q * CP_THREADS + threadIdx.x;
+      if (i >= end) break;
+      int lo = s_lo, hi = s_hi + 1;
+      while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (cmp_off[mid] <= i) lo = mid; else hi = mid;
+      }
+      const long long src = pad_off[lo] + (i - cmp_off[lo]);
+      const int c2 = pad_c2[src], c3 = pad_c3[src];
+      pair_u[i] = pad_u[src];
+      pair_v[i] = v_lo + lo;
+      if (score) score[i] = local_path_score(c2, c3);
+      if (c2_out) c2_out[i] = c2;
+      if (c3_out) c3_out[i] = c3;
+    }
+  }
+}
+
+// Arbitrary pairs: a CTA takes a tile of pairs; per run of equal v it holds the N(v) bitmap, and one warp per pair walks
+// N(u) (c2) and the N(j), j in N(u), as one flattened sequence (c3).  Work sum_{j in N(u)} deg j per pair: for
+// evaluation sets, not for filter candidates.  Runs may come in any order; callers sort by v to make them long.
+constexpr int LPP_THREADS = 512;
+constexpr int LPP_TILE = 1024;
+
+__global__ void __launch_bounds__(LPP_THREADS)
+local_path_pairs_kernel(const int *__restrict__ rowptr, const int *__restrict__ col, int n, const int *__restrict__ pu,
+                        const int *__restrict__ pv, long long M, float *__restrict__ score, int *__restrict__ c2_out,
+                        int *__restrict__ c3_out, unsigned long long *tile_counter) {
+  extern __shared__ uint32_t bitmap[];
+  __shared__ long long s_tile;
+  const int tid = threadIdx.x, lane = lane_id(), warp = tid >> 5;
+  constexpr int NW = LPP_THREADS / 32;
+  for (int w = tid; w < (n + 31) >> 5; w += LPP_THREADS) bitmap[w] = 0;
+  const long long ntiles = (M + LPP_TILE - 1) / LPP_TILE;
+  for (;;) {
+    __syncthreads();
+    if (tid == 0) s_tile = (long long)atomicAdd(tile_counter, 1ull);
+    __syncthreads();
+    const long long tile = s_tile;
+    if (tile >= ntiles) break;
+    const long long i1 = min(M, (tile + 1) * LPP_TILE);
+    for (long long i = tile * LPP_TILE; i < i1;) {
+      const int v = pv[i];
+      long long j = i + 1;                               // end of the run (uniform: every thread scans the same pv)
+      while (j < i1 && pv[j] == v) ++j;
+      const int vs = __ldg(rowptr + v), ve = __ldg(rowptr + v + 1);
+      for (int p = vs + tid; p < ve; p += LPP_THREADS) {
+        const int k = __ldg(col + p);
+        atomicOr(&bitmap[k >> 5], 1u << (k & 31));
+      }
+      __syncthreads();
+      for (long long q = i + warp; q < j; q += NW) {
+        const int u = pu[q];
+        const int su = __ldg(rowptr + u), lu = __ldg(rowptr + u + 1) - su;
+        int c2 = 0, c3 = 0;
+        for (int base = 0; base < lu; base += 32) {
+          const int p = base + lane;
+          int s = 0, len = 0;
+          if (p < lu) {
+            const int x = __ldg(col + su + p);
+            c2 += (bitmap[x >> 5] >> (x & 31)) & 1u;
+            s = __ldg(rowptr + x);
+            len = __ldg(rowptr + x + 1) - s;
+          }
+          int pin = len;
+#pragma unroll
+          for (int d = 1; d < 32; d <<= 1) {
+            const int t = __shfl_up_sync(FULL, pin, d);
+            if (lane >= d) pin += t;
+          }
+          const int pex = pin - len;
+          const int total = __shfl_sync(FULL, pin, 31);
+          for (int jb = 0; jb < total; jb += 32) {
+            const int pp = jb + lane;
+            int sl = 0;
+#pragma unroll
+            for (int step = 16; step >= 1; step >>= 1) {
+              const int t = __shfl_sync(FULL, pin, sl + step - 1);
+              if (t <= pp) sl += step;
+            }
+            const int s_t = __shfl_sync(FULL, s, sl);
+            const int pe_t = __shfl_sync(FULL, pex, sl);
+            if (pp < total) {
+              const int k = __ldg(col + s_t + (pp - pe_t));
+              c3 += (bitmap[k >> 5] >> (k & 31)) & 1u;
+            }
+          }
+        }
+        c2 = __reduce_add_sync(FULL, c2);
+        c3 = __reduce_add_sync(FULL, c3);
+        if (lane == 0) {
+          if (score) score[q] = local_path_score(c2, c3);
+          if (c2_out) c2_out[q] = c2;
+          if (c3_out) c3_out[q] = c3;
+        }
+      }
+      __syncthreads();
+      for (int p = vs + tid; p < ve; p += LPP_THREADS) bitmap[__ldg(col + p) >> 5] = 0;
+      __syncthreads();
+      i = j;
+    }
+  }
+}
+
 }  // namespace eps
 
 extern "C" int eps_score_kinds(void) {
@@ -682,5 +1075,118 @@ extern "C" int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, con
                                                      cn, flags, pair_u, pair_v, score, count);
     EPS_LAUNCH_CHECK();
   }
+  return EPS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Local Path index entry points
+// ---------------------------------------------------------------------------------------------
+extern "C" size_t eps_local_path_onepass_workspace_bytes(int64_t cap, int32_t n_owners, int64_t max_count,
+                                                         int32_t ctas) {
+  const size_t c = (size_t)(cap > 0 ? cap : 0), o = (size_t)(n_owners > 0 ? n_owners : 0);
+  const size_t s = (size_t)(max_count > 0 ? max_count : 0) * (size_t)(ctas > 0 ? ctas : 0);
+  // ticket | work buckets | per-owner counts | owner order | padded u | padded c2 | padded c3 | per-CTA c2 scratch
+  return 512 + 2 * up256(o * 4) + 3 * up256(c * 4) + up256(s * 4);
+}
+
+extern "C" int eps_local_path_onepass(const int32_t *rowptr, const int32_t *col, const int32_t *tri, int32_t n,
+                                      int32_t v_lo, int32_t v_hi, const int64_t *bound_offsets, int64_t cap,
+                                      int64_t max_count, int32_t ctas, int flags, int32_t *pair_u, int32_t *pair_v,
+                                      float *score, int32_t *c2, int32_t *c3, int64_t *offsets_out, void *workspace,
+                                      size_t workspace_bytes, void *stream_) {
+  using namespace eps;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  EPS_CHECK_ARG(rowptr && col && tri && bound_offsets && offsets_out,
+                "null graph, tri, bound_offsets or offsets_out pointer");
+  EPS_CHECK_ARG(n > 0 && v_lo >= 0 && v_hi <= n && v_lo < v_hi && cap >= 0 && cap < (1ll << 31),
+                "bad owner range or cap");
+  EPS_CHECK_ARG(max_count >= 0 && max_count < (1ll << 31) && ctas >= 1, "bad max_count or ctas");
+  EPS_CHECK_ARG(cap == 0 || (pair_u && pair_v), "missing pair output pointer");
+  EPS_CHECK_ARG(!(flags & ~EPS_TWOHOP_UPPER), "unknown flag bits");
+  const int n_own = v_hi - v_lo;
+  if (!workspace || workspace_bytes < eps_local_path_onepass_workspace_bytes(cap, n_own, max_count, ctas)) {
+    set_error("eps_local_path_onepass: workspace too small");
+    return EPS_ERR_WORKSPACE;
+  }
+  const int sms = sm_count();
+  if (sms <= 0) { set_error("eps_local_path_onepass: no CUDA device"); return EPS_ERR_CUDA; }
+  const int W = (n + 31) / 32, W2 = (W + 31) / 32;
+  const size_t smem = (size_t)(W + 2 * W2) * 4 + (size_t)W * 2 + 16;
+  if (smem > 200 * 1024) {
+    set_error("eps_local_path_onepass: n=%d needs %zu bytes of shared memory (> 200 KB)", n, smem);
+    return EPS_ERR_UNSUPPORTED;
+  }
+  uint8_t *ws = (uint8_t *)workspace;
+  unsigned int *buckets = (unsigned int *)(ws + 256);
+  unsigned int *counts = (unsigned int *)(ws + 512);
+  int *order = (int *)(ws + 512 + up256((size_t)n_own * 4));
+  int *pad_u = (int *)(ws + 512 + 2 * up256((size_t)n_own * 4));
+  int *pad_c2 = (int *)((uint8_t *)pad_u + up256((size_t)cap * 4));
+  int *pad_c3 = (int *)((uint8_t *)pad_c2 + up256((size_t)cap * 4));
+  int *scratch = (int *)((uint8_t *)pad_c3 + up256((size_t)cap * 4));
+  EPS_CUDA(cudaMemsetAsync(ws, 0, 512 + up256((size_t)n_own * 4), stream));   // ticket + buckets + counts
+  EPS_CUDA(cudaFuncSetAttribute(local_path_onepass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int occ = 0;
+  EPS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, local_path_onepass_kernel, LP_THREADS, smem));
+  if (occ < 1) occ = 1;
+  const int grid = (int)std::min<long long>(std::min<long long>((long long)n_own, (long long)sms * occ), ctas);
+  {
+    const int ogrid = std::min((n_own + 255) / 256, sms * 8);
+    owner_bucket_kernel<0><<<ogrid, 256, 0, stream>>>((const long long *)bound_offsets, n_own, buckets, order);
+    owner_bucket_kernel<1><<<1, 64, 0, stream>>>((const long long *)bound_offsets, n_own, buckets, order);
+    owner_bucket_kernel<2><<<ogrid, 256, 0, stream>>>((const long long *)bound_offsets, n_own, buckets, order);
+    EPS_LAUNCH_CHECK();
+  }
+  local_path_onepass_kernel<<<grid, LP_THREADS, smem, stream>>>(
+      rowptr, col, tri, n, v_lo, v_hi, (const long long *)bound_offsets, pad_u, pad_c2, pad_c3, scratch,
+      (long long)max_count, (unsigned int *)ws, counts, order, n_own, (flags & EPS_TWOHOP_UPPER) ? 1 : 0);
+  EPS_LAUNCH_CHECK();
+  owner_scan_kernel<<<1, 1024, 0, stream>>>(counts, n_own, (long long *)offsets_out);
+  EPS_LAUNCH_CHECK();
+  if (cap > 0) {
+    const int cgrid = (int)std::min<long long>((cap + CP_TILE - 1) / CP_TILE, (long long)sms * 8);
+    local_path_compact_kernel<<<cgrid, CP_THREADS, 0, stream>>>((const long long *)bound_offsets,
+                                                              (const long long *)offsets_out, v_lo, n_own,
+                                                              (long long)cap, pad_u, pad_c2, pad_c3, pair_u, pair_v,
+                                                              score, c2, c3);
+    EPS_LAUNCH_CHECK();
+  }
+  return EPS_OK;
+}
+
+extern "C" size_t eps_local_path_pairs_workspace_bytes(void) { return 256; }
+
+extern "C" int eps_local_path_pairs(const int32_t *rowptr, const int32_t *col, int32_t n, const int32_t *pair_u,
+                                    const int32_t *pair_v, int64_t M, int flags, float *score, int32_t *c2,
+                                    int32_t *c3, void *workspace, size_t workspace_bytes, void *stream_) {
+  using namespace eps;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  EPS_CHECK_ARG(n > 0 && M >= 0, "bad n or M");
+  EPS_CHECK_ARG(flags == 0, "unknown flag bits");
+  if (M == 0) return EPS_OK;
+  EPS_CHECK_ARG(rowptr && col && pair_u && pair_v, "null graph or pair pointer");
+  EPS_CHECK_ARG(score || c2 || c3, "score, c2 and c3 all NULL");
+  if (!workspace || workspace_bytes < eps_local_path_pairs_workspace_bytes()) {
+    set_error("eps_local_path_pairs: workspace too small");
+    return EPS_ERR_WORKSPACE;
+  }
+  const size_t bitmap_bytes = (size_t)((n + 31) / 32) * 4;
+  if (bitmap_bytes > 200 * 1024) {
+    set_error("eps_local_path_pairs: n=%d needs %zu bytes of shared memory (> 200 KB)", n, bitmap_bytes);
+    return EPS_ERR_UNSUPPORTED;
+  }
+  const int sms = sm_count();
+  if (sms <= 0) { set_error("eps_local_path_pairs: no CUDA device"); return EPS_ERR_CUDA; }
+  EPS_CUDA(cudaMemsetAsync(workspace, 0, 8, stream));
+  EPS_CUDA(cudaFuncSetAttribute(local_path_pairs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)bitmap_bytes));
+  int occ = 0;
+  EPS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, local_path_pairs_kernel, LPP_THREADS, bitmap_bytes));
+  if (occ < 1) occ = 1;
+  const long long ntiles = (M + LPP_TILE - 1) / LPP_TILE;
+  const int grid = (int)std::min<long long>(ntiles, (long long)sms * occ);
+  local_path_pairs_kernel<<<grid, LPP_THREADS, bitmap_bytes, stream>>>(rowptr, col, n, pair_u, pair_v, (long long)M,
+                                                                     score, c2, c3, (unsigned long long *)workspace);
+  EPS_LAUNCH_CHECK();
   return EPS_OK;
 }

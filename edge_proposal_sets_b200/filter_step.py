@@ -33,7 +33,7 @@ import torch
 
 from . import adamic_utils, candidates, ops, parallel
 from .graph import SparseAdj, add_edges
-from .models import GNN_MODELS, SIMILARITY_MODELS, LinkGNN
+from .models import GNN_MODELS, LOCAL_PATH, SIMILARITY_MODELS, LinkGNN
 
 
 def score_edges(model_name: str, model, x, adj: SparseAdj, edges: torch.Tensor,
@@ -45,6 +45,8 @@ def score_edges(model_name: str, model, x, adj: SparseAdj, edges: torch.Tensor,
         return model.linkpred.score_pairs(h, edges)
     if model_name in SIMILARITY_MODELS:
         return ops.cn_aa(adj, edges, kind=model_name, grouped_by_v=grouped_by_v)
+    if model_name == LOCAL_PATH:
+        return ops.local_path(adj, edges)                    # pair lists (rank side); filter jobs take the fused walk
     if model_name in ("simple", "adamic"):
         model.grouped_by_v = grouped_by_v
         return model(x, edges, adj)
@@ -67,9 +69,9 @@ def heuristic_table(model_name: str, adj: SparseAdj, ra_adj: Optional[SparseAdj]
     """(graph, weight table, sigmoid, use_values, kind) of a heuristic filter model when it can take the fused
     enumerate+score kernel (K6+K3, candidates.two_hop_scored): the scoring graph IS the graph whose 2-hop
     neighbourhood defines the candidates and, if weighted (collab), its values are bitwise symmetric.
-    ``None`` otherwise (RA on a rebuilt multigraph) -> two_hop + ops.cn_aa.  ``kind``: the similarity models
-    (structure only, so on weighted graphs too), else ``None``."""
-    if model_name in SIMILARITY_MODELS:
+    ``None`` otherwise (RA on a rebuilt multigraph) -> two_hop + ops.cn_aa.  ``kind``: the similarity models and
+    ``local_path`` (structure only, so on weighted graphs too), else ``None``."""
+    if model_name in SIMILARITY_MODELS or model_name == LOCAL_PATH:
         return adj, None, False, False, model_name
     if not candidates.values_symmetric(adj):
         return None
@@ -127,10 +129,15 @@ def owner_cost(adj: SparseAdj, jobs, upper: bool = False) -> torch.Tensor:
     0.218 ns per candidate against 0.029 ns per 2-path), and the candidate count is bounded by the owner's slot size
     (candidates.owner_bounds).  Balancing on 2-paths alone left the ranks with few hubs 5 % more candidates and the
     others waiting at the merge (N = 4: 33 ms of a 615 ms step).  ``upper`` (mirror mode): the same model on the half
-    work — the 2-paths that end above v and the half-candidate bound — which low owner ids carry most of."""
+    work — the 2-paths that end above v and the half-candidate bound — which low owner ids carry most of.  A
+    ``local_path`` job adds its walk-3 pull work (``candidates.local_path_work``, one list element ~ one 2-path visit),
+    ~160x the 2-path count on the ppa shape: it decides the balance."""
     work = (candidates.half_two_path_work(adj) if upper else candidates.two_path_work(adj)).double()
-    if any((j.name if hasattr(j, "name") else j[0]) in GNN_MODELS for j in jobs):
+    names = [j.name if hasattr(j, "name") else j[0] for j in jobs]
+    if any(nm in GNN_MODELS for nm in names):
         work = work + 8.0 * candidates.owner_bounds(adj, upper).double()
+    if LOCAL_PATH in names:
+        work = work + candidates.local_path_work(adj, upper).double()
     return work
 
 
@@ -436,9 +443,15 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
     if world > 1:
         bounds = parallel.partition_by_work(owner_cost(adj, jobs, half)[o_lo:o_hi], world)
         v_lo, v_hi = o_lo + bounds[rank], o_lo + bounds[rank + 1]
-    # per job: scoring plan + running proposal set
+    # per job: scoring plan + running proposal set.  A local_path job always takes the fused walk (its pair kernel is for
+    # evaluation sets, ~Σ deg u of work per candidate); the other heuristic jobs then go to K3.
+    lp = [i for i, j in enumerate(jobs) if j.name == LOCAL_PATH]
+    if len(lp) > 1:
+        raise ValueError("one filter call takes at most one local_path job (only the fused walk scores its candidates)")
+    if lp:
+        candidates.require_symmetric(adj, "filter_topk(local_path)")
     plans = []
-    fused_job = None
+    fused_job = lp[0] if lp else None
     for j in jobs:
         if j.name in GNN_MODELS:
             assert isinstance(j.model, LinkGNN)
@@ -460,6 +473,9 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
                 fused_job = len(plans)
             plans.append(dict(kind="heuristic", table=table, pn_kept=0, pool=None, run=RunningTopK(k, None, pushdown)))
     ph.mark("embed")
+    if lp:
+        candidates.arc_triangles(adj)                        # tri table of the LP walk: once per graph
+        ph.mark("triangles")
     n_slabs = 0
     n_cand = 0
     for lo, hi, cap in iter_slabs(adj, v_lo, v_hi, slab_pairs, half):

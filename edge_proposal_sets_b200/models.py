@@ -7,7 +7,8 @@ reference's ``models.py`` so its checkpoints load unchanged and its callers
   LinkGNN              /root/reference/models.py:487-506
   CommonNeighborsPredictor ('simple' | 'adamic' | 'adamic_ogb' | 'resource_allocation')
                        /root/reference/models.py:508-554, plus the degree-normalised similarities of
-                       SIMILARITY_MODELS (no reference counterpart; include/eps.h EPS_SCORE_*)
+                       SIMILARITY_MODELS (no reference counterpart; include/eps.h EPS_SCORE_*) and the
+                       Local Path index 'local_path' (no reference counterpart; include/eps.h eps_local_path_*)
   build_model          /root/reference/models.py:578-670
   default_model_configs/root/reference/models.py:673-790
 
@@ -41,7 +42,10 @@ GNN_MODELS = ("gcn", "sage")
 # symmetric, computed from the exact common-neighbour count by the same kernels (``ops.cn_aa(kind=...)``)
 SIMILARITY_MODELS = ("jaccard", "sorensen", "salton", "hub_promoted", "hub_depressed", "leicht_holme_newman",
                      "preferential_attachment")
-HEURISTIC_MODELS = ("simple", "adamic", "adamic_ogb", "resource_allocation") + SIMILARITY_MODELS
+# the Local Path index (Lue, Jin & Zhou 2009): (A^2)_uv + 1e-3 (A^3)_uv, structural and symmetric
+# (``candidates.two_hop_local_path`` on the filter side, ``ops.local_path`` on pair lists)
+LOCAL_PATH = "local_path"
+HEURISTIC_MODELS = ("simple", "adamic", "adamic_ogb", "resource_allocation") + SIMILARITY_MODELS + (LOCAL_PATH,)
 SUPPORTED_MODELS = GNN_MODELS + HEURISTIC_MODELS
 
 
@@ -284,6 +288,8 @@ class CommonNeighborsPredictor(nn.Module):
             return None                            # reference behaviour (models.py:534-535)
         if self.type in SIMILARITY_MODELS:
             return ops.cn_aa(adj, edges, kind=self.type, grouped_by_v=self.grouped_by_v)
+        if self.type == LOCAL_PATH:
+            return ops.local_path(adj, edges)
         if self.type == "simple":
             # sum_k adj[u,k]*adj[v,k]; raw value, no sigmoid (models.py:539-542)
             return ops.cn_aa(adj, edges, None, use_values=True, grouped_by_v=self.grouped_by_v)

@@ -140,6 +140,41 @@ def cn_aa(adj: SparseAdj, edges: torch.Tensor, wtable: Optional[torch.Tensor] = 
     return (score, count) if want_count else score
 
 
+def local_path(adj: SparseAdj, edges: torch.Tensor, want_counts: bool = False):
+    """Local Path index of arbitrary pairs (eps_local_path_pairs): score fp32 [M] (+ c2, c3 int32 [M] with
+    ``want_counts``), the same bits as the fused filter kernel (``candidates.two_hop_local_path``) on the same pair.
+    A pair costs sum_{j in N(u)} deg j: meant for evaluation sets.  The pairs are run sorted by v (one N(v) bitmap
+    per run) and the results put back in input order.  Structure only; the graph must be structurally symmetric."""
+    from .candidates import require_symmetric
+    require_symmetric(adj, "local_path")
+    _need_cuda(adj.col, edges)
+    lib = _lib.load()
+    pu, pv = _pairs(edges)
+    M = pu.numel()
+    dev = adj.device
+    score = torch.empty(M, dtype=torch.float32, device=dev)
+    c2 = torch.empty(M, dtype=torch.int32, device=dev) if want_counts else None
+    c3 = torch.empty(M, dtype=torch.int32, device=dev) if want_counts else None
+    if M:
+        order = torch.argsort(pv, stable=True)
+        su, sv = pu[order].contiguous(), pv[order].contiguous()
+        ss = torch.empty_like(score)
+        s2 = torch.empty(M, dtype=torch.int32, device=dev) if want_counts else None
+        s3 = torch.empty(M, dtype=torch.int32, device=dev) if want_counts else None
+        ws = _ws(lib.eps_local_path_pairs_workspace_bytes(), dev)
+        ev = _event_pair("local_path_pairs")
+        check(lib.eps_local_path_pairs(_ptr(adj.rowptr), _ptr(adj.col), adj.n, _ptr(su), _ptr(sv), M, 0, _ptr(ss),
+                                       _ptr(s2), _ptr(s3), _ptr(ws), ws.numel(), _stream()), "eps_local_path_pairs")
+        if ev is not None:
+            ev[1].record()
+        LAUNCHES["n"] += 1
+        score[order] = ss
+        if want_counts:
+            c2[order] = s2
+            c3[order] = s3
+    return (score, c2, c3) if want_counts else score
+
+
 # K2 arms: "fp32" = FFMA (reference arithmetic); "f16" = tcgen05 tensor cores, fp16 operands / fp32 accumulate
 # ("tc" and the round-1 name "bf16" are aliases)
 MLP_PRECISIONS = {"fp32": EPS_MLP_FP32, "f16": EPS_MLP_TC_F16, "tc": EPS_MLP_TC_F16, "bf16": EPS_MLP_TC_F16}

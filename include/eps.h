@@ -381,6 +381,46 @@ int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, const float *v
 size_t eps_twohop_onepass_workspace_bytes(int64_t cap, int32_t n_owners);
 
 /* ---------------------------------------------------------------------------
+ * Local Path index  LP(u, v) = (A^2)_uv + 1e-3 * (A^3)_uv   (Lue & Zhou)
+ * replaces: no reference counterpart (a heuristic filter / rank model of this
+ *           project, 'local_path').  Structure only: N(x) is the stored list
+ *           (self loops included), edge values are ignored.
+ *   c2 = |N(u) & N(v)|,  c3 = sum_{j in N(u)} |N(j) & N(v)|   (exact int32: c3 <= nnz < 2^31)
+ *   score = __double2float_rn(__dadd_rn((double)c2, __dmul_rn(1e-3, (double)c3)))
+ * The adjacency must be structurally symmetric ((u,k) stored <=> (k,u) stored,
+ * no repeated entry); the caller checks it.
+ *
+ * eps_local_path_onepass: the eps_twohop_onepass contract (padded slots sized
+ *   by bound_offsets / cap, per-owner counts, offsets_out, heaviest owners
+ *   first, EPS_TWOHOP_UPPER) for the Local Path score, from one fused walk.
+ *   tri        int32[nnz]: tri[p] = |N(v) & N(col[p])| for the stored arc p of
+ *              row v (eps_cn_aa counts of the pairs (col[p], v))
+ *   max_count  an upper bound of EVERY owner's full candidate count (u > v
+ *              or not) in [v_lo, v_hi); sizes the per-CTA c2 scratch
+ *   ctas       number of per-CTA scratch areas in the workspace; the kernel
+ *              runs at most that many CTAs
+ *   flags      0 or EPS_TWOHOP_UPPER (only u > v is emitted; bound_offsets
+ *              then bound the half counts)
+ *   score / c2 / c3  fp32 / int32 / int32 [cap] or NULL each
+ * Workspace: eps_local_path_onepass_workspace_bytes(cap, v_hi - v_lo, max_count, ctas).
+ *
+ * eps_local_path_pairs: c2, c3 and the score of any pair list (u == v, edges
+ *   and isolated ends included).  One CTA holds the N(v) bitmap per run of
+ *   equal pair_v; a pair costs sum_{j in N(u)} deg j, so sort the pairs by v
+ *   and keep this for evaluation sets.  flags must be 0.
+ * Both need n/8 + ... bytes of shared memory (<= 200 KB) like the K6 kernels.
+ * ------------------------------------------------------------------------- */
+int eps_local_path_onepass(const int32_t *rowptr, const int32_t *col, const int32_t *tri, int32_t n, int32_t v_lo,
+                           int32_t v_hi, const int64_t *bound_offsets, int64_t cap, int64_t max_count, int32_t ctas,
+                           int flags, int32_t *pair_u, int32_t *pair_v, float *score, int32_t *c2, int32_t *c3,
+                           int64_t *offsets_out, void *workspace, size_t workspace_bytes, void *stream);
+size_t eps_local_path_onepass_workspace_bytes(int64_t cap, int32_t n_owners, int64_t max_count, int32_t ctas);
+int eps_local_path_pairs(const int32_t *rowptr, const int32_t *col, int32_t n, const int32_t *pair_u,
+                         const int32_t *pair_v, int64_t M, int flags, float *score, int32_t *c2, int32_t *c3,
+                         void *workspace, size_t workspace_bytes, void *stream);
+size_t eps_local_path_pairs_workspace_bytes(void);
+
+/* ---------------------------------------------------------------------------
  * K5  multi-GPU merge of per-GPU proposal lists (no counterpart in the
  * single-GPU reference; SURVEY.md section 8e).  One ncclAllGather of the
  * [k_local,3] fp32 (u, v, score) rows of every rank followed by a K4 select
