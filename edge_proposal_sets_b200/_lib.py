@@ -17,7 +17,7 @@ EPS_VERSION = 203          # must equal EPS_VERSION in include/eps.h (checked by
 EPS_REDUCE_SUM, EPS_REDUCE_MEAN = 0, 1
 EPS_CN_SIGMOID, EPS_CN_GROUPED_BY_V = 1, 2
 EPS_TWOHOP_UPPER = 4       # eps_twohop_onepass: only the candidates u > v of every owner v
-# degree-normalised similarity scores: a 3-bit kind field at bit 8 of the eps_cn_aa / eps_twohop_* flags
+# degree-normalised similarity scores: a 3-bit kind field at bit 8 of the eps_cn_aa / eps_twohop_onepass flags
 EPS_SCORE_KIND_SHIFT = 8
 EPS_SCORE_KIND_MASK = 7 << EPS_SCORE_KIND_SHIFT
 SCORE_KINDS = {"jaccard": 1, "sorensen": 2, "salton": 3, "hub_promoted": 4, "hub_depressed": 5,
@@ -57,10 +57,6 @@ SIGNATURES = {
     "eps_segment_topk_select": (_int, [_vp, _i64, _vp, _i64, _i64, C.c_float, _int, _vp, _vp, _sz, _vp]),
     "eps_segment_topk_write": (_int, [_vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "eps_gather_pairs2": (_int, [_vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _vp]),
-    "eps_twohop_candidates": (_int, [_vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
-    "eps_twohop_workspace_bytes": (_sz, []),
-    "eps_twohop_scored": (_int, [_vp, _vp, _vp, _i32, _i32, _i32, _vp, _i64, _int, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
-    "eps_twohop_scored_workspace_bytes": (_sz, [_i64]),
     "eps_twohop_onepass": (_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _i64, _int, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "eps_twohop_onepass_workspace_bytes": (_sz, [_i64, _i32]),
     "eps_local_path_onepass": (_int, [_vp, _vp, _vp, _i32, _i32, _i32, _vp, _i64, _i64, _i32, _int, _vp, _vp, _vp, _vp,

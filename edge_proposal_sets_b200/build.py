@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libeps_b200.so")
-SOURCES = ["eps_abi.cu", "cn_aa.cu", "topk.cu", "spmm.cu", "gcn_norm.cu", "linkpred_simt.cu", "linkpred_tc.cu", "candgen.cu", "twohop_score.cu", "comm.cu", "pair_hadamard.cu"]
+SOURCES = ["eps_abi.cu", "cn_aa.cu", "topk.cu", "spmm.cu", "gcn_norm.cu", "linkpred_simt.cu", "linkpred_tc.cu", "twohop_score.cu", "comm.cu", "pair_hadamard.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--expt-relaxed-constexpr",

@@ -18,19 +18,16 @@ from .ops import _need_cuda, _ptr, _stream, _ws
 
 
 def owner_counts(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None) -> torch.Tensor:
-    """#candidates of every owner v in [v_lo, v_hi) as int64."""
+    """#candidates of every owner v in [v_lo, v_hi) as int64: the differences of the one-pass offsets, enumerated in
+    owner ranges of at most 2^27 bounded candidates (filter_step.iter_slabs), so a large graph needs no buffer of all
+    its candidates."""
+    from .filter_step import iter_slabs
     _need_cuda(adj.col)
-    lib = _lib.load()
     v_hi = adj.n if v_hi is None else v_hi
-    counts = torch.zeros(max(v_hi - v_lo, 0), dtype=torch.int32, device=adj.device)
-    if v_hi <= v_lo:
-        return counts.long()
-    ws = _ws(lib.eps_twohop_workspace_bytes(), adj.device)
-    check(lib.eps_twohop_candidates(_ptr(adj.rowptr), _ptr(adj.col), adj.n, v_lo, v_hi, None, _ptr(counts),
-                                    None, None, _ptr(ws), ws.numel(), _stream()), "eps_twohop_candidates")
-    from . import ops as _ops
-    _ops.LAUNCHES["n"] += 1 if v_hi > v_lo else 0
-    return counts.long() & 0xFFFFFFFF
+    parts = [torch.zeros(0, dtype=torch.int64, device=adj.device)]
+    for lo, hi, cap in iter_slabs(adj, v_lo, v_hi, 1 << 27):
+        parts.append(two_hop(adj, lo, hi, cap=cap, want_offsets=True)[1].diff())
+    return torch.cat(parts)
 
 
 def owner_bounds(adj: SparseAdj, upper: bool = False) -> torch.Tensor:
@@ -154,6 +151,27 @@ def values_symmetric(adj: SparseAdj) -> bool:
     return adj._cache["val_sym"]
 
 
+def _slot_offsets(bounds: torch.Tensor, cap: int | None):
+    """(boff, cap): the padded slot offsets of the one-pass entry points (exclusive prefix of the per-owner ``bounds``,
+    int64 [n_own + 1]) and their total, which sizes the outputs (``cap``, when the caller already has it on the host,
+    saves a sync)."""
+    boff = torch.zeros(bounds.numel() + 1, dtype=torch.int64, device=bounds.device)
+    torch.cumsum(bounds, 0, out=boff[1:])
+    cap = int(boff[-1].item()) if cap is None else int(cap)
+    if cap >= 2**31:
+        raise EpsError(f"up to {cap} candidates in one slab; split the owner range (see filter_step.iter_slabs)")
+    return boff, cap
+
+
+def _compact_size(offsets: torch.Tensor, cap: int, what: str) -> int:
+    """N = offsets[-1], the one host sync of a one-pass call (it sizes the later launches); raises when an owner's
+    candidates exceeded its bound (the kernel then poisons N instead of overrunning the slot)."""
+    N = int(offsets[-1].item())
+    if N > cap:
+        raise EpsError(f"{what}: an owner's candidates exceed the caller's bound (N={N}, cap={cap})")
+    return N
+
+
 def _onepass(adj: SparseAdj, wtable, v_lo: int, v_hi: int, bounds, sigmoid: bool, want_score: bool, want_count: bool,
              cap: int | None = None, val: torch.Tensor | None = None, upper: bool = False, kind_flags: int = 0):
     """eps_twohop_onepass: (edges int32 [2,N] view, score | None, count | None, offsets int64 [n_own+1]).
@@ -170,11 +188,7 @@ def _onepass(adj: SparseAdj, wtable, v_lo: int, v_hi: int, bounds, sigmoid: bool
                 torch.empty(0, dtype=torch.int32, device=dev) if want_count else None, z)
     if bounds is None:
         bounds = owner_bounds(adj, upper)[v_lo:v_hi]
-    boff = torch.zeros(n_own + 1, dtype=torch.int64, device=dev)
-    torch.cumsum(bounds, 0, out=boff[1:])
-    cap = int(boff[-1].item()) if cap is None else int(cap)
-    if cap >= 2**31:
-        raise EpsError(f"up to {cap} candidates in one slab; split the owner range (see filter_step.iter_slabs)")
+    boff, cap = _slot_offsets(bounds, cap)
     buf = torch.empty((2, max(cap, 1)), dtype=torch.int32, device=dev)
     score = torch.empty(max(cap, 1), dtype=torch.float32, device=dev) if want_score else None
     count = torch.empty(max(cap, 1), dtype=torch.int32, device=dev) if want_count else None
@@ -187,69 +201,42 @@ def _onepass(adj: SparseAdj, wtable, v_lo: int, v_hi: int, bounds, sigmoid: bool
                                  _ptr(count), _ptr(offsets), _ptr(ws), ws.numel(), _stream()), "eps_twohop_onepass")
     from . import ops as _ops
     _ops.LAUNCHES["n"] += 3
-    N = int(offsets[-1].item())                 # the one host sync of the slab (sizes the later launches)
-    if N > cap:
-        raise EpsError(f"eps_twohop_onepass: an owner's candidates exceed the caller's bound (N={N}, cap={cap})")
+    N = _compact_size(offsets, cap, "eps_twohop_onepass")
     return (buf[:, :N], None if score is None else score[:N], None if count is None else count[:N], offsets)
 
 
-def two_hop(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, counts: torch.Tensor | None = None,
-            cap: int | None = None, want_offsets: bool = False, upper: bool = False):
-    """(u, v) candidate list of owners [v_lo, v_hi): int32 [2, N], column-major reference order.
-    ``counts`` (from ``owner_counts``) selects the two-pass kernels; without it the one-pass kernel
-    runs (no count pass) and the result is a [2, N] view of a buffer sized by the owner_bounds sum
-    (``cap`` = that sum, when the caller already has it on the host).  ``want_offsets`` returns
-    ``(edges, offsets)``: offsets int64 [v_hi - v_lo + 1], owner v's candidates are
-    ``edges[:, offsets[v - v_lo]:offsets[v - v_lo + 1]]`` (the segments of ``ops.segment_topk``).
-    ``upper`` (one pass only): only the candidates u > v of every owner v — each unordered pair once on a
-    structurally symmetric graph; ``cap`` is then the sum of ``half_bounds``."""
+def two_hop(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, cap: int | None = None,
+            want_offsets: bool = False, upper: bool = False):
+    """(u, v) candidate list of owners [v_lo, v_hi): int32 [2, N], column-major reference order, from the one-pass
+    kernel (no count pass): a [2, N] view of a buffer sized by the owner_bounds sum (``cap`` = that sum, when the caller
+    already has it on the host).  ``want_offsets`` returns ``(edges, offsets)``: offsets int64 [v_hi - v_lo + 1], owner
+    v's candidates are ``edges[:, offsets[v - v_lo]:offsets[v - v_lo + 1]]`` (the segments of ``ops.segment_topk``).
+    ``upper``: only the candidates u > v of every owner v — each unordered pair once on a structurally symmetric graph;
+    ``cap`` is then the sum of ``half_bounds``."""
     _need_cuda(adj.col)
-    lib = _lib.load()
     v_hi = adj.n if v_hi is None else v_hi
-    if upper and counts is not None:
-        raise EpsError("two_hop: the upper-triangle mode is one-pass only (no `counts`)")
-    if counts is None:
-        # one pass: padded per-owner slots sized by owner_bounds, compacted by the finalize pass
-        r = _onepass(adj, None, v_lo, v_hi, None, False, False, False, cap, upper=upper)
-        return (r[0], r[3]) if want_offsets else r[0]
-    offsets = torch.zeros(counts.numel() + 1, dtype=torch.int64, device=adj.device)
-    torch.cumsum(counts, 0, out=offsets[1:])
-    N = int(offsets[-1].item())
-    if N >= 2**31:
-        raise EpsError(f"{N} candidates in one slab; split the owner range (see filter_step.iter_slabs)")
-    edges = torch.empty((2, N), dtype=torch.int32, device=adj.device)
-    if N == 0:
-        return (edges, offsets) if want_offsets else edges
-    ws = _ws(lib.eps_twohop_workspace_bytes(), adj.device)
-    check(lib.eps_twohop_candidates(_ptr(adj.rowptr), _ptr(adj.col), adj.n, v_lo, v_hi, _ptr(offsets), None,
-                                    _ptr(edges[0]), _ptr(edges[1]), _ptr(ws), ws.numel(), _stream()),
-          "eps_twohop_candidates")
-    from . import ops as _ops
-    _ops.LAUNCHES["n"] += 1
-    return (edges, offsets) if want_offsets else edges
+    r = _onepass(adj, None, v_lo, v_hi, None, False, False, False, cap, upper=upper)
+    return (r[0], r[3]) if want_offsets else r[0]
 
 
 def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int = 0, v_hi: int | None = None,
-                   counts: torch.Tensor | None = None, sigmoid: bool = False, want_count: bool = False,
-                   cap: int | None = None, use_values: bool = True, want_offsets: bool = False,
-                   upper: bool = False, kind: str | None = None):
+                   sigmoid: bool = False, want_count: bool = False, cap: int | None = None, use_values: bool = True,
+                   want_offsets: bool = False, upper: bool = False, kind: str | None = None):
     """K6+K3 fused: the candidates of owners [v_lo, v_hi) AND their heuristic scores from one walk
     over the owners' 2-paths (``wtable=None`` -> CN count, else sum of ``wtable[k]`` over the common
     neighbours: AA with 1/log deg, RA with 1/deg).  Returns ``(edges int32 [2,N], score fp32 [N])``
     (+ ``count int32 [N]`` with ``want_count``); scores are bit-identical to ``ops.cn_aa`` on the
     same pairs.  A weighted adjacency (collab, ``use_values``) contributes A[u,k]*(A[v,k]*wtable[k]) per
-    2-path on the one-pass kernel; ``use_values=False`` ignores the values ('adamic', models.py:544-554).
-    Without ``counts`` the one-pass kernel runs: no count pass, outputs are views of buffers sized by
-    the owner_bounds sum of the range.  ``want_offsets`` appends the per-owner offsets (int64
-    [v_hi - v_lo + 1], as in ``two_hop``) to the returned tuple.  ``upper``: as in ``two_hop``.
+    2-path; ``use_values=False`` ignores the values ('adamic', models.py:544-554).  One-pass kernel, no count
+    pass: outputs are views of buffers sized by the owner_bounds sum of the range.  ``want_offsets`` appends the
+    per-owner offsets (int64 [v_hi - v_lo + 1], as in ``two_hop``) to the returned tuple.  ``upper``: as in ``two_hop``.
     ``kind`` (a name of ``_lib.SCORE_KINDS``, e.g. "jaccard"): a degree-normalised similarity of the exact count and
     the degrees of both ends instead (include/eps.h, EPS_SCORE_*): structure only, so needs ``wtable=None`` and no
     sigmoid, and ignores edge values.  ``kind="local_path"``: the Local Path index (``two_hop_local_path``; the count is
     c2)."""
     if kind == LOCAL_PATH:
-        if wtable is not None or sigmoid or counts is not None:
-            raise EpsError("two_hop_scored: the local_path score takes no weight table, no sigmoid and no `counts` "
-                           "(one-pass only)")
+        if wtable is not None or sigmoid:
+            raise EpsError("two_hop_scored: the local_path score takes no weight table and no sigmoid")
         e, s, c2, _, off = two_hop_local_path(adj, v_lo, v_hi, cap, upper, want_offsets=True)
         out = (e, s, c2) if want_count else (e, s)
         return out + (off,) if want_offsets else out
@@ -261,34 +248,12 @@ def two_hop_scored(adj: SparseAdj, wtable: torch.Tensor | None = None, v_lo: int
         use_values = False
     val = adj.val if use_values else None
     check_fixed_point_range(adj, wtable, use_values)
-    if val is not None and (counts is not None or not values_symmetric(adj)):
-        raise EpsError("two_hop_scored: a weighted adjacency takes the one-pass kernel (no `counts`) and needs "
-                       "bitwise symmetric values; otherwise score with two_hop + ops.cn_aa")
-    if upper and counts is not None:
-        raise EpsError("two_hop_scored: the upper-triangle mode is one-pass only (no `counts`)")
-    lib = _lib.load()
+    if val is not None and not values_symmetric(adj):
+        raise EpsError("two_hop_scored: a weighted adjacency needs bitwise symmetric values; otherwise score with "
+                       "two_hop + ops.cn_aa")
     v_hi = adj.n if v_hi is None else v_hi
-    if counts is None:
-        edges, score, count, offsets = _onepass(adj, wtable, v_lo, v_hi, None, sigmoid, True, want_count, cap, val,
-                                                upper, kind_flags)
-        out = (edges, score, count) if want_count else (edges, score)
-        return out + (offsets,) if want_offsets else out
-    offsets = torch.zeros(counts.numel() + 1, dtype=torch.int64, device=adj.device)
-    torch.cumsum(counts, 0, out=offsets[1:])
-    N = int(offsets[-1].item())
-    if N >= 2**31:
-        raise EpsError(f"{N} candidates in one slab; split the owner range (see filter_step.iter_slabs)")
-    edges = torch.empty((2, N), dtype=torch.int32, device=adj.device)
-    score = torch.empty(N, dtype=torch.float32, device=adj.device)
-    count = torch.empty(N, dtype=torch.int32, device=adj.device) if want_count else None
-    if N:
-        wt = None if wtable is None else wtable.contiguous().float()
-        ws = _ws(lib.eps_twohop_scored_workspace_bytes(N), adj.device)
-        check(lib.eps_twohop_scored(_ptr(adj.rowptr), _ptr(adj.col), _ptr(wt), adj.n, v_lo, v_hi, _ptr(offsets), N,
-                                    (EPS_CN_SIGMOID if sigmoid else 0) | kind_flags, _ptr(edges[0]), _ptr(edges[1]), _ptr(score),
-                                    _ptr(count), _ptr(ws), ws.numel(), _stream()), "eps_twohop_scored")
-        from . import ops as _ops
-        _ops.LAUNCHES["n"] += 2
+    edges, score, count, offsets = _onepass(adj, wtable, v_lo, v_hi, None, sigmoid, True, want_count, cap, val,
+                                            upper, kind_flags)
     out = (edges, score, count) if want_count else (edges, score)
     return out + (offsets,) if want_offsets else out
 
@@ -393,11 +358,7 @@ def two_hop_local_path(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, c
         out = (torch.empty((2, 0), dtype=torch.int32, device=dev), torch.empty(0, dtype=torch.float32, device=dev), i0, i0)
         return out + (z,) if want_offsets else out
     tri = arc_triangles(adj)
-    boff = torch.zeros(n_own + 1, dtype=torch.int64, device=dev)
-    torch.cumsum(owner_bounds(adj, upper)[v_lo:v_hi], 0, out=boff[1:])
-    cap = int(boff[-1].item()) if cap is None else int(cap)
-    if cap >= 2**31:
-        raise EpsError(f"up to {cap} candidates in one slab; split the owner range (see filter_step.iter_slabs)")
+    boff, cap = _slot_offsets(owner_bounds(adj, upper)[v_lo:v_hi], cap)
     if "max_bound" not in adj._cache:
         adj._cache["max_bound"] = int(owner_bounds(adj).max().item()) if adj.n else 0
     max_count, ctas = adj._cache["max_bound"], _lp_ctas(dev)
@@ -413,8 +374,6 @@ def two_hop_local_path(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, c
           "eps_local_path_onepass")
     from . import ops as _ops
     _ops.LAUNCHES["n"] += 6
-    N = int(offsets[-1].item())
-    if N > cap:
-        raise EpsError(f"eps_local_path_onepass: an owner's candidates exceed the caller's bound (N={N}, cap={cap})")
+    N = _compact_size(offsets, cap, "eps_local_path_onepass")
     out = (buf[:, :N], score[:N], c2[:N], c3[:N])
     return out + (offsets,) if want_offsets else out

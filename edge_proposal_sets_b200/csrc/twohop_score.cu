@@ -11,36 +11,29 @@
 // its candidates one by one (K3) costs  sum_{u in cand(v)} deg(u)  — ~100x more on the ogbl-ppa
 // shape (mean CN ~ 1.4, mean degree of a candidate ~ 150).
 //
-// One CTA per owner v (handed out dynamically), everything in shared memory but the outputs:
+// One CTA per owner v (handed out dynamically, heaviest first), everything in shared memory but the outputs:
 //   1. mark     bitmap of U = union of N(k), k in N(v)              (flattened coalesced walk)
 //   2. clear    N(v) and v                                           (filter.py:100,103)
 //   3. rank     per-word exclusive popcount prefix (u16 inside a 32-word block + u32 per block),
-//               and emission of pair_u / pair_v in ascending u — the reference's column-major order
+//               and emission of pair_u in ascending u — the reference's column-major order
 //   4. score    second walk over the same 2-paths: a set bit u -> rank(u) -> one RED.ADD into the
-//               compact accumulator of that candidate (count as int32, weight as 64-bit fixed point,
+//               accumulator of that candidate (count as int32, weight as 64-bit fixed point,
 //               eps_common.cuh) — integer atomics, hence exact and order-independent
 //   5. cleanup  zero the touched bitmap words
-// A tiny element-wise pass then turns the fixed-point sums into fp32 scores (+ sigmoid), or the exact counts and the
-// degrees of both ends (two rowptr loads each) into a similarity score (EPS_SCORE_*, after the count-only walk).
-// Results are bit-identical to eps_cn_aa on the same pairs.
-//
-// Where an owner's output starts:
-//   * two-pass (eps_twohop_scored): from the caller's prefix sum of a separate count pass
-//     (eps_twohop_candidates) — the count pass repeats step 1 for every owner;
-//   * ONE-PASS (eps_twohop_onepass): every owner writes into a PADDED slot whose offset is the prefix sum
-//     of a cheap per-owner upper bound (min(#2-paths, n-1-deg), host-side torch ops), and records its
-//     real count; a single-block scan turns the counts into compact offsets and the finalize pass —
-//     which has to read every accumulator anyway — moves (u, score, count) to the compact position and
-//     regenerates v from the owner id.  No count pass, no inter-CTA dependency.
-// Upper-triangle mode (EPS_TWOHOP_UPPER, one-pass only): only the candidates u > v of owner v.  The candidate relation
-// of a symmetric adjacency is symmetric, so this is every unordered pair once; both walks start each N(k) at its lower
-// bound of v + 1 and the rank / emission / cleanup passes start at the bitmap block that holds v + 1.
+// No count pass: every owner writes into a PADDED slot whose offset is the prefix sum of a cheap per-owner upper bound
+// (min(#2-paths, n-1-deg), host-side torch ops) and records its real count; a single-block scan turns the counts into
+// compact offsets, and the compaction pass — which has to read every accumulator anyway — moves (u, score, count) to the
+// compact position, regenerates v from the owner id, and turns the fixed-point sums into fp32 scores (+ sigmoid), or the
+// exact counts and the degrees of both ends (two rowptr loads each) into a similarity score (EPS_SCORE_*, after the
+// count-only walk).  No inter-CTA dependency.  Results are bit-identical to eps_cn_aa on the same pairs.
+// Upper-triangle mode (EPS_TWOHOP_UPPER): only the candidates u > v of owner v.  The candidate relation of a symmetric
+// adjacency is symmetric, so this is every unordered pair once; both walks start each N(k) at its lower bound of v + 1
+// and the rank / emission / cleanup passes start at the bitmap block that holds v + 1.
 #include "eps_common.cuh"
 
 namespace eps {
 
-constexpr int TS_THREADS = 512;           // two-pass entry point
-constexpr int TS_DEFAULT_THREADS = 512;   // one-pass entry point (see eps_twohop_onepass)
+constexpr int TS_THREADS = 512;   // measured against 1,024 (DESIGN.md, K6+K3 walk groups)
 constexpr int TS_LONG = 96;   // lists at least this long are streamed warp-wide without a search
 constexpr int TS_DEPTH = 8;   // ... with this many loads in flight per lane (a hub owner's walk is one CTA's latency chain)
 
@@ -181,14 +174,76 @@ struct ScoreVisitor {
   }
 };
 
-template <bool HAS_W, bool WANT_CN, bool ONEPASS, bool HAS_VAL = false, int THREADS = TS_THREADS>
-__global__ void __launch_bounds__(THREADS)
+// Rank pass over the bitmap blocks g0 .. W2 - 1, thread t owning block c + t (32 bitmap words): pre[w] = #candidates
+// before word w inside its block (u16), blk[g] = #candidates in the blocks g0 .. g - 1 (u32).  *s_carry is zero on
+// entry.  Returns the total, behind a barrier.
+template <int THREADS>
+__device__ __forceinline__ uint32_t rank_blocks(const uint32_t *bm, const uint32_t *bm2, uint32_t *blk, uint16_t *pre,
+                                                int g0, int W2, uint32_t *s_scan, uint32_t *s_carry) {
+  const int tid = threadIdx.x, lane = lane_id(), warp = tid >> 5;
+  constexpr int NW = THREADS / 32;
+  for (int c = g0; c < W2; c += THREADS) {
+    const int g = c + tid;
+    const uint32_t m2 = (g < W2) ? bm2[g] : 0u;
+    uint32_t cnt = 0;
+    {
+      uint32_t m = m2;
+      while (m) {
+        const int b = __ffs(m) - 1;
+        m &= m - 1;
+        const int w = g * 32 + b;
+        pre[w] = (uint16_t)cnt;
+        cnt += __popc(bm[w]);
+      }
+    }
+    uint32_t inc = cnt;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      uint32_t t = __shfl_up_sync(FULL, inc, d);
+      if (lane >= d) inc += t;
+    }
+    if (lane == 31) s_scan[warp] = inc;
+    __syncthreads();
+    uint32_t wbase = 0, tot = 0;
+#pragma unroll
+    for (int w = 0; w < NW; ++w) {
+      const uint32_t x = s_scan[w];
+      if (w < warp) wbase += x;
+      tot += x;
+    }
+    const uint32_t carry = *s_carry;
+    if (g < W2) blk[g] = carry + wbase + (inc - cnt);
+    __syncthreads();
+    if (tid == 0) *s_carry = carry + tot;
+  }
+  __syncthreads();
+  return *s_carry;
+}
+
+// Zero the bitmap words that bm2 marks in the blocks g0 .. W2 - 1, and those bm2 blocks.
+template <int THREADS>
+__device__ __forceinline__ void clear_blocks(uint32_t *bm, uint32_t *bm2, int g0, int W2) {
+  for (int g = g0 + threadIdx.x; g < W2; g += THREADS) {
+    uint32_t m = bm2[g];
+    while (m) {
+      const int b = __ffs(m) - 1;
+      m &= m - 1;
+      bm[g * 32 + b] = 0;
+    }
+    bm2[g] = 0;
+  }
+}
+
+// n_order and upper sit before acc: the parameter offsets decide which constant loads ptxas merges, and this order keeps
+// the instruction sequence the kernel was measured with.
+template <bool HAS_W, bool WANT_CN, bool HAS_VAL>
+__global__ void __launch_bounds__(TS_THREADS)
 twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col, const float *__restrict__ val,
                     const float *__restrict__ wtable, int n, int v_lo, int v_hi,
-                    const long long *__restrict__ offsets, int *__restrict__ pair_u,
-                    int *__restrict__ pair_v, unsigned long long *__restrict__ acc, int *__restrict__ cn,
+                    const long long *__restrict__ offsets, int *__restrict__ pair_u, int n_order, int upper,
+                    unsigned long long *__restrict__ acc, int *__restrict__ cn,
                     unsigned int *owner_counter, unsigned int *__restrict__ counts_out,
-                    const int *__restrict__ owner_order, int n_order, int upper) {
+                    const int *__restrict__ owner_order) {
   extern __shared__ uint32_t sm[];
   const int W = (n + 31) >> 5;       // bitmap words
   const int W2 = (W + 31) >> 5;      // blocks of 32 words
@@ -198,17 +253,17 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
   uint16_t *pre = reinterpret_cast<uint16_t *>(blk + W2);   // #candidates before word w inside its block
   __shared__ int s_owner;
   __shared__ int s_walk;             // next list group of the current walk
-  __shared__ uint32_t s_scan[THREADS / 32];
+  __shared__ uint32_t s_scan[TS_THREADS / 32];
   __shared__ uint32_t s_carry;
-  const int tid = threadIdx.x, lane = lane_id(), warp = tid >> 5;
-  constexpr int NW = THREADS / 32;
-  for (int w = tid; w < W + W2; w += THREADS) sm[w] = 0;
+  const int tid = threadIdx.x, lane = lane_id();
+  constexpr int NW = TS_THREADS / 32;
+  for (int w = tid; w < W + W2; w += TS_THREADS) sm[w] = 0;
   for (;;) {
     __syncthreads();
     if (tid == 0) {
-      // owners are handed out HEAVIEST FIRST when the caller supplies an order (one-pass entry point): a hub owner
-      // costs ~40 average owners, and drawn late by one CTA it kept the other 295 waiting — SMs were busy 48 % of the
-      // kernel's duration (profiles/round2_e_twohop.md)
+      // owners are handed out HEAVIEST FIRST when the caller supplies an order: a hub owner costs ~40 average owners,
+      // and drawn late by one CTA it kept the other 295 waiting — SMs were busy 48 % of the kernel's duration
+      // (profiles/round2_e_twohop.md)
       const int t = (int)atomicAdd(owner_counter, 1u);
       s_owner = (owner_order && t < n_order) ? v_lo + owner_order[t] : v_lo + t;
       s_walk = 0;
@@ -229,69 +284,24 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
     walk_two_paths(rowptr, col, vs, ve, lane, LG, &s_walk, umin, MarkVisitor{bm, bm2});
     __syncthreads();
     // ---- 2. clear known edges and the diagonal ----
-    for (int p = vs + tid; p < ve; p += THREADS) {
+    for (int p = vs + tid; p < ve; p += TS_THREADS) {
       const int k = __ldg(col + p);
       if (k >= umin) atomicAnd(&bm[k >> 5], ~(1u << (k & 31)));
     }
     if (tid == 0 && v >= umin) atomicAnd(&bm[v >> 5], ~(1u << (v & 31)));
     if (tid == 0) { s_carry = 0; s_walk = 0; }        // the first walk is over (barrier above): reset for the second
     __syncthreads();
-    // ---- 3a. rank: thread t owns block c + t (32 bitmap words) ----
-    for (int c = g0; c < W2; c += THREADS) {
-      const int g = c + tid;
-      const uint32_t m2 = (g < W2) ? bm2[g] : 0u;
-      uint32_t cnt = 0;
-      {
-        uint32_t m = m2;
-        while (m) {
-          const int b = __ffs(m) - 1;
-          m &= m - 1;
-          const int w = g * 32 + b;
-          pre[w] = (uint16_t)cnt;
-          cnt += __popc(bm[w]);
-        }
-      }
-      uint32_t inc = cnt;
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        uint32_t t = __shfl_up_sync(FULL, inc, d);
-        if (lane >= d) inc += t;
-      }
-      if (lane == 31) s_scan[warp] = inc;
-      __syncthreads();
-      uint32_t wbase = 0, tot = 0;
-#pragma unroll
-      for (int w = 0; w < NW; ++w) {
-        const uint32_t x = s_scan[w];
-        if (w < warp) wbase += x;
-        tot += x;
-      }
-      const uint32_t carry = s_carry;
-      if (g < W2) blk[g] = carry + wbase + (inc - cnt);
-      __syncthreads();
-      if (tid == 0) s_carry = carry + tot;
+    // ---- 3a. rank ----
+    const uint32_t total = rank_blocks<TS_THREADS>(bm, bm2, blk, pre, g0, W2, s_scan, &s_carry);
+    const bool fits = (long long)total <= offsets[v - v_lo + 1] - out_base;
+    // padded slot: record the real count (a violated bound poisons N instead of overrunning the slot)
+    if (tid == 0) counts_out[v - v_lo] = fits ? total : 0xffffffffu;
+    if (!fits) {
+      clear_blocks<TS_THREADS>(bm, bm2, g0, W2);
+      continue;
     }
-    __syncthreads();
-    if (ONEPASS) {
-      const uint32_t total = s_carry;
-      const bool fits = (long long)total <= offsets[v - v_lo + 1] - out_base;
-      // padded slot: record the real count (a violated bound poisons N instead of overrunning the slot)
-      if (tid == 0) counts_out[v - v_lo] = fits ? total : 0xffffffffu;
-      if (!fits) {
-        for (int g = g0 + tid; g < W2; g += THREADS) {
-          uint32_t m = bm2[g];
-          while (m) {
-            const int b = __ffs(m) - 1;
-            m &= m - 1;
-            bm[g * 32 + b] = 0;
-          }
-          bm2[g] = 0;
-        }
-        continue;
-      }
-    }
-    // ---- 3b. emit pair_u / pair_v in ascending u ----
-    for (int g = g0 + tid; g < W2; g += THREADS) {
+    // ---- 3b. emit pair_u in ascending u (v is regenerated by the compaction) ----
+    for (int g = g0 + tid; g < W2; g += TS_THREADS) {
       uint32_t m = bm2[g];
       long long o = out_base + blk[g];
       while (m) {
@@ -303,7 +313,6 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
           const int q = __ffs(bits) - 1;
           bits &= bits - 1;
           pair_u[o] = (w << 5) + q;
-          if (!ONEPASS) pair_v[o] = v;                 // one-pass: v is regenerated by the compaction
           ++o;
         }
       }
@@ -316,8 +325,8 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
       walk_two_paths(rowptr, col, vs, ve, lane, LG, &s_walk, umin, sv);
     }
     __syncthreads();
-    // ---- 5. cleanup ----
-    for (int c = g0; c < W2; c += THREADS) {
+    // ---- 5. cleanup: a block-uniform loop, not clear_blocks, which changes this kernel's instruction sequence ----
+    for (int c = g0; c < W2; c += TS_THREADS) {
       const int g = c + tid;
       if (g < W2) {
         uint32_t m = bm2[g];
@@ -329,25 +338,6 @@ twohop_score_kernel(const int *__restrict__ rowptr, const int *__restrict__ col,
         bm2[g] = 0;
       }
     }
-  }
-}
-
-template <int KIND>
-__global__ void __launch_bounds__(256)
-twohop_finalize_kernel(const int *__restrict__ rowptr, const int *__restrict__ pair_u, const int *__restrict__ pair_v,
-                       const unsigned long long *__restrict__ acc, const int *__restrict__ cn,
-                       long long N, int flags, float *__restrict__ score) {
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += stride) {
-    float sc;
-    if (KIND) {
-      const int u = pair_u[i], v = pair_v[i];
-      sc = similarity_score<KIND>(cn[i], __ldg(rowptr + u + 1) - __ldg(rowptr + u), __ldg(rowptr + v + 1) - __ldg(rowptr + v));
-    } else {
-      sc = acc ? from_fixed(acc[i]) : (float)cn[i];
-      if (flags & EPS_CN_SIGMOID) sc = sigmoidf_ref(sc);
-    }
-    score[i] = sc;
   }
 }
 
@@ -409,6 +399,34 @@ owner_scan_kernel(const unsigned int *__restrict__ counts, int n_own, long long 
 // compact offsets of the (few) owners the tile touches.
 constexpr int CP_THREADS = 256, CP_PER = 8, CP_TILE = CP_THREADS * CP_PER;
 
+// The owner of compact position x < end: lo becomes the largest o in [lo, hi) with cmp_off[o] <= x (invariant:
+// cmp_off[lo] <= x < cmp_off[hi]).  For x >= end, lo is left as it is.
+__device__ __forceinline__ void owner_search(const long long *cmp_off, int &lo, int hi, long long x, long long end) {
+  if (x < end) {
+    while (hi - lo > 1) {
+      const int mid = (lo + hi) >> 1;
+      if (cmp_off[mid] <= x) lo = mid; else hi = mid;
+    }
+  }
+}
+
+// the owners of the first and last positions of the tile [base, end), for the whole block (a search of its own:
+// owner_search's bound test changes the compaction kernels' instructions here)
+__device__ __forceinline__ void tile_owners(const long long *__restrict__ cmp_off, int n_own, long long base,
+                                            long long end, int *s_lo, int *s_hi) {
+  __syncthreads();
+  if (threadIdx.x < 2) {
+    const long long x = threadIdx.x == 0 ? base : end - 1;
+    int lo = 0, hi = n_own;                       // invariant: cmp_off[lo] <= x < cmp_off[hi]
+    while (hi - lo > 1) {
+      const int mid = (lo + hi) >> 1;
+      if (cmp_off[mid] <= x) lo = mid; else hi = mid;
+    }
+    if (threadIdx.x == 0) *s_lo = lo; else *s_hi = lo;
+  }
+  __syncthreads();
+}
+
 template <int KIND>
 __global__ void __launch_bounds__(CP_THREADS)
 twohop_compact_kernel(const int *__restrict__ rowptr, const long long *__restrict__ pad_off,
@@ -422,31 +440,15 @@ twohop_compact_kernel(const int *__restrict__ rowptr, const long long *__restric
   const long long ntiles = (N + CP_TILE - 1) / CP_TILE;
   for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     const long long base = tile * CP_TILE, end = min(base + (long long)CP_TILE, N);
-    __syncthreads();
-    if (threadIdx.x < 2) {
-      // largest o with cmp_off[o] <= x  (x = first / last position of the tile)
-      const long long x = threadIdx.x == 0 ? base : end - 1;
-      int lo = 0, hi = n_own;                       // invariant: cmp_off[lo] <= x < cmp_off[hi]
-      while (hi - lo > 1) {
-        const int mid = (lo + hi) >> 1;
-        if (cmp_off[mid] <= x) lo = mid; else hi = mid;
-      }
-      if (threadIdx.x == 0) s_lo = lo; else s_hi = lo;
-    }
-    __syncthreads();
+    tile_owners(cmp_off, n_own, base, end, &s_lo, &s_hi);
     const int o_lo = s_lo, o_hi = s_hi;
     long long src[CP_PER];
     int own[CP_PER];
 #pragma unroll
     for (int q = 0; q < CP_PER; ++q) {
       const long long i = base + q * CP_THREADS + threadIdx.x;
-      int lo = o_lo, hi = o_hi + 1;
-      if (i < end) {
-        while (hi - lo > 1) {
-          const int mid = (lo + hi) >> 1;
-          if (cmp_off[mid] <= i) lo = mid; else hi = mid;
-        }
-      }
+      int lo = o_lo;
+      owner_search(cmp_off, lo, o_hi + 1, i, end);
       own[q] = lo;
       src[q] = i < end ? pad_off[lo] + (i - cmp_off[lo]) : -1;
     }
@@ -494,14 +496,9 @@ twohop_compact_kernel(const int *__restrict__ rowptr, const long long *__restric
   }
 }
 
-using FinalizeKernel = void (*)(const int *, const int *, const int *, const unsigned long long *, const int *, long long,
-                                int, float *);
 using CompactKernel = void (*)(const int *, const long long *, const long long *, int, int, long long, const int *,
                                const unsigned long long *, const int *, int, int *, int *, float *, int *);
 // index = score_kind(flags): 0 = CN / AA / RA, 1..7 = the similarity kinds
-static const FinalizeKernel kFinalizeKinds[8] = {
-    twohop_finalize_kernel<0>, twohop_finalize_kernel<1>, twohop_finalize_kernel<2>, twohop_finalize_kernel<3>,
-    twohop_finalize_kernel<4>, twohop_finalize_kernel<5>, twohop_finalize_kernel<6>, twohop_finalize_kernel<7>};
 static const CompactKernel kCompactKinds[8] = {
     twohop_compact_kernel<0>, twohop_compact_kernel<1>, twohop_compact_kernel<2>, twohop_compact_kernel<3>,
     twohop_compact_kernel<4>, twohop_compact_kernel<5>, twohop_compact_kernel<6>, twohop_compact_kernel<7>};
@@ -649,7 +646,7 @@ local_path_onepass_kernel(const int *__restrict__ rowptr, const int *__restrict_
   __shared__ int s_owner, s_walk, s_walk3;
   __shared__ uint32_t s_scan[LP_THREADS / 32];
   __shared__ uint32_t s_carry, s_lo;
-  const int tid = threadIdx.x, lane = lane_id(), warp = tid >> 5;
+  const int tid = threadIdx.x, lane = lane_id();
   constexpr int NW = LP_THREADS / 32;
   int *c2s = scratch + (long long)blockIdx.x * scratch_cap;
   for (int w = tid; w < W + W2; w += LP_THREADS) sm[w] = 0;
@@ -680,38 +677,8 @@ local_path_onepass_kernel(const int *__restrict__ rowptr, const int *__restrict_
     }
     if (tid == 0) { atomicAnd(&bm[v >> 5], ~(1u << (v & 31))); s_carry = 0; s_walk = 0; }
     __syncthreads();
-    // ---- rank (as twohop_score_kernel, from block 0) ----
-    for (int c = 0; c < W2; c += LP_THREADS) {
-      const int g = c + tid;
-      const uint32_t m2 = (g < W2) ? bm2[g] : 0u;
-      uint32_t cnt = 0;
-      for (uint32_t m = m2; m; m &= m - 1) {
-        const int w = g * 32 + __ffs(m) - 1;
-        pre[w] = (uint16_t)cnt;
-        cnt += __popc(bm[w]);
-      }
-      uint32_t inc = cnt;
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        const uint32_t t = __shfl_up_sync(FULL, inc, d);
-        if (lane >= d) inc += t;
-      }
-      if (lane == 31) s_scan[warp] = inc;
-      __syncthreads();
-      uint32_t wbase = 0, tot = 0;
-#pragma unroll
-      for (int w = 0; w < NW; ++w) {
-        const uint32_t x = s_scan[w];
-        if (w < warp) wbase += x;
-        tot += x;
-      }
-      const uint32_t carry = s_carry;
-      if (g < W2) blk[g] = carry + wbase + (inc - cnt);
-      __syncthreads();
-      if (tid == 0) s_carry = carry + tot;
-    }
-    __syncthreads();
-    const uint32_t total = s_carry;
+    // ---- rank, from block 0 (walk 3 looks up candidates below umin too) ----
+    const uint32_t total = rank_blocks<LP_THREADS>(bm, bm2, blk, pre, 0, W2, s_scan, &s_carry);
     if (tid == 0) {                                    // lo = #candidates below umin
       uint32_t r = total;
       const int w0 = umin >> 5;
@@ -764,10 +731,7 @@ local_path_onepass_kernel(const int *__restrict__ rowptr, const int *__restrict_
       __syncthreads();
     }
     // ---- cleanup ----
-    for (int g = tid; g < W2; g += LP_THREADS) {
-      for (uint32_t m = bm2[g]; m; m &= m - 1) bm[g * 32 + __ffs(m) - 1] = 0;
-      bm2[g] = 0;
-    }
+    clear_blocks<LP_THREADS>(bm, bm2, 0, W2);
   }
 }
 
@@ -783,25 +747,12 @@ local_path_compact_kernel(const long long *__restrict__ pad_off, const long long
   const long long ntiles = (N + CP_TILE - 1) / CP_TILE;
   for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     const long long base = tile * CP_TILE, end = min(base + (long long)CP_TILE, N);
-    __syncthreads();
-    if (threadIdx.x < 2) {
-      const long long x = threadIdx.x == 0 ? base : end - 1;
-      int lo = 0, hi = n_own;
-      while (hi - lo > 1) {
-        const int mid = (lo + hi) >> 1;
-        if (cmp_off[mid] <= x) lo = mid; else hi = mid;
-      }
-      if (threadIdx.x == 0) s_lo = lo; else s_hi = lo;
-    }
-    __syncthreads();
+    tile_owners(cmp_off, n_own, base, end, &s_lo, &s_hi);
     for (int q = 0; q < CP_PER; ++q) {
       const long long i = base + q * CP_THREADS + threadIdx.x;
       if (i >= end) break;
-      int lo = s_lo, hi = s_hi + 1;
-      while (hi - lo > 1) {
-        const int mid = (lo + hi) >> 1;
-        if (cmp_off[mid] <= i) lo = mid; else hi = mid;
-      }
+      int lo = s_lo;
+      owner_search(cmp_off, lo, s_hi + 1, i, end);
       const long long src = pad_off[lo] + (i - cmp_off[lo]);
       const int c2 = pad_c2[src], c3 = pad_c3[src];
       pair_u[i] = pad_u[src];
@@ -908,79 +859,82 @@ extern "C" int eps_score_kinds(void) {
          (1 << eps::score_kind(EPS_SCORE_PREF_ATTACH));
 }
 
-extern "C" size_t eps_twohop_scored_workspace_bytes(int64_t N) {
-  return 256 + (size_t)(N > 0 ? N : 0) * 8;
-}
+// ---------------------------------------------------------------------------------------------
+// Host plan of the one-pass entry points (eps_twohop_onepass, eps_local_path_onepass).  Workspace:
+//   ticket (256 B) | 64 work buckets (256 B) | per-owner counts | owner order | the entry point's padded slots ...
+// ---------------------------------------------------------------------------------------------
+static inline size_t up256(size_t x) { return (x + 255) & ~(size_t)255; }
+static inline size_t onepass_header_bytes(size_t n_own) { return 512 + 2 * up256(n_own * 4); }
 
-extern "C" int eps_twohop_scored(const int32_t *rowptr, const int32_t *col, const float *wtable,
-                                 int32_t n, int32_t v_lo, int32_t v_hi, const int64_t *offsets,
-                                 int64_t N, int flags, int32_t *pair_u, int32_t *pair_v, float *score,
-                                 int32_t *count, void *workspace, size_t workspace_bytes,
-                                 void *stream_) {
-  using namespace eps;
-  cudaStream_t stream = (cudaStream_t)stream_;
-  EPS_CHECK_ARG(rowptr && col && offsets, "null graph or offsets pointer");
-  EPS_CHECK_ARG(n > 0 && v_lo >= 0 && v_hi <= n && v_lo <= v_hi && N >= 0, "bad owner range or N");
-  EPS_CHECK_ARG(!(flags & EPS_TWOHOP_UPPER), "EPS_TWOHOP_UPPER needs the one-pass entry point (eps_twohop_onepass)");
-  EPS_CHECK_ARG(!(flags & ~(EPS_CN_SIGMOID | EPS_SCORE_KIND_MASK)), "unknown flag bits");
-  const int kind = score_kind(flags);
-  EPS_CHECK_ARG(!kind || (!wtable && !(flags & EPS_CN_SIGMOID)),
-                "a similarity kind (EPS_SCORE_*) needs wtable == NULL and no EPS_CN_SIGMOID");
-  if (v_lo == v_hi || N == 0) return EPS_OK;
-  EPS_CHECK_ARG(pair_u && pair_v && (score || count), "missing output pointer");
-  const int sms = sm_count();
-  if (sms <= 0) { set_error("eps_twohop_scored: no CUDA device"); return EPS_ERR_CUDA; }
-  if (!workspace || workspace_bytes < eps_twohop_scored_workspace_bytes(N)) {
-    set_error("eps_twohop_scored: workspace too small");
-    return EPS_ERR_WORKSPACE;
-  }
+namespace eps {
+
+struct OnepassPlan {
+  size_t smem;                  // one owner's bitmap and rank tables
+  unsigned int *ticket, *buckets, *counts;
+  int *order;
+  uint8_t *slots;               // the padded slots behind the header
+  int cgrid;                    // grid of the compaction pass
+};
+
+// The owner bitmap's shared memory (<= 200 KB) and the workspace header; zeroes the ticket, buckets and counts.
+static int onepass_begin(const char *what, int n, int n_own, void *workspace, cudaStream_t stream, OnepassPlan &p) {
   const int W = (n + 31) / 32, W2 = (W + 31) / 32;
-  const size_t smem = (size_t)(W + 2 * W2) * 4 + (size_t)W * 2 + 16;
-  if (smem > 200 * 1024) {
-    set_error("eps_twohop_scored: n=%d needs %zu bytes of shared memory (> 200 KB)", n, smem);
+  p.smem = (size_t)(W + 2 * W2) * 4 + (size_t)W * 2 + 16;
+  if (p.smem > 200 * 1024) {
+    set_error("%s: n=%d needs %zu bytes of shared memory (> 200 KB)", what, n, p.smem);
     return EPS_ERR_UNSUPPORTED;
   }
-  unsigned long long *acc = nullptr;
-  int *cn = count;
   uint8_t *ws = (uint8_t *)workspace;
-  EPS_CUDA(cudaMemsetAsync(ws, 0, 4, stream));
-  if (wtable) {
-    acc = (unsigned long long *)(ws + 256);
-    EPS_CUDA(cudaMemsetAsync(acc, 0, (size_t)N * 8, stream));
-  } else if (!cn) {
-    cn = (int *)(ws + 256);          // CN scores only: count lives in the workspace
-  }
-  if (cn) EPS_CUDA(cudaMemsetAsync(cn, 0, (size_t)N * 4, stream));
-  void (*kern)(const int *, const int *, const float *, const float *, int, int, int, const long long *, int *,
-               int *, unsigned long long *, int *, unsigned int *, unsigned int *, const int *, int, int);
-  if (wtable) kern = cn ? twohop_score_kernel<true, true, false> : twohop_score_kernel<true, false, false>;
-  else kern = twohop_score_kernel<false, true, false>;
-  EPS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int occ = 0;
-  EPS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, TS_THREADS, smem));
-  if (occ < 1) occ = 1;
-  const int grid = (int)std::min<long long>((long long)(v_hi - v_lo), (long long)sms * occ);
-  kern<<<grid, TS_THREADS, smem, stream>>>(rowptr, col, nullptr, wtable, n, v_lo, v_hi,
-                                           (const long long *)offsets, pair_u, pair_v, acc, cn,
-                                           (unsigned int *)ws, nullptr, nullptr, 0, 0);
-  EPS_LAUNCH_CHECK();
-  if (score) {
-    const int fgrid = (int)std::min<long long>((N + 255) / 256, (long long)sms * 8);
-    kFinalizeKinds[kind]<<<fgrid, 256, 0, stream>>>(rowptr, pair_u, pair_v, acc, cn, (long long)N, flags, score);
-    EPS_LAUNCH_CHECK();
-  }
+  p.ticket = (unsigned int *)ws;
+  p.buckets = (unsigned int *)(ws + 256);
+  p.counts = (unsigned int *)(ws + 512);
+  p.order = (int *)(ws + 512 + up256((size_t)n_own * 4));
+  p.slots = ws + onepass_header_bytes(n_own);
+  EPS_CUDA(cudaMemsetAsync(ws, 0, 512 + up256((size_t)n_own * 4), stream));   // ticket + buckets + counts
   return EPS_OK;
 }
 
-// ---------------------------------------------------------------------------------------------
-// one-pass entry: enumerate (+ score) the owner range without a count pass
-// ---------------------------------------------------------------------------------------------
-static inline size_t up256(size_t x) { return (x + 255) & ~(size_t)255; }
+// Heaviest-first owner order, the owner kernel on as many CTAs as fit (at most max_ctas), the scan of the real counts
+// into offsets_out; sets the compaction grid.
+template <typename... P, typename... A>
+static int onepass_run(OnepassPlan &p, void (*kern)(P...), int threads, long long max_ctas, int n_own,
+                       const int64_t *bound_offsets, int64_t cap, int64_t *offsets_out, int sms, cudaStream_t stream,
+                       A... args) {
+  EPS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
+  int occ = 0;
+  EPS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, p.smem));
+  if (occ < 1) occ = 1;
+  const int grid = (int)std::min<long long>(std::min<long long>((long long)n_own, (long long)sms * occ), max_ctas);
+  {  // heaviest-first hand-out: counting sort of the owners by the power of two of their slot size (the bound)
+    const int ogrid = std::min((n_own + 255) / 256, sms * 8);
+    owner_bucket_kernel<0><<<ogrid, 256, 0, stream>>>((const long long *)bound_offsets, n_own, p.buckets, p.order);
+    owner_bucket_kernel<1><<<1, 64, 0, stream>>>((const long long *)bound_offsets, n_own, p.buckets, p.order);
+    owner_bucket_kernel<2><<<ogrid, 256, 0, stream>>>((const long long *)bound_offsets, n_own, p.buckets, p.order);
+    EPS_LAUNCH_CHECK();
+  }
+  kern<<<grid, threads, p.smem, stream>>>(args...);
+  EPS_LAUNCH_CHECK();
+  owner_scan_kernel<<<1, 1024, 0, stream>>>(p.counts, n_own, (long long *)offsets_out);
+  EPS_LAUNCH_CHECK();
+  p.cgrid = (int)std::min<long long>((cap + CP_TILE - 1) / CP_TILE, (long long)sms * 8);
+  return EPS_OK;
+}
+
+using ScoreKernel = void (*)(const int *, const int *, const float *, const float *, int, int, int, const long long *,
+                             int *, int, int, unsigned long long *, int *, unsigned int *, unsigned int *, const int *);
+// index [HAS_W][WANT_CN][HAS_VAL]
+static const ScoreKernel kScoreKernels[2][2][2] = {
+    {{twohop_score_kernel<false, false, false>, twohop_score_kernel<false, false, true>},
+     {twohop_score_kernel<false, true, false>, twohop_score_kernel<false, true, true>}},
+    {{twohop_score_kernel<true, false, false>, twohop_score_kernel<true, false, true>},
+     {twohop_score_kernel<true, true, false>, twohop_score_kernel<true, true, true>}}};
+
+}  // namespace eps
 
 extern "C" size_t eps_twohop_onepass_workspace_bytes(int64_t cap, int32_t n_owners) {
   const size_t c = (size_t)(cap > 0 ? cap : 0), o = (size_t)(n_owners > 0 ? n_owners : 0);
-  // ticket | work buckets | per-owner counts | owner order | padded u | padded CN counts | padded fixed-point sums
-  return 512 + 2 * up256(o * 4) + up256(c * 4) + up256(c * 4) + up256(c * 8);
+  // header | padded u | padded CN counts | padded fixed-point sums
+  return onepass_header_bytes(o) + up256(c * 4) + up256(c * 4) + up256(c * 8);
 }
 
 extern "C" int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, const float *val,
@@ -1006,20 +960,11 @@ extern "C" int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, con
     set_error("eps_twohop_onepass: workspace too small");
     return EPS_ERR_WORKSPACE;
   }
-  const int W = (n + 31) / 32, W2 = (W + 31) / 32;
-  const size_t smem = (size_t)(W + 2 * W2) * 4 + (size_t)W * 2 + 16;
-  if (smem > 200 * 1024) {
-    set_error("eps_twohop_onepass: n=%d needs %zu bytes of shared memory (> 200 KB)", n, smem);
-    return EPS_ERR_UNSUPPORTED;
-  }
-  uint8_t *ws = (uint8_t *)workspace;
-  unsigned int *buckets = (unsigned int *)(ws + 256);
-  unsigned int *counts = (unsigned int *)(ws + 512);
-  int *order = (int *)(ws + 512 + up256((size_t)n_own * 4));
-  int *pad_u = (int *)(ws + 512 + 2 * up256((size_t)n_own * 4));
+  OnepassPlan p;
+  if (const int st = onepass_begin("eps_twohop_onepass", n, n_own, workspace, stream, p)) return st;
+  int *pad_u = (int *)p.slots;
   int *pad_cn = (int *)((uint8_t *)pad_u + up256((size_t)cap * 4));
   unsigned long long *pad_acc = (unsigned long long *)((uint8_t *)pad_cn + up256((size_t)cap * 4));
-  EPS_CUDA(cudaMemsetAsync(ws, 0, 512 + up256((size_t)n_own * 4), stream));   // ticket + buckets + counts
   const bool want_score = score != nullptr || count != nullptr;
   unsigned long long *acc = nullptr;
   int *cn = nullptr;
@@ -1031,48 +976,15 @@ extern "C" int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, con
     cn = pad_cn;
   }
   if (cn) EPS_CUDA(cudaMemsetAsync(cn, 0, (size_t)cap * 4, stream));
-  void (*kern)(const int *, const int *, const float *, const float *, int, int, int, const long long *, int *,
-               int *, unsigned long long *, int *, unsigned int *, unsigned int *, const int *, int, int);
-  // CTA size.  Measured (gpurun_out/r31, fused phase per step): 1024 threads help only where the bitmap limits
-  // the kernel to 2 CTAs per SM (ppa 12.6 -> 11.6 ms) and hurt where 512-thread CTAs already fill the SM
-  // (collab 4.6 -> 7.7 ms; ddi 8.1 -> 8.2): 512 stays the default, EPS_TS_THREADS=1024 overrides (A/B runs)
-  int threads = TS_DEFAULT_THREADS;
-  if (const char *e = getenv("EPS_TS_THREADS")) threads = atoi(e) == 1024 ? 1024 : 512;
-#define EPS_TS_PICK(T)                                                                                                  \
-  do {                                                                                                                  \
-    if (!want_score) kern = twohop_score_kernel<false, false, true, false, T>;                                         \
-    else if (val && wtable) kern = cn ? twohop_score_kernel<true, true, true, true, T> : twohop_score_kernel<true, false, true, true, T>;   \
-    else if (val) kern = cn ? twohop_score_kernel<false, true, true, true, T> : twohop_score_kernel<false, false, true, true, T>;           \
-    else if (wtable) kern = cn ? twohop_score_kernel<true, true, true, false, T> : twohop_score_kernel<true, false, true, false, T>;        \
-    else kern = twohop_score_kernel<false, true, true, false, T>;                                                      \
-  } while (0)
-  if (threads == 1024) EPS_TS_PICK(1024); else EPS_TS_PICK(512);
-#undef EPS_TS_PICK
-  EPS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int occ = 0;
-  EPS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem));
-  if (occ < 1) occ = 1;
-  const int grid = (int)std::min<long long>((long long)n_own, (long long)sms * occ);
-  {  // heaviest-first hand-out: counting sort of the owners by the power of two of their slot size (the bound)
-    const int ogrid = std::min((n_own + 255) / 256, sms * 8);
-    owner_bucket_kernel<0><<<ogrid, 256, 0, stream>>>((const long long *)bound_offsets, n_own, buckets, order);
-    owner_bucket_kernel<1><<<1, 64, 0, stream>>>((const long long *)bound_offsets, n_own, buckets, order);
-    owner_bucket_kernel<2><<<ogrid, 256, 0, stream>>>((const long long *)bound_offsets, n_own, buckets, order);
-    EPS_LAUNCH_CHECK();
-  }
-  kern<<<grid, threads, smem, stream>>>(rowptr, col, val, wtable, n, v_lo, v_hi,
-                                           (const long long *)bound_offsets, pad_u, nullptr, acc, cn,
-                                           (unsigned int *)ws, counts, order, n_own,
-                                           (flags & EPS_TWOHOP_UPPER) ? 1 : 0);
-  EPS_LAUNCH_CHECK();
-  owner_scan_kernel<<<1, 1024, 0, stream>>>(counts, n_own, (long long *)offsets_out);
-  EPS_LAUNCH_CHECK();
+  if (const int st = onepass_run(p, kScoreKernels[wtable != nullptr][cn != nullptr][val != nullptr], TS_THREADS, n_own,
+                                 n_own, bound_offsets, cap, offsets_out, sms, stream, rowptr, col, val, wtable, n, v_lo,
+                                 v_hi, (const long long *)bound_offsets, pad_u, n_own, (flags & EPS_TWOHOP_UPPER) ? 1 : 0,
+                                 acc, cn, p.ticket, p.counts, p.order))
+    return st;
   if (cap > 0) {
-    const int cgrid = (int)std::min<long long>((cap + CP_TILE - 1) / CP_TILE, (long long)sms * 8);
-    kCompactKinds[kind]<<<cgrid, CP_THREADS, 0, stream>>>(rowptr, (const long long *)bound_offsets,
-                                                     (const long long *)offsets_out, v_lo, n_own, (long long)cap,
-                                                     pad_u, acc,
-                                                     cn, flags, pair_u, pair_v, score, count);
+    kCompactKinds[kind]<<<p.cgrid, CP_THREADS, 0, stream>>>(rowptr, (const long long *)bound_offsets,
+                                                           (const long long *)offsets_out, v_lo, n_own, (long long)cap,
+                                                           pad_u, acc, cn, flags, pair_u, pair_v, score, count);
     EPS_LAUNCH_CHECK();
   }
   return EPS_OK;
@@ -1085,8 +997,8 @@ extern "C" size_t eps_local_path_onepass_workspace_bytes(int64_t cap, int32_t n_
                                                          int32_t ctas) {
   const size_t c = (size_t)(cap > 0 ? cap : 0), o = (size_t)(n_owners > 0 ? n_owners : 0);
   const size_t s = (size_t)(max_count > 0 ? max_count : 0) * (size_t)(ctas > 0 ? ctas : 0);
-  // ticket | work buckets | per-owner counts | owner order | padded u | padded c2 | padded c3 | per-CTA c2 scratch
-  return 512 + 2 * up256(o * 4) + 3 * up256(c * 4) + up256(s * 4);
+  // header | padded u | padded c2 | padded c3 | per-CTA c2 scratch
+  return onepass_header_bytes(o) + 3 * up256(c * 4) + up256(s * 4);
 }
 
 extern "C" int eps_local_path_onepass(const int32_t *rowptr, const int32_t *col, const int32_t *tri, int32_t n,
@@ -1110,45 +1022,22 @@ extern "C" int eps_local_path_onepass(const int32_t *rowptr, const int32_t *col,
   }
   const int sms = sm_count();
   if (sms <= 0) { set_error("eps_local_path_onepass: no CUDA device"); return EPS_ERR_CUDA; }
-  const int W = (n + 31) / 32, W2 = (W + 31) / 32;
-  const size_t smem = (size_t)(W + 2 * W2) * 4 + (size_t)W * 2 + 16;
-  if (smem > 200 * 1024) {
-    set_error("eps_local_path_onepass: n=%d needs %zu bytes of shared memory (> 200 KB)", n, smem);
-    return EPS_ERR_UNSUPPORTED;
-  }
-  uint8_t *ws = (uint8_t *)workspace;
-  unsigned int *buckets = (unsigned int *)(ws + 256);
-  unsigned int *counts = (unsigned int *)(ws + 512);
-  int *order = (int *)(ws + 512 + up256((size_t)n_own * 4));
-  int *pad_u = (int *)(ws + 512 + 2 * up256((size_t)n_own * 4));
+  OnepassPlan p;
+  if (const int st = onepass_begin("eps_local_path_onepass", n, n_own, workspace, stream, p)) return st;
+  int *pad_u = (int *)p.slots;
   int *pad_c2 = (int *)((uint8_t *)pad_u + up256((size_t)cap * 4));
   int *pad_c3 = (int *)((uint8_t *)pad_c2 + up256((size_t)cap * 4));
   int *scratch = (int *)((uint8_t *)pad_c3 + up256((size_t)cap * 4));
-  EPS_CUDA(cudaMemsetAsync(ws, 0, 512 + up256((size_t)n_own * 4), stream));   // ticket + buckets + counts
-  EPS_CUDA(cudaFuncSetAttribute(local_path_onepass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int occ = 0;
-  EPS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, local_path_onepass_kernel, LP_THREADS, smem));
-  if (occ < 1) occ = 1;
-  const int grid = (int)std::min<long long>(std::min<long long>((long long)n_own, (long long)sms * occ), ctas);
-  {
-    const int ogrid = std::min((n_own + 255) / 256, sms * 8);
-    owner_bucket_kernel<0><<<ogrid, 256, 0, stream>>>((const long long *)bound_offsets, n_own, buckets, order);
-    owner_bucket_kernel<1><<<1, 64, 0, stream>>>((const long long *)bound_offsets, n_own, buckets, order);
-    owner_bucket_kernel<2><<<ogrid, 256, 0, stream>>>((const long long *)bound_offsets, n_own, buckets, order);
-    EPS_LAUNCH_CHECK();
-  }
-  local_path_onepass_kernel<<<grid, LP_THREADS, smem, stream>>>(
-      rowptr, col, tri, n, v_lo, v_hi, (const long long *)bound_offsets, pad_u, pad_c2, pad_c3, scratch,
-      (long long)max_count, (unsigned int *)ws, counts, order, n_own, (flags & EPS_TWOHOP_UPPER) ? 1 : 0);
-  EPS_LAUNCH_CHECK();
-  owner_scan_kernel<<<1, 1024, 0, stream>>>(counts, n_own, (long long *)offsets_out);
-  EPS_LAUNCH_CHECK();
+  if (const int st = onepass_run(p, local_path_onepass_kernel, LP_THREADS, ctas, n_own, bound_offsets, cap, offsets_out,
+                                 sms, stream, rowptr, col, tri, n, v_lo, v_hi, (const long long *)bound_offsets, pad_u,
+                                 pad_c2, pad_c3, scratch, (long long)max_count, p.ticket, p.counts, p.order, n_own,
+                                 (flags & EPS_TWOHOP_UPPER) ? 1 : 0))
+    return st;
   if (cap > 0) {
-    const int cgrid = (int)std::min<long long>((cap + CP_TILE - 1) / CP_TILE, (long long)sms * 8);
-    local_path_compact_kernel<<<cgrid, CP_THREADS, 0, stream>>>((const long long *)bound_offsets,
-                                                              (const long long *)offsets_out, v_lo, n_own,
-                                                              (long long)cap, pad_u, pad_c2, pad_c3, pair_u, pair_v,
-                                                              score, c2, c3);
+    local_path_compact_kernel<<<p.cgrid, CP_THREADS, 0, stream>>>((const long long *)bound_offsets,
+                                                                (const long long *)offsets_out, v_lo, n_own,
+                                                                (long long)cap, pad_u, pad_c2, pad_c3, pair_u, pair_v,
+                                                                score, c2, c3);
     EPS_LAUNCH_CHECK();
   }
   return EPS_OK;

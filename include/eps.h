@@ -104,7 +104,7 @@ int eps_gcn_norm_fill(const int32_t *rowptr, const int32_t *col, const float *va
  * ------------------------------------------------------------------------- */
 #define EPS_CN_SIGMOID 1
 #define EPS_CN_GROUPED_BY_V 2
-/* Degree-normalised similarity scores (eps_cn_aa, eps_twohop_scored, eps_twohop_onepass): a 3-bit kind field at
+/* Degree-normalised similarity scores (eps_cn_aa, eps_twohop_onepass): a 3-bit kind field at
  * bit 8 of `flags`.  With c = |N(u) & N(v)| (the exact count), a = |N(u)|, b = |N(v)| (stored lists, self loops
  * included, edge values ignored), score =
  *   JACCARD        __fdiv_rn(c, a + b - c)             SORENSEN       __fdiv_rn(2c, a + b)
@@ -295,56 +295,24 @@ int eps_segment_topk_write(const float *score, const int32_t *pair_u, const int3
                            size_t workspace_bytes, void *stream);
 
 /* ---------------------------------------------------------------------------
- * K6  2-hop candidate enumeration for the owner range [v_lo, v_hi)
+ * K6 / K6+K3  2-hop candidates of the owner range [v_lo, v_hi), optionally
+ * TOGETHER WITH their CN / AA / RA scores from one walk over the 2-paths of
+ * each owner, without a count pass.
  * replaces: A2 = adj_t @ adj_t; remove_diag; A2[adj>0] = 0; nonzero
- *           (/root/reference/filter.py:96-109, CPU, single thread).
+ *           (/root/reference/filter.py:96-109, CPU, single thread; the A@A
+ *           values are discarded at :108-109) + the scoring loop
+ *           filter.py:113-142 for the heuristic models (models.py:536-554,
+ *           adamic_utils.py:13-25, train_and_eval.py:195-216).
  * Candidates of owner v (= all_edges[:,1]) are every u != v with a common
  * neighbour and no edge (u,v); they are emitted in ascending u, owners in
  * ascending v: the reference's column-major order, no sort needed.
- *   count pass: offsets == NULL -> counts[v - v_lo] = #candidates of v
- *   fill  pass: offsets[v - v_lo] = exclusive prefix sum of counts (int64);
- *               pair_u / pair_v receive the (u, v) lists
- * Needs n/8 + n/256 bytes of shared memory (<= 200 KB, i.e. n <= ~1.6M).
- * ------------------------------------------------------------------------- */
-int eps_twohop_candidates(const int32_t *rowptr, const int32_t *col, int32_t n, int32_t v_lo,
-                          int32_t v_hi, const int64_t *offsets, uint32_t *counts, int32_t *pair_u,
-                          int32_t *pair_v, void *workspace, size_t workspace_bytes, void *stream);
-size_t eps_twohop_workspace_bytes(void);
-
-/* ---------------------------------------------------------------------------
- * K6+K3 fused  2-hop candidates of [v_lo, v_hi) TOGETHER WITH their CN / AA / RA
- * scores, from one walk over the 2-paths of each owner.
- * replaces: filter.py:96-109 (A@A enumeration, values discarded at :108-109)
- *           + the scoring loop filter.py:113-142 for the heuristic models
- *           (models.py:536-554, adamic_utils.py:13-25,
- *           train_and_eval.py:195-216).
  * A2's values ARE the scores: each 2-path v-k-u adds 1 (CN) or wtable[k]
  * (AA: 1/log deg, RA: 1/deg) to candidate (u, v).  Sums are accumulated as
  * 64-bit fixed-point integers with atomics (exact, order-independent), so
  * score[i] == eps_cn_aa's score of the same pair, bit for bit.
- *   offsets  int64[v_hi - v_lo + 1] exclusive prefix of the per-owner counts
- *            returned by eps_twohop_candidates' count pass; N = offsets[last]
- *   wtable   NULL -> score = CN count; else score = sum of wtable[k]
- *   flags    EPS_CN_SIGMOID | a similarity kind (EPS_SCORE_*, see eps_cn_aa; degrees from rowptr)
- *            (EPS_TWOHOP_UPPER is rejected: one-pass only)
- *   score    fp32[N] or NULL;  count int32[N] or NULL (exact CN)
- * Unweighted adjacency only (weighted graphs: eps_twohop_candidates + eps_cn_aa).
- * Needs ~3n/16 bytes of shared memory (<= 200 KB, i.e. n <= ~1.0M).
- * ------------------------------------------------------------------------- */
-int eps_twohop_scored(const int32_t *rowptr, const int32_t *col, const float *wtable, int32_t n,
-                      int32_t v_lo, int32_t v_hi, const int64_t *offsets, int64_t N, int flags,
-                      int32_t *pair_u, int32_t *pair_v, float *score, int32_t *count,
-                      void *workspace, size_t workspace_bytes, void *stream);
-size_t eps_twohop_scored_workspace_bytes(int64_t N);
-
-/* ---------------------------------------------------------------------------
- * K6 / K6+K3 ONE-PASS  the same enumeration (and, optionally, the same scores)
- * without the count pass and without a host prefix sum.
- * replaces: filter.py:96-109 (+ filter.py:113-142 for the heuristic models),
- *           exactly like eps_twohop_candidates / eps_twohop_scored above.
  * Every owner writes into a padded slot sized by a cheap upper bound of its
- * candidate count and records the real count; a scan of the counts and a
- * finalize pass (fixed point -> fp32, which reads every accumulator anyway)
+ * candidate count and records its real count; a scan of the counts and a
+ * compaction pass (fixed point -> fp32, which reads every accumulator anyway)
  * move the results to their compact positions.  No inter-CTA dependency.
  *   bound_offsets int64[v_hi - v_lo + 1] (device): exclusive prefix of any
  *                upper bound of the per-owner candidate counts, e.g.
@@ -359,10 +327,14 @@ size_t eps_twohop_scored_workspace_bytes(int64_t N);
  *                a 2-path v-k-u contributes A[u,k] * (A[v,k] * wtable[k]) (or
  *                A[u,k] * A[v,k] without wtable) — eps_cn_aa's products; the
  *                kernel reads A[k,u] for A[u,k], so A must be bitwise symmetric.
- *   wtable / flags / score / count as in eps_twohop_scored; score == NULL and
- *   count == NULL -> enumeration only (the GNN filter models).  A similarity
- *   kind (EPS_SCORE_*) runs the count-only walk and applies its formula in the
- *   compaction pass: weighted graphs pass val == NULL (structure only).
+ *   wtable       NULL -> score = CN count; else score = sum of wtable[k]
+ *   flags        EPS_CN_SIGMOID | a similarity kind (EPS_SCORE_*, see eps_cn_aa;
+ *                degrees from rowptr) | EPS_TWOHOP_UPPER
+ *   score        fp32[cap] or NULL;  count int32[cap] or NULL (exact CN).
+ *                score == NULL and count == NULL -> enumeration only (the GNN
+ *                filter models).  A similarity kind runs the count-only walk
+ *                and applies its formula in the compaction pass: weighted
+ *                graphs pass val == NULL (structure only).
  *   flags |= EPS_TWOHOP_UPPER: upper-triangle mode, only the candidates u > v
  *                of every owner v (each unordered pair once, under its smaller
  *                end).  Both walks visit only the suffix u > v of every N(k)
@@ -371,7 +343,7 @@ size_t eps_twohop_scored_workspace_bytes(int64_t N);
  *                n - 1 - v - |N(v) & (v, n)|).  Owner v's output is (u, v) in
  *                ascending u, and every score equals the full kernel's score
  *                of the same pair, bit for bit.
- * Results are bit-identical to the two-pass entry points.
+ * Needs ~3n/16 bytes of shared memory (<= 200 KB, i.e. n <= ~1.0M).
  * ------------------------------------------------------------------------- */
 #define EPS_TWOHOP_UPPER 4
 int eps_twohop_onepass(const int32_t *rowptr, const int32_t *col, const float *val, const float *wtable,

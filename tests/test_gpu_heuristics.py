@@ -210,10 +210,11 @@ def test_fused_twohop_scored_vs_oracle(shape):
 
 
 @pytest.mark.parametrize("shape", ["tiny", "small", "twitch"])
-def test_onepass_equals_twopass(shape):
-    """eps_twohop_onepass (padded per-owner slots sized by a bound, then scan + compaction) == count pass + prefix sum +
-    fill / fused kernels, bit for bit: pairs, order, scores, counts, per-owner offsets."""
-    from edge_proposal_sets_b200 import candidates
+def test_onepass_slots(shape):
+    """eps_twohop_onepass (padded per-owner slots sized by a bound, then scan + compaction): the per-owner counts are the
+    oracle's, exact bounds give the default-bound results bit for bit (pairs, order, scores, counts, offsets), an owner
+    sub-range is the matching slice of the full run, and a bound one too small raises."""
+    from edge_proposal_sets_b200 import candidates, ops
     from edge_proposal_sets_b200._lib import EpsError
     if shape == "twitch":
         z, ei, g = golden_graph("twitch")
@@ -221,39 +222,38 @@ def test_onepass_equals_twopass(shape):
         s, ei, w, g = synth_graph(shape)
     adj = to_adj(g, DEV)
     wt = _dev(oh.aa_ogb_weights(g))
+    cand = og.two_hop_candidates(g)
     counts = candidates.owner_counts(adj)
+    assert np.array_equal(counts.cpu().numpy(), np.bincount(cand[1], minlength=adj.n))
     N = int(counts.sum())
     bound = int(candidates.owner_bounds(adj).sum())
     assert bool((candidates.owner_bounds(adj) >= counts).all()) and bound >= N
-    e2 = candidates.two_hop(adj, counts=counts)
+    f = candidates.two_hop_scored(adj, wt, want_count=True, want_offsets=True)
     e1 = candidates.two_hop(adj)
-    assert e1.shape == (2, N) and torch.equal(e1, e2)
-    f2 = candidates.two_hop_scored(adj, wt, counts=counts, want_count=True)
-    f1 = candidates.two_hop_scored(adj, wt, want_count=True)
-    for a, b in zip(f1, f2):
-        assert torch.equal(a, b)
+    assert e1.shape == (2, N) and torch.equal(e1, f[0])
     c1 = candidates.two_hop_scored(adj, None)
-    assert torch.equal(c1[0], e2) and torch.equal(c1[1], f2[2].float())
+    assert torch.equal(c1[0], e1) and torch.equal(c1[1], f[2].float())
+    assert torch.equal(c1[1], ops.cn_aa(adj, e1, None, grouped_by_v=True))
     sg1 = candidates.two_hop_scored(adj, wt, sigmoid=True)
-    sg2 = candidates.two_hop_scored(adj, wt, counts=counts, sigmoid=True)
-    assert torch.equal(sg1[1], sg2[1])
+    assert torch.equal(sg1[0], e1) and torch.equal(sg1[1], ops.cn_aa(adj, e1, wt, sigmoid=True, grouped_by_v=True))
     # offsets, a tight capacity, an owner sub-range, and a violated bound
     e, sc, cn, off = candidates._onepass(adj, wt, 0, adj.n, counts, False, True, True)   # exact bounds
     assert torch.equal(off[1:], torch.cumsum(counts, 0)) and int(off[0]) == 0
-    assert torch.equal(e, e2) and torch.equal(sc, f2[1]) and torch.equal(cn, f2[2])
+    for a, b in zip((e, sc, cn, off), f):
+        assert torch.equal(a, b)
     lo, hi = adj.n // 3, (2 * adj.n) // 3
     sub = candidates.two_hop_scored(adj, wt, lo, hi, want_count=True)
-    sub2 = candidates.two_hop_scored(adj, wt, lo, hi, counts=counts[lo:hi], want_count=True)
-    for a, b in zip(sub, sub2):
-        assert torch.equal(a, b)
+    a, b = int(off[lo]), int(off[hi])
+    for x, y in zip(sub, (e[:, a:b], sc[a:b], cn[a:b])):
+        assert torch.equal(x, y)
     short = counts.clone()
     short[int(torch.argmax(counts))] -= 1                       # one owner's bound one too small
     with pytest.raises(EpsError):
         candidates._onepass(adj, wt, 0, adj.n, short, False, True, True)
-    # repeated runs are identical (the look-back is order-independent)
+    # repeated runs are identical (the owners' hand-out order does not reach the outputs)
     for _ in range(3):
-        again = candidates.two_hop_scored(adj, wt, want_count=True)
-        for a, b in zip(again, f2):
+        again = candidates.two_hop_scored(adj, wt, want_count=True, want_offsets=True)
+        for a, b in zip(again, f):
             assert torch.equal(a, b)
 
 
@@ -279,9 +279,6 @@ def test_fused_twohop_scored_tiny_graphs():
     assert not candidates.values_symmetric(adjw)
     with pytest.raises(EpsError):
         candidates.two_hop_scored(adjw, None)
-    with pytest.raises(EpsError):                      # the two-pass kernels have no weighted variant
-        candidates.two_hop_scored(to_adj(synth_graph("tiny")[3], DEV, keep_values=True), None,
-                                  counts=candidates.owner_counts(adj))
 
 
 def test_fused_weighted_collab_equals_pairwise_kernel():

@@ -63,7 +63,6 @@ def test_fused_and_k3_bit_exact_against_oracle(graphs, gname):
     from edge_proposal_sets_b200 import candidates, ops
     g, adj, cand, cnt = graphs[gname]
     assert (adj.val is not None) == (gname == "weighted")
-    counts = candidates.owner_counts(adj)
     rng = np.random.default_rng(1)
     arb = torch.from_numpy(np.concatenate([rng.integers(0, g.n, (2, 3000)),
                                            np.array([[0, 5, 2700, 2701, 17], [2700, 5, 2701, 2701, 17]]) % g.n], 1)).to(DEV)
@@ -76,10 +75,6 @@ def test_fused_and_k3_bit_exact_against_oracle(graphs, gname):
         he, hs = candidates.two_hop_scored(adj, kind=kind, upper=True)
         keep = e[0] > e[1]
         assert torch.equal(he, e[:, keep]) and torch.equal(hs.view(torch.int32), s[keep].view(torch.int32)), kind
-        # two-pass entry point (unweighted graphs only take it)
-        if adj.val is None:
-            e2, s2 = candidates.two_hop_scored(adj, kind=kind, counts=counts)
-            assert torch.equal(e2, e) and torch.equal(s2.view(torch.int32), s.view(torch.int32)), kind
         # K3 grouped and K3 pairs on the candidates, K3 pairs on arbitrary pairs (zero denominators included)
         for grouped in (True, False):
             k3 = ops.cn_aa(adj, e, kind=kind, grouped_by_v=grouped)

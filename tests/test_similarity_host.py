@@ -194,21 +194,16 @@ def test_kind_abi_rejects_before_any_cuda_call():
     def cn_aa(flags, val=None, wt=None):
         return lib.eps_cn_aa(d, d, val, wt, 10, d, d, 5, flags, d, None, d, 256, None)
 
-    def scored(flags, wt=None):
-        return lib.eps_twohop_scored(d, d, wt, 10, 0, 5, d, 3, flags, d, d, d, None, d, 1 << 20, None)
-
     def onepass(flags, val=None, wt=None):
         return lib.eps_twohop_onepass(d, d, val, wt, 10, 0, 5, d, 3, flags, d, d, d, None, d, d, 1 << 20, None)
 
-    for fn in (cn_aa, scored, onepass):
+    for fn in (cn_aa, onepass):
         for bad in unknown:
             assert fn(bad) == -1 and b"unknown flag bits" in lib.eps_last_error(), (fn.__name__, bad)
         assert fn(jac | _lib.EPS_CN_SIGMOID) == -1 and b"similarity kind" in lib.eps_last_error()
         assert fn(jac, wt=d) == -1 and b"similarity kind" in lib.eps_last_error()
     assert cn_aa(jac, val=d) == -1 and b"similarity kind" in lib.eps_last_error()
     assert onepass(jac, val=d) == -1 and b"similarity kind" in lib.eps_last_error()
-    # the upper-triangle flag keeps its own message on the two-pass entry point
-    assert scored(_lib.EPS_TWOHOP_UPPER | jac) == -1 and b"EPS_TWOHOP_UPPER" in lib.eps_last_error()
 
 
 def test_degree_guard_and_unknown_kind():
