@@ -64,6 +64,9 @@ SIGNATURES = {
     "eps_local_path_onepass_workspace_bytes": (_sz, [_i64, _i32, _i64, _i32]),
     "eps_local_path_pairs": (_int, [_vp, _vp, _i32, _vp, _vp, _i64, _int, _vp, _vp, _vp, _vp, _sz, _vp]),
     "eps_local_path_pairs_workspace_bytes": (_sz, []),
+    "eps_threehop_onepass": (_int, [_vp, _vp, _i32, _i32, _i32, _vp, _i64, _i64, _i32, _int, _vp, _vp, _vp, _vp, _sz,
+                                    _vp]),
+    "eps_threehop_onepass_workspace_bytes": (_sz, [_i64, _i32, _i64, _i32]),
     "eps_comm_unique_id": (_int, [_vp]),
     "eps_comm_init": (_int, [_vp, _int, _int, C.POINTER(_vp)]),
     "eps_comm_destroy": (_int, [_vp]),

@@ -30,12 +30,22 @@ def owner_counts(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None) -> torc
     return torch.cat(parts)
 
 
-def owner_bounds(adj: SparseAdj, upper: bool = False) -> torch.Tensor:
+def owner_bounds(adj: SparseAdj, upper: bool = False, hops: int = 2) -> torch.Tensor:
     """Upper bound of every owner's candidate count, int64 [n]: a candidate of v is the end point of
     a 2-path from v (<= #2-paths) and is neither v nor a neighbour of v: <= n - |N(v) U {v}|, i.e.
     n - 1 - deg v, or n - deg v when v carries a self loop (add_edges keeps them; v is then in N(v)).
     Torch ops only; sizes the outputs of the one-pass kernel and cuts owner ranges into slabs / GPU shards.
-    ``upper``: the bound of the half candidates u > v (``half_bounds``)."""
+    ``upper``: the bound of the half candidates u > v (``half_bounds``).  ``hops=3``: the distance-3 candidates
+    (``three_hop``), whose 2- and 3-walk counts add ``local_path_work`` (the 3-walks) to the first term."""
+    if hops == 3:
+        key = ("three_hop_bounds", bool(upper))
+        if key not in adj._cache:
+            owner_bounds(adj, upper)                      # caches the second term ("free" / "half_free")
+            walks = (half_two_path_work(adj) if upper else two_path_work(adj)) + local_path_work(adj)
+            adj._cache[key] = torch.minimum(walks, adj._cache["half_free" if upper else "free"])
+        return adj._cache[key]
+    if hops != 2:
+        raise ValueError(f"hops must be 2 or 3 (got {hops})")
     if upper:
         return half_bounds(adj)
     if "owner_bounds" not in adj._cache:
@@ -49,7 +59,8 @@ def owner_bounds(adj: SparseAdj, upper: bool = False) -> torch.Tensor:
             loop = (key[pos] == ar * adj.n + ar).long() if adj.nnz else torch.zeros_like(deg)
         else:
             loop = torch.ones_like(deg)                 # large graphs: the looser n - deg for everyone
-        adj._cache["owner_bounds"] = torch.minimum(two_path_work(adj), (adj.n - 1 - deg + loop).clamp_(min=0))
+        adj._cache["free"] = (adj.n - 1 - deg + loop).clamp_(min=0)
+        adj._cache["owner_bounds"] = torch.minimum(two_path_work(adj), adj._cache["free"])
     return adj._cache["owner_bounds"]
 
 
@@ -77,6 +88,7 @@ def half_bounds(adj: SparseAdj) -> torch.Tensor:
         if adj.nnz == 0:
             adj._cache["half_bounds"] = torch.zeros(n, dtype=torch.int64, device=adj.device)
             adj._cache["half_two_path_work"] = adj._cache["half_bounds"]
+            adj._cache["half_free"] = (n - 1 - torch.arange(n, device=adj.device)).clamp_(min=0)
             return adj._cache["half_bounds"]
         key, _, pos = _mirror_search(adj)
         # entry (v, k): the suffix of N(k) above v starts at the first key >= k * n + v + 1
@@ -87,7 +99,8 @@ def half_bounds(adj: SparseAdj) -> torch.Tensor:
         ar = torch.arange(n, device=adj.device)
         above = rp[1:] - torch.searchsorted(key, ar * n + ar + 1)          # |N(v) & (v, n)|
         adj._cache["half_two_path_work"] = paths
-        adj._cache["half_bounds"] = torch.minimum(paths, (n - 1 - ar - above).clamp_(min=0))
+        adj._cache["half_free"] = (n - 1 - ar - above).clamp_(min=0)
+        adj._cache["half_bounds"] = torch.minimum(paths, adj._cache["half_free"])
     return adj._cache["half_bounds"]
 
 
@@ -334,8 +347,8 @@ def local_path_work(adj: SparseAdj, upper: bool = False) -> torch.Tensor:
 
 
 def _lp_ctas(device) -> int:
-    """Per-CTA scratch areas handed to eps_local_path_onepass: every CTA that can be resident (<= 4 per SM at 512
-    threads)."""
+    """Per-CTA scratch areas handed to eps_local_path_onepass and eps_threehop_onepass: every CTA that can be resident
+    (<= 4 per SM at 512 threads)."""
     return 4 * torch.cuda.get_device_properties(device).multi_processor_count
 
 
@@ -377,3 +390,36 @@ def two_hop_local_path(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, c
     N = _compact_size(offsets, cap, "eps_local_path_onepass")
     out = (buf[:, :N], score[:N], c2[:N], c3[:N])
     return out + (offsets,) if want_offsets else out
+
+
+# ---------------------------------------------------------------------------------------------
+# Distance-3 candidates: the ends of 2- and 3-walks (include/eps.h, eps_threehop_onepass)
+# ---------------------------------------------------------------------------------------------
+def three_hop(adj: SparseAdj, v_lo: int = 0, v_hi: int | None = None, cap: int | None = None,
+              want_offsets: bool = False, upper: bool = False):
+    """The distance-<= 3 candidates of owners [v_lo, v_hi): every u with (A^2)_uv + (A^3)_uv > 0 that is neither v nor
+    a neighbour of v, as int32 [2, N] in the column-major order of ``two_hop`` (whose list is a subset).  Enumeration
+    only, one fused walk per owner (eps_threehop_onepass); ``cap`` / ``want_offsets`` / ``upper`` as in ``two_hop``,
+    with the bounds of ``owner_bounds(adj, upper, hops=3)``.  Structure only (edge values ignored)."""
+    _need_cuda(adj.col)
+    lib = _lib.load()
+    dev = adj.device
+    v_hi = adj.n if v_hi is None else v_hi
+    n_own = v_hi - v_lo
+    if n_own <= 0:
+        e = torch.empty((2, 0), dtype=torch.int32, device=dev)
+        return (e, torch.zeros(1, dtype=torch.int64, device=dev)) if want_offsets else e
+    boff, cap = _slot_offsets(owner_bounds(adj, upper, hops=3)[v_lo:v_hi], cap)
+    if "max_two_walk_ends" not in adj._cache:                # distinct 2-walk ends: <= #2-walks and <= n
+        adj._cache["max_two_walk_ends"] = int(two_path_work(adj).clamp(max=adj.n).max().item()) if adj.n else 0
+    max_ends, ctas = adj._cache["max_two_walk_ends"], _lp_ctas(dev)
+    buf = torch.empty((2, max(cap, 1)), dtype=torch.int32, device=dev)
+    offsets = torch.empty(n_own + 1, dtype=torch.int64, device=dev)
+    ws = _ws(lib.eps_threehop_onepass_workspace_bytes(cap, n_own, max_ends, ctas), dev)
+    check(lib.eps_threehop_onepass(_ptr(adj.rowptr), _ptr(adj.col), adj.n, v_lo, v_hi, _ptr(boff), cap, max_ends, ctas,
+                                   EPS_TWOHOP_UPPER if upper else 0, _ptr(buf[0]), _ptr(buf[1]), _ptr(offsets),
+                                   _ptr(ws), ws.numel(), _stream()), "eps_threehop_onepass")
+    from . import ops as _ops
+    _ops.LAUNCHES["n"] += 6
+    N = _compact_size(offsets, cap, "eps_threehop_onepass")
+    return (buf[:, :N], offsets) if want_offsets else buf[:, :N]

@@ -850,6 +850,187 @@ local_path_pairs_kernel(const int *__restrict__ rowptr, const int *__restrict__ 
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// K6 at distance 3 (eps_threehop_onepass; include/eps.h): the candidates of owner v are the ends of the 2-walks and
+// 3-walks from v that are neither v nor in N(v).  A 3-walk v - k - j - u passes through a 2-walk end j, so
+//   ends_3(v) = union of N(j) over j in ends_2(v) = union of N(k), k in N(v).
+// One CTA per owner, enumeration only (the compaction is twohop_compact_kernel<0> without scores):
+//   1. mark      ends_2 into the bitmap (walk_two_paths from every N(k), whole lists: the middle hop passes any id)
+//   2. freeze    rank + list ends_2 in ascending order into a per-CTA scratch: walk 3 must not iterate the live bitmap,
+//                which it fills (that would add 4-walk ends)
+//   3. walk 3    N(j) for every listed j, 32 lists per warp, flattened as lp_walk3_batch (lists >= TH_LONG warp-wide),
+//                atomicOr into the same bitmap; upper mode starts every N(j) at its lower bound of v + 1 and first
+//                clears the ends_2 bits below v + 1
+//   4. clear     N(v) and v
+//   5. rank, emit ascending u into the padded slot, cleanup — as twohop_score_kernel.
+// ---------------------------------------------------------------------------------------------
+constexpr int TH_THREADS = 512;
+constexpr int TH_LONG = 64;      // walk 3: lists at least this long are streamed warp-wide
+
+// Walk 3 for the listed 2-walk ends e0 .. e0 + cnt - 1 (one warp): every element u >= umin of their lists is marked.
+// The list was written by this CTA behind a barrier (possibly over lines an earlier owner left in L1): ld.global.cg.
+__device__ __forceinline__ void threehop_walk3_batch(const int *__restrict__ rowptr, const int *__restrict__ col,
+                                                     const int *ends, int e0, int cnt, int umin, MarkVisitor mv) {
+  const int lane = lane_id();
+  int s = 0, len = 0;
+  if (lane < cnt) {
+    const int j = __ldcg(ends + e0 + lane);
+    s = __ldg(rowptr + j);
+    const int e = __ldg(rowptr + j + 1);
+    if (umin > 0) {                                      // upper-triangle mode: first position with col >= umin
+      int lo = s, hi = e;
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (__ldg(col + mid) < umin) lo = mid + 1; else hi = mid;
+      }
+      s = lo;
+    }
+    len = e - s;
+  }
+  // ---- long lists: the whole warp streams one list, TS_DEPTH loads in flight per lane ----
+  unsigned longmask = __ballot_sync(FULL, len >= TH_LONG);
+  while (longmask) {
+    const int b = __ffs(longmask) - 1;
+    longmask &= longmask - 1;
+    const int sb = __shfl_sync(FULL, s, b);
+    const int lb = __shfl_sync(FULL, len, b);
+    const int *__restrict__ lp = col + sb;
+    for (int off = 0; off < lb; off += 32 * TS_DEPTH) {
+      int u[TS_DEPTH];
+#pragma unroll
+      for (int q = 0; q < TS_DEPTH; ++q) {
+        const int p = off + q * 32 + lane;
+        u[q] = p < lb ? __ldg(lp + p) : -1;
+      }
+#pragma unroll
+      for (int q = 0; q < TS_DEPTH; ++q)
+        if (u[q] >= 0) mv.visit(u[q], 0);
+    }
+  }
+  // ---- short lists: one flattened sequence ----
+  const int slen = len >= TH_LONG ? 0 : len;
+  int pin = slen;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const int t = __shfl_up_sync(FULL, pin, d);
+    if (lane >= d) pin += t;
+  }
+  const int pex = pin - slen;
+  const int total = __shfl_sync(FULL, pin, 31);
+  for (int jb = 0; jb < total; jb += 32) {
+    const int p = jb + lane;
+    int slot = 0;
+#pragma unroll
+    for (int step = 16; step >= 1; step >>= 1) {
+      const int t = __shfl_sync(FULL, pin, slot + step - 1);
+      if (t <= p) slot += step;
+    }
+    const int s_t = __shfl_sync(FULL, s, slot);
+    const int pe_t = __shfl_sync(FULL, pex, slot);
+    if (p < total) mv.visit(__ldg(col + s_t + (p - pe_t)), 0);
+  }
+}
+
+__global__ void __launch_bounds__(TH_THREADS)
+threehop_onepass_kernel(const int *__restrict__ rowptr, const int *__restrict__ col, int n, int v_lo, int v_hi,
+                        const long long *__restrict__ offsets, int *__restrict__ pad_u, int *scratch,
+                        long long scratch_cap, unsigned int *owner_counter, unsigned int *__restrict__ counts_out,
+                        const int *__restrict__ owner_order, int n_order, int upper) {
+  extern __shared__ uint32_t sm[];
+  const int W = (n + 31) >> 5;
+  const int W2 = (W + 31) >> 5;
+  uint32_t *bm = sm;
+  uint32_t *bm2 = bm + W;
+  uint32_t *blk = bm2 + W2;
+  uint16_t *pre = reinterpret_cast<uint16_t *>(blk + W2);
+  __shared__ int s_owner, s_walk, s_walk3;
+  __shared__ uint32_t s_scan[TH_THREADS / 32];
+  __shared__ uint32_t s_carry;
+  const int tid = threadIdx.x, lane = lane_id();
+  constexpr int NW = TH_THREADS / 32;
+  int *ends = scratch + (long long)blockIdx.x * scratch_cap;
+  for (int w = tid; w < W + W2; w += TH_THREADS) sm[w] = 0;
+  for (;;) {
+    __syncthreads();
+    if (tid == 0) {
+      const int t = (int)atomicAdd(owner_counter, 1u);
+      s_owner = (owner_order && t < n_order) ? v_lo + owner_order[t] : v_lo + t;
+      s_walk = 0;
+      s_walk3 = 0;
+      s_carry = 0;
+    }
+    __syncthreads();
+    const int v = s_owner;
+    if (v >= v_hi) break;
+    const int vs = __ldg(rowptr + v), ve = __ldg(rowptr + v + 1);
+    int LG = 32;
+    while (LG > 1 && (ve - vs + LG - 1) / LG < 4 * NW) LG >>= 1;
+    const long long out_base = offsets[v - v_lo];
+    if (offsets[v - v_lo + 1] == out_base) continue;  // no (room for) candidates (uniform): bitmap untouched
+    const int umin = upper ? v + 1 : 0;
+    const int g0 = umin >> 10;
+    // ---- 1. mark the 2-walk ends ----
+    walk_two_paths(rowptr, col, vs, ve, lane, LG, &s_walk, 0, MarkVisitor{bm, bm2});
+    __syncthreads();
+    // ---- 2. freeze them: ascending list in the per-CTA scratch ----
+    const uint32_t n2 = rank_blocks<TH_THREADS>(bm, bm2, blk, pre, 0, W2, s_scan, &s_carry);
+    if ((long long)n2 > scratch_cap) {                 // the caller's bound of the 2-walk ends is violated: poison N
+      if (tid == 0) counts_out[v - v_lo] = 0xffffffffu;
+      clear_blocks<TH_THREADS>(bm, bm2, 0, W2);
+      continue;
+    }
+    for (int g = tid; g < W2; g += TH_THREADS) {
+      uint32_t o = blk[g];
+      for (uint32_t m = bm2[g]; m; m &= m - 1) {
+        const int w = g * 32 + __ffs(m) - 1;
+        for (uint32_t bits = bm[w]; bits; bits &= bits - 1) ends[o++] = (w << 5) + __ffs(bits) - 1;
+      }
+    }
+    __syncthreads();
+    if (upper) {                                       // keep only marks >= umin: blocks below g0, then words below umin
+      clear_blocks<TH_THREADS>(bm, bm2, 0, g0);
+      const int w0 = umin >> 5;
+      for (int w = g0 * 32 + tid; w <= w0 && w < W; w += TH_THREADS)
+        bm[w] &= w < w0 ? 0u : ~((1u << (umin & 31)) - 1u);
+    }
+    __syncthreads();
+    // ---- 3. walk 3: N(j) of every 2-walk end j, 32 lists per warp, handed out dynamically ----
+    for (;;) {
+      int b = 0;
+      if (lane == 0) b = atomicAdd(&s_walk3, 1);
+      const int e0 = __shfl_sync(FULL, b, 0) * 32;
+      if (e0 >= (int)n2) break;
+      threehop_walk3_batch(rowptr, col, ends, e0, min(32, (int)n2 - e0), umin, MarkVisitor{bm, bm2});
+    }
+    __syncthreads();
+    // ---- 4. clear known edges and the diagonal ----
+    for (int p = vs + tid; p < ve; p += TH_THREADS) {
+      const int k = __ldg(col + p);
+      if (k >= umin) atomicAnd(&bm[k >> 5], ~(1u << (k & 31)));
+    }
+    if (tid == 0) {
+      if (v >= umin) atomicAnd(&bm[v >> 5], ~(1u << (v & 31)));
+      s_carry = 0;
+    }
+    __syncthreads();
+    // ---- 5. rank, emit ascending u, cleanup ----
+    const uint32_t total = rank_blocks<TH_THREADS>(bm, bm2, blk, pre, g0, W2, s_scan, &s_carry);
+    const bool fits = (long long)total <= offsets[v - v_lo + 1] - out_base;
+    if (tid == 0) counts_out[v - v_lo] = fits ? total : 0xffffffffu;
+    if (fits) {
+      for (int g = g0 + tid; g < W2; g += TH_THREADS) {
+        long long o = out_base + blk[g];
+        for (uint32_t m = bm2[g]; m; m &= m - 1) {
+          const int w = g * 32 + __ffs(m) - 1;
+          for (uint32_t bits = bm[w]; bits; bits &= bits - 1) pad_u[o++] = (w << 5) + __ffs(bits) - 1;
+        }
+      }
+    }
+    __syncthreads();
+    clear_blocks<TH_THREADS>(bm, bm2, g0, W2);
+  }
+}
+
 }  // namespace eps
 
 extern "C" int eps_score_kinds(void) {
@@ -1077,5 +1258,53 @@ extern "C" int eps_local_path_pairs(const int32_t *rowptr, const int32_t *col, i
   local_path_pairs_kernel<<<grid, LPP_THREADS, bitmap_bytes, stream>>>(rowptr, col, n, pair_u, pair_v, (long long)M,
                                                                      score, c2, c3, (unsigned long long *)workspace);
   EPS_LAUNCH_CHECK();
+  return EPS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Distance-3 enumeration entry point
+// ---------------------------------------------------------------------------------------------
+extern "C" size_t eps_threehop_onepass_workspace_bytes(int64_t cap, int32_t n_owners, int64_t max_ends, int32_t ctas) {
+  const size_t c = (size_t)(cap > 0 ? cap : 0), o = (size_t)(n_owners > 0 ? n_owners : 0);
+  const size_t s = (size_t)(max_ends > 0 ? max_ends : 0) * (size_t)(ctas > 0 ? ctas : 0);
+  // header | padded u | per-CTA list of the 2-walk ends
+  return onepass_header_bytes(o) + up256(c * 4) + up256(s * 4);
+}
+
+extern "C" int eps_threehop_onepass(const int32_t *rowptr, const int32_t *col, int32_t n, int32_t v_lo, int32_t v_hi,
+                                    const int64_t *bound_offsets, int64_t cap, int64_t max_ends, int32_t ctas, int flags,
+                                    int32_t *pair_u, int32_t *pair_v, int64_t *offsets_out, void *workspace,
+                                    size_t workspace_bytes, void *stream_) {
+  using namespace eps;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  EPS_CHECK_ARG(rowptr && col && bound_offsets && offsets_out, "null graph, bound_offsets or offsets_out pointer");
+  EPS_CHECK_ARG(n > 0 && v_lo >= 0 && v_hi <= n && v_lo < v_hi && cap >= 0 && cap < (1ll << 31),
+                "bad owner range or cap");
+  EPS_CHECK_ARG(max_ends >= 0 && max_ends < (1ll << 31) && ctas >= 1, "bad max_ends or ctas");
+  EPS_CHECK_ARG(cap == 0 || (pair_u && pair_v), "missing pair output pointer");
+  EPS_CHECK_ARG(!(flags & ~EPS_TWOHOP_UPPER), "unknown flag bits");
+  const int n_own = v_hi - v_lo;
+  if (!workspace || workspace_bytes < eps_threehop_onepass_workspace_bytes(cap, n_own, max_ends, ctas)) {
+    set_error("eps_threehop_onepass: workspace too small");
+    return EPS_ERR_WORKSPACE;
+  }
+  const int sms = sm_count();
+  if (sms <= 0) { set_error("eps_threehop_onepass: no CUDA device"); return EPS_ERR_CUDA; }
+  OnepassPlan p;
+  if (const int st = onepass_begin("eps_threehop_onepass", n, n_own, workspace, stream, p)) return st;
+  int *pad_u = (int *)p.slots;
+  int *scratch = (int *)((uint8_t *)pad_u + up256((size_t)cap * 4));
+  if (const int st = onepass_run(p, threehop_onepass_kernel, TH_THREADS, ctas, n_own, bound_offsets, cap, offsets_out,
+                                 sms, stream, rowptr, col, n, v_lo, v_hi, (const long long *)bound_offsets, pad_u,
+                                 scratch, (long long)max_ends, p.ticket, p.counts, p.order, n_own,
+                                 (flags & EPS_TWOHOP_UPPER) ? 1 : 0))
+    return st;
+  if (cap > 0) {
+    twohop_compact_kernel<0><<<p.cgrid, CP_THREADS, 0, stream>>>(rowptr, (const long long *)bound_offsets,
+                                                                (const long long *)offsets_out, v_lo, n_own,
+                                                                (long long)cap, pad_u, nullptr, nullptr, 0, pair_u,
+                                                                pair_v, nullptr, nullptr);
+    EPS_LAUNCH_CHECK();
+  }
   return EPS_OK;
 }

@@ -102,14 +102,15 @@ def ra_graph_from_train_edges(train_edges: torch.Tensor, num_nodes: int) -> Spar
 
 
 def iter_slabs(adj: SparseAdj, v_lo: int, v_hi: int, slab_pairs: int,
-               upper: bool = False) -> Iterator[Tuple[int, int, int]]:
+               upper: bool = False, hops: int = 2) -> Iterator[Tuple[int, int, int]]:
     """Yield (lo, hi, cap) owner ranges whose candidate count is at most ``cap <= slab_pairs``
     (a single owner whose bound exceeds that gets a slab of its own).  ``cap`` is the sum of the
     per-owner upper bounds (candidates.owner_bounds) — it sizes the one-pass kernel's outputs, so no
-    count pass over the graph is needed to plan the slabs.  ``upper``: the bounds of the half candidates u > v."""
+    count pass over the graph is needed to plan the slabs.  ``upper``: the bounds of the half candidates u > v.
+    ``hops=3``: the bounds of the distance-3 candidates (``candidates.three_hop``)."""
     if v_hi <= v_lo:
         return
-    cs = torch.cumsum(candidates.owner_bounds(adj, upper)[v_lo:v_hi], 0).cpu()
+    cs = torch.cumsum(candidates.owner_bounds(adj, upper, hops)[v_lo:v_hi], 0).cpu()
     lo = 0
     n_own = v_hi - v_lo
     base = 0
@@ -123,7 +124,7 @@ def iter_slabs(adj: SparseAdj, v_lo: int, v_hi: int, slab_pairs: int,
         lo = hi
 
 
-def owner_cost(adj: SparseAdj, jobs, upper: bool = False) -> torch.Tensor:
+def owner_cost(adj: SparseAdj, jobs, upper: bool = False, hops: int = 2) -> torch.Tensor:
     """Per-owner cost estimate that the multi-GPU owner ranges are balanced on.  Enumeration (K6) costs the owner's
     2-paths; scoring a candidate with a GNN filter model (K2) costs ~8 x a 2-path visit (measured on the ppa shape:
     0.218 ns per candidate against 0.029 ns per 2-path), and the candidate count is bounded by the owner's slot size
@@ -131,12 +132,14 @@ def owner_cost(adj: SparseAdj, jobs, upper: bool = False) -> torch.Tensor:
     others waiting at the merge (N = 4: 33 ms of a 615 ms step).  ``upper`` (mirror mode): the same model on the half
     work — the 2-paths that end above v and the half-candidate bound — which low owner ids carry most of.  A
     ``local_path`` job adds its walk-3 pull work (``candidates.local_path_work``, one list element ~ one 2-path visit),
-    ~160x the 2-path count on the ppa shape: it decides the balance."""
+    ~160x the 2-path count on the ppa shape: it decides the balance.  ``hops=3``: the distance-3 enumeration also
+    streams N(j) of every 2-walk end j, estimated the same way (``local_path_work``), and the GNN term uses the
+    distance-3 bound."""
     work = (candidates.half_two_path_work(adj) if upper else candidates.two_path_work(adj)).double()
     names = [j.name if hasattr(j, "name") else j[0] for j in jobs]
     if any(nm in GNN_MODELS for nm in names):
-        work = work + 8.0 * candidates.owner_bounds(adj, upper).double()
-    if LOCAL_PATH in names:
+        work = work + 8.0 * candidates.owner_bounds(adj, upper, hops).double()
+    if LOCAL_PATH in names or hops == 3:
         work = work + candidates.local_path_work(adj, upper).double()
     return work
 
@@ -170,7 +173,9 @@ def mirror_topk(half: torch.Tensor, k: int, n: int, select=None) -> torch.Tensor
     before P's first row in the full order, so fewer than k pairs precede P and P is in the half top-k.
     Hence: the half top-k (``half``, k rows), its mirrored rows (v, u, s) added, the 2k rows put into candidate order
     by one int64 key sort (v * n + u), and K4's select (score descending, ties by position) gives the full list.
-    ``select(edges, score, k)`` stands in for ``ops.topk_edges`` (the CPU tests pass a stable sort)."""
+    ``select(edges, score, k)`` stands in for ``ops.topk_edges`` (the CPU tests pass a stable sort).
+    The proof uses only that the candidate relation is symmetric and that the stream is in column-major order, so it
+    holds for the distance-3 candidates (``hops=3``) as for the 2-hop ones."""
     if half.shape[0] == 0:
         return half
     both = torch.cat([half, half[:, [1, 0, 2]]], 0)
@@ -361,12 +366,12 @@ def tc_arm_supported(model) -> bool:
 def filter_topk_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: int = 1 << 27,
                       distributed: bool = False, stats: Optional[dict] = None, pushdown: bool = True,
                       owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None,
-                      mirror: Optional[bool] = None):
+                      mirror: Optional[bool] = None, hops: int = 2):
     """``_filter_multi`` (see there) with the prefilter's safety net: when a job's tensor-core scores leave the
     calibrated tolerance, or its band cannot prune, the call is repeated with that job on the fp32 arm."""
     jobs = [j if isinstance(j, FilterJob) else FilterJob(*j) for j in jobs]
     try:
-        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners, per_node, mirror)
+        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners, per_node, mirror, hops)
     except PrefilterToleranceError as exc:
         import warnings
         warnings.warn(f"{exc}; re-running the filter step on the fp32 arm")
@@ -375,14 +380,14 @@ def filter_topk_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pai
                 j.precision = "fp32"
         if stats is not None:
             stats["prefilter_fallback"] = str(exc)
-        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners, per_node, mirror)
+        return _filter_multi(jobs, x, adj, k, slab_pairs, distributed, stats, pushdown, owners, per_node, mirror, hops)
 
 
 @torch.no_grad()
 def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: int = 1 << 27,
                   distributed: bool = False, stats: Optional[dict] = None, pushdown: bool = True,
                   owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None,
-                  mirror: Optional[bool] = None):
+                  mirror: Optional[bool] = None, hops: int = 2):
     """The filter step for several filter models over ONE enumeration of the 2-hop candidates: a list of
     sorted proposal lists (float32 ``[k,3]`` rows (u, v, score) on the device; score descending, ties by
     the reference's candidate order), one per job.  ``k=None`` keeps every candidate like the reference.
@@ -422,7 +427,20 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
     its running top-k over them by K4's rule — the prefilter's calibration, band, pool and fp32 re-scoring run
     unchanged on the half pairs — the ranks merge the half lists as usual, and ``mirror_topk`` rebuilds the full list,
     bit for bit the list of ``mirror=False``.  ``stats["candidates_scored"]`` still counts the directed candidates the
-    lists rank (2 x ``stats["pairs_evaluated"]``, the half pairs scored); ``stats["mirror"]`` says which path ran."""
+    lists rank (2 x ``stats["pairs_evaluated"]``, the half pairs scored); ``stats["mirror"]`` says which path ran.
+
+    ``hops=3`` draws the candidates from distance <= 3 (``candidates.three_hop``: the ends of 2- and 3-walks from v
+    that are neither v nor its neighbours) instead of the 2-hop set, for GNN jobs only: the CN-family scores are 0 on
+    every added pair, and the Local Path walk is built on the 2-hop set, so a heuristic job raises ValueError before
+    anything is launched.  Everything after the enumeration (prefilter, per-node budgets, mirror mode, the multi-GPU
+    merge) takes the stream unchanged; ``stats["hops"]`` records it."""
+    if hops not in (2, 3):
+        raise ValueError(f"hops must be 2 or 3 (got {hops})")
+    if hops == 3:
+        bad = sorted({(j.name if isinstance(j, FilterJob) else j[0]) for j in jobs} - set(GNN_MODELS))
+        if bad:
+            raise ValueError(f"hops=3 takes GNN filter models only ({', '.join(GNN_MODELS)}), not {', '.join(bad)}: "
+                             "the heuristic scores are built on the 2-hop candidates")
     rank, world = parallel.world_info() if distributed else (0, 1)
     if per_node is not None and int(per_node) < 1:
         raise ValueError(f"per_node must be >= 1 (got {per_node})")
@@ -436,12 +454,12 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
         raise ValueError("mirror=True: this call cannot score each unordered pair once (it needs the whole graph, a k, "
                          "no per-node budget, a structurally symmetric graph and bit-symmetric scores)")
     if half:
-        candidates.owner_bounds(adj, upper=True)             # half slot bounds: planned with the symmetry check
+        candidates.owner_bounds(adj, True, hops)             # half slot bounds: planned with the symmetry check
         ph.mark("mirror")                                    # (one search over the entries, once per graph)
     o_lo, o_hi = (0, adj.n) if owners is None else (max(int(owners[0]), 0), min(int(owners[1]), adj.n))
     v_lo, v_hi = o_lo, o_hi
     if world > 1:
-        bounds = parallel.partition_by_work(owner_cost(adj, jobs, half)[o_lo:o_hi], world)
+        bounds = parallel.partition_by_work(owner_cost(adj, jobs, half, hops)[o_lo:o_hi], world)
         v_lo, v_hi = o_lo + bounds[rank], o_lo + bounds[rank + 1]
     # per job: scoring plan + running proposal set.  A local_path job always takes the fused walk (its pair kernel is for
     # evaluation sets, ~Σ deg u of work per candidate); the other heuristic jobs then go to K3.
@@ -478,7 +496,7 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
         ph.mark("triangles")
     n_slabs = 0
     n_cand = 0
-    for lo, hi, cap in iter_slabs(adj, v_lo, v_hi, slab_pairs, half):
+    for lo, hi, cap in iter_slabs(adj, v_lo, v_hi, slab_pairs, half, hops):
         n_slabs += 1
         scores = {}
         offsets = None
@@ -493,7 +511,8 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
             offsets = r[2] if m is not None else None
             ph.mark("enum_score")
         else:
-            r = candidates.two_hop(adj, lo, hi, cap=cap, want_offsets=m is not None, upper=half)
+            enum = candidates.three_hop if hops == 3 else candidates.two_hop
+            r = enum(adj, lo, hi, cap=cap, want_offsets=m is not None, upper=half)
             edges, offsets = r if m is not None else (r, None)
             ph.mark("enum")
         if edges.shape[1] == 0:
@@ -549,6 +568,7 @@ def _filter_multi(jobs, x, adj: SparseAdj, k: Optional[int] = None, slab_pairs: 
         stats["candidates_scored"] = 2 * seen if half else seen
         stats["pairs_evaluated"] = seen
         stats["mirror"] = half
+        stats["hops"] = hops
         if m is not None:
             stats["per_node"] = dict(m=m, survivors=[p["pn_kept"] for p in plans])
         stats["slabs"] = n_slabs
@@ -696,14 +716,14 @@ def filter_topk(model_name: str, model, x, adj: SparseAdj, k: Optional[int] = No
                 slab_pairs: int = 1 << 27, distributed: bool = False, ra_adj: Optional[SparseAdj] = None,
                 stats: Optional[dict] = None, precision: Optional[str] = None,
                 owners: Optional[Tuple[int, int]] = None, per_node: Optional[int] = None,
-                mirror: Optional[bool] = None) -> torch.Tensor:
+                mirror: Optional[bool] = None, hops: int = 2) -> torch.Tensor:
     """Sorted proposal list of one filter model, float32 ``[k,3]`` rows (u, v, score) on the device: score
     descending, ties by the reference's candidate order.  ``k=None`` keeps every candidate like the
     reference.  ``precision`` (GNN models): see ``FilterJob``; default = the model's ``linkpred.precision``.
-    ``per_node=m``: only the m best candidates of every owner v; ``mirror``: see ``_filter_multi``."""
+    ``per_node=m``: only the m best candidates of every owner v; ``mirror`` / ``hops``: see ``_filter_multi``."""
     job = FilterJob(model_name, model, ra_adj, precision)
     return filter_topk_multi([job], x, adj, k, slab_pairs, distributed, stats, owners=owners, per_node=per_node,
-                             mirror=mirror)[0]
+                             mirror=mirror, hops=hops)[0]
 
 
 def load_extra_edges(path: str, num_sorted_edge: int) -> torch.Tensor:

@@ -22,6 +22,8 @@ Differences from the reference, all on the fast side of the same semantics:
     kept rows are ordered like the global list (and cut to ``--topk`` when given), so the file is read the same way.
     The budget belongs to v, the second column; (v, u) need not be in u's list (the rank graph is symmetrised, so
     either row adds the undirected edge);
+  * ``--hops 3`` (GNN filters) draws the candidates from distance <= 3: every pair joined by a 2-walk or a 3-walk
+    that is not an edge, a superset of the reference's 2-hop candidates.  The file name and format are unchanged;
   * under ``torchrun`` the owners are sharded across the GPUs and merged with one all-gather.
 """
 from __future__ import annotations
@@ -64,6 +66,9 @@ def parse_args(argv=None):
     p.add_argument("--per_node_topk", type=_budget, default=None, metavar="M",
                    help="per-node proposal budget: keep only the M best candidates (u, v) of every node v, then order "
                         "them like the global list (and keep the first --topk rows when given); default: off")
+    p.add_argument("--hops", type=int, choices=[2, 3], default=2,
+                   help="candidate distance: 2 = pairs with a common neighbour (default); 3 = also the ends of 3-walks "
+                        "(GNN filters only: the heuristic scores are 0 on the added pairs)")
     p.add_argument("--slab_pairs", type=int, default=1 << 27)
     p.add_argument("--random_init", action="store_true",
                    help="score with seeded random weights when models/{checkpoint} does not exist")
@@ -125,7 +130,7 @@ def main(argv=None):
         raise SystemExit("filter.py: --topk is required under torchrun (only top-k lists are merged)")
     sorted_edges = filter_step.filter_topk(args.model, model, data.x, data.adj_t, k=k, slab_pairs=args.slab_pairs,
                                            distributed=distributed, ra_adj=ra_adj, stats=stats,
-                                           per_node=args.per_node_topk).cpu()
+                                           per_node=args.per_node_topk, hops=args.hops).cpu()
     print(f"using {stats.get('candidates_scored')} edges" + (" (this rank)" if distributed else ""))
     if rank == 0:
         print(sorted_edges)

@@ -393,6 +393,37 @@ int eps_local_path_pairs(const int32_t *rowptr, const int32_t *col, int32_t n, c
 size_t eps_local_path_pairs_workspace_bytes(void);
 
 /* ---------------------------------------------------------------------------
+ * K6 at distance 3: the distance-<= 3 candidates of the owner range [v_lo, v_hi)
+ * replaces: no reference counterpart (the reference enumerates 2-hop pairs
+ *           only, filter.py:96-109); proposal sets for the GNN filters that
+ *           include pairs without a common neighbour.
+ * Candidates of owner v are every u with (A^2)_uv + (A^3)_uv > 0 that is
+ * neither v nor in N(v): the ends of 2-walks and 3-walks from v (stored lists,
+ * self loops included, edge values ignored).  The 2-hop set of
+ * eps_twohop_onepass is a subset.  Enumeration only; owners ascending,
+ * candidates ascending in u (column-major order).
+ * The eps_twohop_onepass contract: padded slots sized by bound_offsets / cap
+ * (any upper bound of the per-owner counts, e.g. min(#2-walks + #3-walks,
+ * n - 1 - deg v + [self loop])), offsets_out, heaviest owners first,
+ * EPS_TWOHOP_UPPER (only u > v; the bounds then bound the half counts), and a
+ * violated bound poisons N (offsets_out[last] > cap) instead of overrunning.
+ *   max_ends   an upper bound of EVERY owner's number of distinct 2-walk ends
+ *              in [v_lo, v_hi) (e.g. min(#2-walks, n)); sizes the per-CTA list
+ *              the kernel freezes them in
+ *   ctas       number of per-CTA lists in the workspace; the kernel runs at
+ *              most that many CTAs
+ *   flags      0 or EPS_TWOHOP_UPPER
+ * Every argument is checked before any CUDA call.
+ * Workspace: eps_threehop_onepass_workspace_bytes(cap, v_hi - v_lo, max_ends, ctas).
+ * Needs ~3n/16 bytes of shared memory (<= 200 KB, i.e. n <= ~1.0M), as K6.
+ * ------------------------------------------------------------------------- */
+int eps_threehop_onepass(const int32_t *rowptr, const int32_t *col, int32_t n, int32_t v_lo, int32_t v_hi,
+                         const int64_t *bound_offsets, int64_t cap, int64_t max_ends, int32_t ctas, int flags,
+                         int32_t *pair_u, int32_t *pair_v, int64_t *offsets_out, void *workspace,
+                         size_t workspace_bytes, void *stream);
+size_t eps_threehop_onepass_workspace_bytes(int64_t cap, int32_t n_owners, int64_t max_ends, int32_t ctas);
+
+/* ---------------------------------------------------------------------------
  * K5  multi-GPU merge of per-GPU proposal lists (no counterpart in the
  * single-GPU reference; SURVEY.md section 8e).  One ncclAllGather of the
  * [k_local,3] fp32 (u, v, score) rows of every rank followed by a K4 select
