@@ -47,11 +47,16 @@ constexpr int P_MAX_CHUNKS = 8;                                    // 32-column 
 constexpr int P_GROUP_WARPS = 4;                                   // warps per producer group
 // Warp roles: 4 epilogue warps (one per TMEM lane quarter), then the MMA warp, the pair-id warp, NL loader warps
 // (fp16-table path) and NG producer groups of four warps each.
+//   fp16 table: NL = 4 loaders + NG = 1 group multiplying in place.  4 or 8 loaders with 1 or 2 groups all ran within
+//               3 % (profiles/round2_d_k2_timeline.md, step 11); this is the shape with the fewest warps.
+//   fp32 source (short lists): NL = 0, NG = 2 groups that load through registers.
+constexpr int p_groups(bool hb) { return hb ? 1 : 2; }
+constexpr int p_loaders(bool hb) { return hb ? 4 : 0; }
 // one CTA per SM: the whole register file is there to be used
-// (16384 registers per SM sub-partition, warps dealt round-robin: 18 warps -> 5 on one -> 96; 14 -> 4 -> 128)
+// (16384 registers per SM sub-partition, warps dealt round-robin: 14 warps -> 4 on one -> 128)
 constexpr int P_EPI_WARPS = 4;                                     // one per TMEM lane quarter
-constexpr int p_threads(int ng, int nl) { return (P_EPI_WARPS + 2 + nl + ng * P_GROUP_WARPS) * 32; }
-constexpr int p_maxreg(int ng, int nl) { return (16384 / (((p_threads(ng, nl) / 32) + 3) / 4) / 32) / 8 * 8; }
+constexpr int p_threads(bool hb) { return (P_EPI_WARPS + 2 + p_loaders(hb) + p_groups(hb) * P_GROUP_WARPS) * 32; }
+constexpr int p_maxreg(bool hb) { return (16384 / (((p_threads(hb) / 32) + 3) / 4) / 32) / 8 * 8; }
 constexpr int P_CHUNK_K = 32;
 constexpr int P_STAGE_BYTES = TC_BM * P_CHUNK_K * 2;               // 8 KB
 
@@ -200,19 +205,19 @@ __device__ __forceinline__ float2 fma_f32x2(float2 a, float2 b, float2 c) {
   asm("mov.b64 {%0, %1}, %2;" : "=f"(r.x), "=f"(r.y) : "l"(pr));
   return r;
 }
-template <int H, bool HB /* h is the fp16 table (else fp32) */, int NG /* producer groups */, int NL /* loader warps (fp16 table) */>
-__global__ void __cluster_dims__(2, 1, 1) __maxnreg__(p_maxreg(NG, NL))
+template <int H, bool HB /* h is the fp16 table (else fp32) */>
+__global__ void __cluster_dims__(2, 1, 1) __maxnreg__(p_maxreg(HB))
 linkpred_tc3_kernel(const void *__restrict__ h, const int *__restrict__ pu, const int *__restrict__ pv,
                     long long M, const MlpParams prm, int L, int apply_sigmoid,
-                    const uint8_t *__restrict__ wimg, float *__restrict__ score, int tune, int ring,
-                    const int *__restrict__ tile_order, const TcScale *__restrict__ scale) {
+                    const uint8_t *__restrict__ wimg, float *__restrict__ score, int ring,
+                    const TcScale *__restrict__ scale) {
   static_assert(H % 64 == 0 && H >= 64 && H <= 256, "H in {64,128,192,256}");
-  static_assert(HB ? (NL == 4 || NL == 8) : NL == 0, "loader warps exist on the fp16-table path only");
+  constexpr int NG = p_groups(HB), NL = p_loaders(HB);       // producer groups, loader warps
   constexpr int HH = H / 2;
   constexpr int WH_BYTES = HH * H * 2;
   constexpr int NCHUNK = H / P_CHUNK_K;                       // 32-column K-chunks per layer (8 KB of A operand each)
   constexpr int P_IDS_WARP = P_EPI_WARPS + 1, P_FIRST_LOAD_WARP = P_EPI_WARPS + 2, P_FIRST_PROD_WARP = P_FIRST_LOAD_WARP + NL;
-  constexpr int P_THREADS = p_threads(NG, NL);
+  constexpr int P_THREADS = p_threads(HB);
   constexpr int P_PROD_WARPS = NG * P_GROUP_WARPS;
   constexpr uint32_t TMEM_COLS = 2 * H <= 128 ? 128 : (2 * H <= 256 ? 256 : 512);
   constexpr uint32_t IDESC = umma_idesc_f16(2 * TC_BM, H);
@@ -326,8 +331,7 @@ linkpred_tc3_kernel(const void *__restrict__ h, const int *__restrict__ pu, cons
     const int q = warp & 3;
     const int row = q * 32 + lane;
     for (long long tile = cluster_id; tile < npair_tiles; tile += nclusters) {
-      const long long p0 = (tile_order ? (long long)__ldg(tile_order + tile) : tile) * (2 * TC_BM) +
-                           (long long)cta_rank * TC_BM;
+      const long long p0 = tile * (2 * TC_BM) + (long long)cta_rank * TC_BM;
       for (int l = 0; l < nhidden; ++l) {
         const uint32_t slot = seq++ & 1u;
         mbar_wait_cluster(smem_u32(&bars.acc_full[slot]), (acph >> slot) & 1u);
@@ -336,8 +340,7 @@ linkpred_tc3_kernel(const void *__restrict__ h, const int *__restrict__ pu, cons
         if (tid == 0) TR(5, l, 0);
         const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + slot * H;
         // 16-column loads, the next one always in flight (same TMEM read rate as 32-column loads,
-        // tools/micro/tmem_ld_bw.cu, at half the registers: the kernel fits 96 registers without spills, which is what
-        // lets it run 18 warps)
+        // tools/micro/tmem_ld_bw.cu, at half the registers)
         constexpr int NLD = 2 * NCHUNK;
         uint32_t buf[2][16];
         tmem_ld16_issue(taddr, buf[0]);
@@ -476,22 +479,24 @@ linkpred_tc3_kernel(const void *__restrict__ h, const int *__restrict__ pu, cons
   } else if (warp == P_IDS_WARP) {
     // =============================== PAIR IDS ===============================
     // (u, v) of this CTA's 128 rows -> shared memory, one tile ahead of the warps that gather, so a row gather never
-    // waits on a dependent index load.  The ids of the tile after that are already in registers, and their embedding
-    // rows are pulled into L2 from there (one DRAM page visit per 512-byte row instead of eight chunk-sized ones;
-    // the gathers, about one tile-time later, then hit L2).
+    // waits on a dependent index load.  Tiles run in list order: a u-blocked order that keeps a node range's rows in
+    // L2 was measured slower (profiles/round1_e_k2_tile_schedule.md).  The ids of the tile after that are already in
+    // registers; on the fp32-source path their embedding rows are pulled into L2 from there (one DRAM page visit per
+    // row instead of one per chunk-sized piece; the gathers, about one tile-time later, then hit L2).  The fp16-table
+    // path has no prefetch: its loaders run a ring ahead themselves, and the prefetch cost 2-4 % there
+    // (profiles/round2_d_k2_timeline.md, steps 10-11).
     constexpr int RB = H * (HB ? 2 : 4);
     const char *hb = reinterpret_cast<const char *>(h);
     int nu[4], nv[4];
     auto load_ids = [&](long long tile) {
-      const long long p0 = (tile_order ? (long long)__ldg(tile_order + tile) : tile) * (2 * TC_BM) +
-                           (long long)cta_rank * TC_BM;
+      const long long p0 = tile * (2 * TC_BM) + (long long)cta_rank * TC_BM;
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
         const long long p = p0 + lane + 32 * q;
         nu[q] = -1; nv[q] = -1;
         if (p < M) { nu[q] = __ldg(pu + p); nv[q] = __ldg(pv + p); }
       }
-      if (tune & 1) {
+      if constexpr (!HB) {
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
           const int vprev = __shfl_up_sync(FULL, nv[q], 1);
@@ -680,10 +685,7 @@ linkpred_tc3_kernel(const void *__restrict__ h, const int *__restrict__ pu, cons
         if (pstage >= (uint32_t)ring) { pstage -= (uint32_t)ring; lphase ^= 1u; }
         if (t == 0) TR(9, c, group);
         uint8_t *dst = sRing + stage * P_STAGE_BYTES;
-        if (tune & 32) {
-          // EXPERIMENT (EPS_TC3_TUNE bit 5, wrong scores): no multiply pass — what the kernel would run at if the A operand
-          // needed no shared-memory read-modify-write
-        } else if (uni) {
+        if (uni) {
           // the thread's four rows share one staged owner row (almost always): all five shared-memory loads are issued
           // before the first multiply, so the chunk costs ONE load latency, not four in a row
           const uint4 xv = *reinterpret_cast<const uint4 *>(sVt + kq[0] * (H * 2) + boff);       // warp-wide broadcast
@@ -773,96 +775,23 @@ linkpred_tc3_kernel(const void *__restrict__ h, const int *__restrict__ pu, cons
   }
 }
 
-// ---- L2-aware tile schedule -------------------------------------------------------------------------
-// The pair list is owner-major with u ascending inside an owner, so consecutive tiles sweep the whole
-// embedding table (295 MB of fp16 rows on the ppa shape, 2.3x the L2) once per owner and the row gathers
-// hit L2 only ~50 % of the time.  Scores are written by pair index, so the ORDER in which tiles are
-// processed is free: tiles are scheduled u-block by u-block (block = a node range whose rows fit the L2
-// budget), owners ascending inside a block — every row is then fetched from HBM about once per block
-// instead of once per owner.  tile_order[slot] = pair tile; a stable counting sort by the block of the
-// tile's first u (one CTA; a few hundred thousand tiles).  An experiment knob, see tc3_ublock_nodes.
-constexpr int TO_THREADS = 256, TO_MAX_BLOCKS = 32;     // 33 KB of static shared memory
-
-__global__ void __launch_bounds__(TO_THREADS)
-tile_order_kernel(const int *__restrict__ pu, long long M, long long ntiles, int tile_pairs, int block_nodes,
-                  int nblocks, int *__restrict__ order) {
-  __shared__ int cnt[TO_MAX_BLOCKS][TO_THREADS + 1];
-  const int t = threadIdx.x;
-  const long long per = (ntiles + TO_THREADS - 1) / TO_THREADS;
-  const long long lo = min(ntiles, (long long)t * per), hi = min(ntiles, lo + per);
-  for (int b = 0; b < nblocks; ++b) cnt[b][t] = 0;
-  for (long long i = lo; i < hi; ++i) cnt[min(__ldg(pu + i * tile_pairs) / block_nodes, nblocks - 1)][t]++;
-  __syncthreads();
-  // exclusive scan in (block, thread) order: thread b*... a single warp per block row is plenty
-  __shared__ int base[TO_MAX_BLOCKS + 1];
-  if (t < nblocks) {
-    int run = 0;
-    for (int j = 0; j < TO_THREADS; ++j) { const int c = cnt[t][j]; cnt[t][j] = run; run += c; }
-    cnt[t][TO_THREADS] = run;
-  }
-  __syncthreads();
-  if (t == 0) {
-    int run = 0;
-    for (int b = 0; b < nblocks; ++b) { base[b] = run; run += cnt[b][TO_THREADS]; }
-  }
-  __syncthreads();
-  int pos[TO_MAX_BLOCKS];
-#pragma unroll 1
-  for (int b = 0; b < nblocks; ++b) pos[b] = base[b] + cnt[b][t];
-  for (long long i = lo; i < hi; ++i) {
-    const int b = min(__ldg(pu + i * tile_pairs) / block_nodes, nblocks - 1);
-    order[pos[b]++] = (int)i;
-  }
-}
-
-// node-range size whose embedding rows fit the L2 budget; 0 = keep the natural order
-int tc3_ublock_nodes(int n, int row_bytes, long long M) {
-  // OFF by default: measured on the ppa shape (profiles/round1_e_k2_tile_schedule.md) the schedule does not
-  // pay — 64.9 ms per 4 slabs in natural order vs 65.7 / 66.7 / 66.6 / 68.3 ms with 32 / 48 / 64 / 96 MB
-  // blocks: the id warp's L2 prefetch already hides the misses, and blocking gives up the h[v] reuse of
-  // long owner runs.  EPS_TC3_UBLOCK_MB=<MB> switches it on for A/B runs.
-  int mb = 0;
-  if (const char *e = getenv("EPS_TC3_UBLOCK_MB")) mb = atoi(e);
-  if (mb <= 0) return 0;
-  const long long table = (long long)n * row_bytes, budget = (long long)mb << 20;
-  if (table <= budget || M < 8ll * n) return 0;          // table already L2-resident / too few pairs per row
-  long long nb = (table + budget - 1) / budget;
-  if (nb > TO_MAX_BLOCKS) nb = TO_MAX_BLOCKS;
-  return (int)((n + nb - 1) / nb);
-}
-
-template <int H, bool HB, int NG, int NL>
-static int tc3_launch_g(const void *h, const int *pu, const int *pv, long long M, const MlpParams &prm, int L,
-                        int apply_sigmoid, float *score, uint8_t *img, int n, int *tile_order, const TcScale *scale,
-                        cudaStream_t stream) {
+template <int H, bool HB>
+static int tc3_launch(const void *h, const int *pu, const int *pv, long long M, const MlpParams &prm, int L,
+                      int apply_sigmoid, float *score, uint8_t *img, const TcScale *scale, cudaStream_t stream) {
   const int nhidden = L - 1;
   const size_t fixed = (size_t)nhidden * (H / 2) * H * 2 +
                        (size_t)TC_BM * 32 + (size_t)nhidden * (H / 2) * 32 +          // bias K-step tiles
                        sizeof(float) * (size_t)H + 2 * TC_BM * sizeof(int2) + 2 * TC_BM * sizeof(int) +
                        (HB ? (size_t)2 * P_VROWS * H * 2 : 0) + 32 + sizeof(PipeBarriers);
   const size_t budget = 227 * 1024;
-  if (fixed + (size_t)(NG + 1) * P_STAGE_BYTES > budget) return EPS_ERR_UNSUPPORTED;   // the resident weights do not fit (H = 256, L >= 4)
-  int ring = (int)std::min<size_t>((budget - fixed) / P_STAGE_BYTES, (size_t)P_MAX_RING);
-  const char *rg = getenv("EPS_TC3_RING");    // cap the ring depth (A/B measurements)
-  if (rg && atoi(rg) >= NG + 1) ring = std::min(ring, atoi(rg));
+  if (fixed + (size_t)(p_groups(HB) + 1) * P_STAGE_BYTES > budget) return EPS_ERR_UNSUPPORTED;   // the resident weights do not fit (H = 256, L >= 4)
+  const int ring = (int)std::min<size_t>((budget - fixed) / P_STAGE_BYTES, (size_t)P_MAX_RING);
   const size_t smem = fixed + (size_t)ring * P_STAGE_BYTES;
-  auto kern = linkpred_tc3_kernel<H, HB, NG, NL>;
+  auto kern = linkpred_tc3_kernel<H, HB>;
   EPS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const long long npair_tiles = (M + 2 * TC_BM - 1) / (2 * TC_BM);
   const int clusters = (int)std::min<long long>(npair_tiles, (long long)(sm_count() / 2));
-  // EPS_TC3_TUNE bit 0: L2 prefetch of whole embedding rows by the ids warp, one tile ahead.  On for the fp32 source;
-  // off for the fp16 table, whose loaders run a tile ahead themselves (measured: 7.06 ms without, 7.20 with; a
-  // row-completing prefetch at the first chunk of a tile changed nothing either, gpurun_out/r3g_call.log)
-  const char *tn = getenv("EPS_TC3_TUNE");
-  const int tune = tn ? atoi(tn) : (HB ? 0 : 1);
-  const int block_nodes = tile_order ? tc3_ublock_nodes(n, H * (HB ? 2 : 4), M) : 0;
-  if (block_nodes > 0) {
-    const int nblocks = (n + block_nodes - 1) / block_nodes;
-    tile_order_kernel<<<1, TO_THREADS, 0, stream>>>(pu, M, npair_tiles, 2 * TC_BM, block_nodes, nblocks, tile_order);
-    EPS_LAUNCH_CHECK();
-  }
-  kern<<<2 * clusters, p_threads(NG, NL), smem, stream>>>(h, pu, pv, M, prm, L, apply_sigmoid, img, score, tune, ring,
-                                                     block_nodes > 0 ? tile_order : nullptr, scale);
+  kern<<<2 * clusters, p_threads(HB), smem, stream>>>(h, pu, pv, M, prm, L, apply_sigmoid, img, score, ring, scale);
   EPS_LAUNCH_CHECK();
 #ifdef EPS_TC3_TRACE
   if (const char *tf = getenv("EPS_TC3_TRACE_FILE")) {
@@ -875,26 +804,6 @@ static int tc3_launch_g(const void *h, const int *pu, const int *pv, long long M
   }
 #endif
   return EPS_OK;
-}
-
-template <int H, bool HB>
-static int tc3_launch_h(const void *h, const int *pu, const int *pv, long long M, const MlpParams &prm, int L,
-                        int apply_sigmoid, float *score, uint8_t *img, int n, int *tile_order, const TcScale *scale,
-                        cudaStream_t stream) {
-  // Warp budget (one CTA per SM): 4 epilogue + MMA + ids + NL loaders + 4 NG producers.
-  //   fp16 table: NL = 4 loaders + 1 group multiplying in place (14 warps -> 128 registers) by default;
-  //               EPS_TC3_SHAPE=42 / 81 / 82: NL NG = 4 2 / 8 1 / 8 2 (18-22 warps -> 96-80 registers) for A/B runs;
-  //   fp32 source (short lists): 2 groups that load through registers, no loaders.
-  if constexpr (HB) {
-    const char *e = getenv("EPS_TC3_SHAPE");
-    const int shape = e ? atoi(e) : 41;
-    if (shape == 42) return tc3_launch_g<H, true, 2, 4>(h, pu, pv, M, prm, L, apply_sigmoid, score, img, n, tile_order, scale, stream);
-    if (shape == 81) return tc3_launch_g<H, true, 1, 8>(h, pu, pv, M, prm, L, apply_sigmoid, score, img, n, tile_order, scale, stream);
-    if (shape == 82) return tc3_launch_g<H, true, 2, 8>(h, pu, pv, M, prm, L, apply_sigmoid, score, img, n, tile_order, scale, stream);
-    return tc3_launch_g<H, true, 1, 4>(h, pu, pv, M, prm, L, apply_sigmoid, score, img, n, tile_order, scale, stream);
-  } else {
-    return tc3_launch_g<H, false, 2, 0>(h, pu, pv, M, prm, L, apply_sigmoid, score, img, n, tile_order, scale, stream);
-  }
 }
 
 // ---- prepare kernels: scale, fp16 table, weight images (once per (h, weights); EPS_MLP_REUSE_WORKSPACE skips them) ----
@@ -1000,9 +909,8 @@ static size_t tc_img_bytes(int H, int L) {
 }
 
 size_t linkpred_tc_workspace_bytes(int n, int H, int L, long long M) {
-  // header (TcScale, max |h|) | weight images | fp16 embedding table | tile schedule (one int per 256 pairs)
-  return 256 + tc_img_bytes(H, L) + (linkpred_tc_uses_table(n, M) ? (((size_t)n * H * 2 + 255) & ~(size_t)255) : 0) +
-         (size_t)((M + 255) / 256) * 4 + 256;
+  // header (TcScale, max |h|) | weight images | fp16 embedding table: on the table path the size does not depend on M
+  return 256 + tc_img_bytes(H, L) + (linkpred_tc_uses_table(n, M) ? (((size_t)n * H * 2 + 255) & ~(size_t)255) : 0);
 }
 
 int linkpred_tc_launch(const float *h, int n, int H, const int *pu, const int *pv, long long M,
@@ -1021,10 +929,8 @@ int linkpred_tc_launch(const float *h, int n, int H, const int *pu, const int *p
   TcScale *scale = (TcScale *)ws;
   unsigned int *hmax_bits = (unsigned int *)(ws + 64);
   uint8_t *img = ws + 256;
-  uint8_t *tail = img + tc_img_bytes(H, L);
   const bool use_table = linkpred_tc_uses_table(n, M);
-  void *table = use_table ? tail : nullptr;
-  if (use_table) tail += ((size_t)n * H * 2 + 255) & ~(size_t)255;
+  void *table = use_table ? img + tc_img_bytes(H, L) : nullptr;
   if (!prepared) {                                  // EPS_MLP_REUSE_WORKSPACE: scale, table and images are still there
     const int sms = sm_count();
     EPS_CUDA(cudaMemsetAsync(hmax_bits, 0, 4, stream));
@@ -1040,10 +946,9 @@ int linkpred_tc_launch(const float *h, int n, int H, const int *pu, const int *p
     pack_weights_halves_kernel<<<(total + 255) / 256, 256, 0, stream>>>(prm, H, L - 1, img);
     EPS_LAUNCH_CHECK();
   }
-  int *tile_order = (int *)tail;
-#define EPS_TC3(HV)                                                                                                              \
-  return use_table ? tc3_launch_h<HV, true>(table, pu, pv, M, prm, L, apply_sigmoid, score, img, n, tile_order, scale, stream)  \
-                   : tc3_launch_h<HV, false>(h, pu, pv, M, prm, L, apply_sigmoid, score, img, n, tile_order, scale, stream)
+#define EPS_TC3(HV)                                                                                           \
+  return use_table ? tc3_launch<HV, true>(table, pu, pv, M, prm, L, apply_sigmoid, score, img, scale, stream) \
+                   : tc3_launch<HV, false>(h, pu, pv, M, prm, L, apply_sigmoid, score, img, scale, stream)
   if (H == 64) { EPS_TC3(64); }
   if (H == 128) { EPS_TC3(128); }
   EPS_TC3(256);

@@ -248,10 +248,8 @@ class LinkpredTC:
         M = pu.numel()
         if M < 2 * n:                      # short list: no fp16 table in the workspace, nothing to reuse
             return linkpred_mlp(self.h, edges, self.Ws, self.bs, "f16", sigmoid)
-        need = int(lib.eps_linkpred_workspace_bytes(n, H, L, M, EPS_MLP_TC_F16))
-        if self.ws is None or self.ws.numel() < need:
-            self.ws = _ws(need + (M // 256) * 2, self.h.device)      # headroom for somewhat longer slabs
-            self.prepared = False
+        if self.ws is None:                # on the table path the size depends on (n, H, L) only
+            self.ws = _ws(lib.eps_linkpred_workspace_bytes(n, H, L, M, EPS_MLP_TC_F16), self.h.device)
         Wp = (C.c_void_p * L)(*[w.data_ptr() for w in self.Ws])
         bp = (C.c_void_p * L)(*[b.data_ptr() for b in self.bs])
         score = torch.empty(M, dtype=torch.float32, device=self.h.device)

@@ -155,8 +155,8 @@ size_t eps_cn_aa_workspace_bytes(void);
 /* OR-ed into `precision` with EPS_MLP_TC_F16: `workspace` is the buffer of an EARLIER call with the same h
  * (contents), weights, n, H and L, and both calls have M >= 2n (the fp16 copy of h exists) — the scale, the fp16 table
  * and the weight images in it are reused instead of rebuilt (one filter job scores ~100 slabs against the
- * same embeddings).  The workspace must be at least eps_linkpred_workspace_bytes(n, H, L, M_max, ...) for
- * the largest M of the series; its layout does not depend on M except for the tail. */
+ * same embeddings).  For M >= 2n, eps_linkpred_workspace_bytes(n, H, L, M, EPS_MLP_TC_F16) and the workspace
+ * layout depend on (n, H, L) only, so one buffer sized by any call of the series serves all of them. */
 #define EPS_MLP_REUSE_WORKSPACE 0x100
 int eps_linkpred_mlp(const float *h, int32_t n, int32_t H, const int32_t *pair_u,
                      const int32_t *pair_v, int64_t M, const float *const *W_h,

@@ -40,6 +40,8 @@ def test_argument_validation_needs_no_device():
     assert lib.eps_topk_workspace_bytes(1 << 20, 1000) > 0
     assert lib.eps_linkpred_workspace_bytes(1000, 256, 3, 5000, 0) >= 256
     assert lib.eps_linkpred_workspace_bytes(1000, 256, 3, 5000, 1) >= 256 + 2 * 256 * 256 * 2 + 1000 * 256 * 2
+    # on the fp16-table path (M >= 2n) the size does not depend on M: ops.LinkpredTC sizes one buffer for a whole series
+    assert len({lib.eps_linkpred_workspace_bytes(1000, 256, 3, M, 1) for M in (2000, 5000, 1 << 20, 1 << 33)}) == 1
 
 
 def test_no_cpu_fallback():
